@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define PSVAE_ABI_VERSION 4      /* 4: + psvae_adam_step_ex (amsgrad / maximize) */
+#define PSVAE_ABI_VERSION 5      /* 4: + psvae_adam_step_ex (amsgrad / maximize); 5: + device step counters (CUDA-graph replay) */
 #define PSVAE_MAX_LAYERS 8      /* Linear layers per MLP (num_hidden + 1) */
 #define PSVAE_MAX_CLF_TRUNK 4   /* hidden Linear layers of the latent classifier */
 #define PSVAE_MAX_CLF_HEADS 4   /* output heads of the latent classifier */
@@ -226,6 +226,33 @@ int psvae_train_fwd_bwd_consistency(const psvae_model_desc* desc, const float* p
                                     float* losses, void* workspace, int64_t workspace_bytes, void* stream,
                                     const psvae_consistency_desc* cons, const float* cons_params, const int64_t* cons_y,
                                     float cons_weight);
+
+/* ---- the train step with its per-step scalars in device memory (a CUDA graph replays it unchanged) ---------------------------------
+ * A captured launch freezes its kernel arguments, so the three values that change every step -- the Philox offset of the eps draw, Adam's
+ * step count and the learning rate -- are read from caller-allocated device memory instead.  The caller keeps one counter block per
+ * parameter group it steps together and one fp64 lr per group, writes them (cudaMemcpyAsync) whenever its own host copies change, and
+ * ends each step with psvae_step_counters_advance. */
+typedef struct psvae_step_counters {
+  uint64_t rng_offset; /* Philox offset of the next train step's eps draw                        */
+  int64_t adam_step;   /* Adam steps taken so far (the next update uses t = adam_step + 1)       */
+  int64_t reserved_[2];
+} psvae_step_counters;
+/* psvae_train_fwd_bwd_consistency (cons may be NULL: no consistency term) whose in-kernel Philox draw takes its offset from
+ * counters->rng_offset (`offset` is then ignored).  counters == NULL: exactly psvae_train_fwd_bwd(_consistency). */
+int psvae_train_fwd_bwd_dc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x,
+                           int32_t x_dtype, const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows,
+                           float kl_weight, float clf_weight, int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat,
+                           float* mu, float* log_sigma, float* losses, void* workspace, int64_t workspace_bytes, void* stream,
+                           const psvae_consistency_desc* cons, const float* cons_params, const int64_t* cons_y, float cons_weight,
+                           const psvae_step_counters* counters);
+/* psvae_adam_step_ex with t = counters->adam_step + 1 and the learning rate *lr (fp64, device) read on the device: for the same t and lr
+ * the update is bit-identical (lr / (1 - beta1^t) and sqrt(1 - beta2^t) formed in fp64 with the same expressions, each rounded to fp32
+ * once).  Does not advance the counters. */
+int psvae_adam_step_dc(float* p, const float* g, float* m, float* v, float* vmax, int64_t n, const double* lr,
+                       const psvae_step_counters* counters, double beta1, double beta2, double eps, double weight_decay, double grad_scale,
+                       int32_t amsgrad, int32_t maximize, void* shadow_bf16, void* stream);
+/* rng_offset += 1, adam_step += 1 (one thread); enqueue after the step's last reader of the block */
+int psvae_step_counters_advance(psvae_step_counters* counters, void* stream);
 
 /* ---- conditional_synthesis Langevin loop (ps_vae/inference.py:72-103) --------------------------- */
 /* z_io [rows][L]: z0 == NULL-initialised by the caller or (init_from_philox != 0) drawn in-kernel with

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # PSVAE_B200_LIB: load another build of the same ABI instead (A/B timing of two kernel versions in one process tree; tools only)
 LIB_PATH = os.environ.get("PSVAE_B200_LIB") or os.path.join(HERE, "libpsvae_b200.so")
 
-PSVAE_ABI_VERSION = 4
+PSVAE_ABI_VERSION = 5
 MAX_LAYERS = 8
 MAX_CLF_TRUNK = 4
 MAX_CLF_HEADS = 4
@@ -32,8 +32,12 @@ EXPORTS = [
     "psvae_refresh_shadow", "psvae_forward", "psvae_decode", "psvae_train_fwd_bwd", "psvae_langevin", "psvae_gemm_bf16",
     "psvae_gemm_fp32", "psvae_gemm_probe", "psvae_launch_count", "psvae_consistency_desc_init", "psvae_consistency_workspace_bytes",
     "psvae_consistency_forward", "psvae_train_fwd_bwd_consistency", "psvae_vae_backward", "psvae_gather_rows",
-    "psvae_embedding_classifier_workspace_bytes", "psvae_embedding_classifier_step",
+    "psvae_embedding_classifier_workspace_bytes", "psvae_embedding_classifier_step", "psvae_train_fwd_bwd_dc", "psvae_adam_step_dc",
+    "psvae_step_counters_advance",
 ]
+
+#: int64 slots of ``psvae_step_counters`` (a device tensor of COUNTER_SLOTS int64)
+COUNTER_RNG_OFFSET, COUNTER_ADAM_STEP, COUNTER_SLOTS = 0, 1, 4
 
 
 class ModelDesc(C.Structure):
@@ -115,6 +119,12 @@ def _declare(l: C.CDLL) -> None:
     l.psvae_embedding_classifier_step.argtypes = [CD, VP, VP, VP, VP, I64, I32, VP, VP, VP, I64, VP]
     l.psvae_train_fwd_bwd_consistency.restype = C.c_int
     l.psvae_train_fwd_bwd_consistency.argtypes = l.psvae_train_fwd_bwd.argtypes + [CD, VP, VP, F]
+    l.psvae_train_fwd_bwd_dc.restype = C.c_int
+    l.psvae_train_fwd_bwd_dc.argtypes = l.psvae_train_fwd_bwd_consistency.argtypes + [VP]
+    l.psvae_adam_step_dc.restype = C.c_int
+    l.psvae_adam_step_dc.argtypes = [VP, VP, VP, VP, VP, I64, VP, VP, DBL, DBL, DBL, DBL, DBL, C.c_int32, C.c_int32, VP, VP]
+    l.psvae_step_counters_advance.restype = C.c_int
+    l.psvae_step_counters_advance.argtypes = [VP, VP]
     l.psvae_langevin.restype = C.c_int
     l.psvae_langevin.argtypes = [D, VP, VP, I64, P(I32), F, I32, F, U64, U64, I64, I32, VP, VP, VP, F, F, VP, VP, VP]
     l.psvae_gemm_bf16.restype = C.c_int

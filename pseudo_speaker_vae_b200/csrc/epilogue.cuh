@@ -244,7 +244,9 @@ struct EpiStore {
 // the linear-head classifier on mu, cross entropy, accuracy, d loss / d logits -- with a row's mu AND log_sigma in one thread's registers
 // (model.py:54-57, lightning.py:73-83,115-117).  Outputs: mu / log_sigma (fp32) and z / sigma eps / 2 (TZ) through TMA stores, d loss / d logits
 // rows for the backward (latent_bwd_clf_kernel), one (kl, nll, acc) partial per CTA.  Single classifier head with <= 4 classes, or none.
-template <typename TZ>
+// DEV_OFF: the Philox offset is *offset_dev (device step counters), read by the epilogue warps after their accumulator-ready wait (only the
+// producer passes griddepcontrol.wait; the epilogue is ordered behind it by the mbarrier chain, so by then what earlier kernels wrote is visible)
+template <typename TZ, bool DEV_OFF = false>
 struct EpiLatent {
   using TOut = float;
   static constexpr bool kReduce = false, kColSum = false, kSplit = false;
@@ -268,6 +270,12 @@ struct EpiLatent {
   float* kl_part;        // [CTAs]
   float* nll_part;       // [CTAs]
   float* acc_part;       // [CTAs]
+  const uint64_t* offset_dev;   // DEV_OFF only
+  // read where the noise is drawn: after the accumulator-ready wait
+  __device__ __forceinline__ uint64_t rng_offset() const {
+    if constexpr (DEV_OFF) return *offset_dev;
+    else return offset;
+  }
   // the generic epilogue loop is never entered for this functor (the kernel's kLat branch takes every tile); these keep it compilable
   __device__ __forceinline__ uint32_t tc_pre(int64_t, int, bool) const { return 0u; }
   __device__ __forceinline__ void tc_transform(int64_t, int, int, bool, float (&)[32], const float (&)[32], uint32_t, float&) const {}

@@ -551,7 +551,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& tma_a, const CUt
           float4* const scratch = reinterpret_cast<float4*>(st_mu);
           const uint64_t q0 = (uint64_t)epi.first_quad + (((uint64_t)row * (uint64_t)epi.L + (uint64_t)lat0) >> 2);
 #pragma unroll 2
-          for (int q = 0; q < 8; ++q) scratch[q * 32 + lane] = philox_normal4(q0 + (uint64_t)q, epi.seed, epi.offset);
+          for (int q = 0; q < 8; ++q) scratch[q * 32 + lane] = philox_normal4(q0 + (uint64_t)q, epi.seed, epi.rng_offset());
 #pragma unroll
           for (int q = 0; q < 8; ++q) {
             const float4 t = scratch[q * 32 + lane];
@@ -1061,10 +1061,10 @@ int gemm_tc_launch_bn(const TcOperand& A, const TcOperand& B, int64_t M, int N, 
 
 // Fused encoder head (EpiLatent): he [M][2H] bf16 (mu half | sigma half), Wstack [2L][H] bf16 (W_mu rows, then W_sigma rows).  One CTA per
 // 128-row tile; outputs through 3D maps (slice 0 / 1 = mu / log_sigma, z / sigma eps / 2).  Returns the CTAs launched in *ctas.
-template <typename TZ>
-int gemm_tc_launch_latent(const void* he, int64_t ldhe, const void* Wstack, int H, int64_t M, const EpiLatent<TZ>& epi, float* mu, float* ls, TZ* z, TZ* hs,
-                          cudaStream_t st, int* ctas) {
-  using Epi = EpiLatent<TZ>;
+template <typename TZ, bool DEV_OFF>
+int gemm_tc_launch_latent(const void* he, int64_t ldhe, const void* Wstack, int H, int64_t M, const EpiLatent<TZ, DEV_OFF>& epi, float* mu, float* ls, TZ* z,
+                          TZ* hs, cudaStream_t st, int* ctas) {
+  using Epi = EpiLatent<TZ, DEV_OFF>;
   constexpr int BN = 128;
   using Cfg = TcCfg<BN, Epi, 1>;
   const int Lz = TC_LAT_L;

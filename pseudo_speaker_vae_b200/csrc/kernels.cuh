@@ -44,9 +44,8 @@ __device__ __forceinline__ void adam_one_ex(float& p, float g, float& m, float& 
   p = p - a.lr_step * (m / denom);
 }
 // the general form: one element per thread and trip (these configurations are not on any benchmarked path)
-__global__ void __launch_bounds__(256) adam_ex_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
-                                                      float* __restrict__ vmax, int64_t n, AdamArgs a, int amsgrad, int maximize, bf16* __restrict__ shadow) {
-  PSVAE_GRID_DEP();
+__device__ __forceinline__ void adam_ex_pass(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                                             float* __restrict__ vmax, int64_t n, const AdamArgs& a, int amsgrad, int maximize, bf16* __restrict__ shadow) {
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
     float pp = p[i], mm = m[i], vv = v[i], vx = amsgrad ? vmax[i] : 0.f;
@@ -57,9 +56,14 @@ __global__ void __launch_bounds__(256) adam_ex_kernel(float* __restrict__ p, con
   }
 }
 
-__global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
-                                                   float* __restrict__ v, int64_t n, AdamArgs a, bf16* __restrict__ shadow) {
+__global__ void __launch_bounds__(256) adam_ex_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                                                      float* __restrict__ vmax, int64_t n, AdamArgs a, int amsgrad, int maximize, bf16* __restrict__ shadow) {
   PSVAE_GRID_DEP();
+  adam_ex_pass(p, g, m, v, vmax, n, a, amsgrad, maximize, shadow);
+}
+
+__device__ __forceinline__ void adam_pass(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, int64_t n,
+                                          const AdamArgs& a, bf16* __restrict__ shadow) {
   const int64_t n4 = n >> 2;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
@@ -89,6 +93,43 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const 
     p[t] = pp; m[t] = mm; v[t] = vv;
     if (shadow) shadow[t] = __float2bfloat16_rn(pp);
   }
+}
+
+__global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
+                                                   float* __restrict__ v, int64_t n, AdamArgs a, bf16* __restrict__ shadow) {
+  PSVAE_GRID_DEP();
+  adam_pass(p, g, m, v, n, a, shadow);
+}
+
+// Device-counter form (CUDA-graph replay): t = *step_done + 1 and lr = *lr come from device memory, read after the grid dependency (the
+// previous step's counter advance and a host write of the block are complete by then).  `a` arrives with lr_step / bc2_sqrt unset; they are
+// formed here in fp64 exactly as psvae_adam_step forms them on the host, each rounded to fp32 once.  EX: the amsgrad / maximize form.
+template <bool EX>
+__global__ void __launch_bounds__(256) adam_dc_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                                                      float* __restrict__ vmax, int64_t n, AdamArgs a, double beta1, double beta2,
+                                                      const double* __restrict__ lr, const int64_t* __restrict__ step_done, int amsgrad, int maximize,
+                                                      bf16* __restrict__ shadow) {
+  PSVAE_GRID_DEP();
+  __shared__ float s_lr_step, s_bc2_sqrt;
+  if (threadIdx.x == 0) {
+    const double t = (double)(*step_done + 1);
+    const double bc1 = 1.0 - pow(beta1, t);
+    const double bc2 = 1.0 - pow(beta2, t);
+    s_lr_step = (float)(*lr / bc1);
+    s_bc2_sqrt = (float)sqrt(bc2);
+  }
+  __syncthreads();
+  a.lr_step = s_lr_step;
+  a.bc2_sqrt = s_bc2_sqrt;
+  if constexpr (EX) adam_ex_pass(p, g, m, v, vmax, n, a, amsgrad, maximize, shadow);
+  else adam_pass(p, g, m, v, n, a, shadow);
+}
+
+// rng_offset += 1, adam_step += 1 at the end of a device-counter step (every reader of the block has finished: it is the last launch)
+__global__ void step_counters_advance_kernel(uint64_t* __restrict__ rng_offset, int64_t* __restrict__ adam_step) {
+  PSVAE_GRID_DEP();
+  *rng_offset += 1;
+  *adam_step += 1;
 }
 
 // ---------------------------------------------------------------- Philox
@@ -164,13 +205,15 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const uint4* __restric
 
 // ---------------------------------------------------------------- latent forward / backward
 // Thread = 4 consecutive latent elements (= one Philox block).  KL partial: one slot per block.
-template <typename TAct>
+// DEV_OFF: the Philox offset is *offset_dev (device step counters, read after the grid dependency) instead of `offset`
+template <typename TAct, bool DEV_OFF = false>
 __global__ void __launch_bounds__(256) latent_fwd_kernel(const float* __restrict__ mu, const float* __restrict__ ls, const float* __restrict__ eps,
                                                          uint64_t seed, uint64_t offset, int64_t first_elem, int64_t n_elems,
                                                          TAct* __restrict__ z, float* __restrict__ z_f32, float* __restrict__ kl_partials,
-                                                         TAct* __restrict__ hs) {
+                                                         TAct* __restrict__ hs, const uint64_t* __restrict__ offset_dev) {
   // hs (optional): sigma * eps / 2 = d z / d log_sigma, stashed for the backward pass (which then needs neither eps nor exp(ls / 2))
   PSVAE_GRID_DEP();
+  if constexpr (DEV_OFF) offset = *offset_dev;
   __shared__ float scratch[32];
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   const int64_t nq = n_elems >> 2;
@@ -548,6 +591,7 @@ struct ReparamArgs {
   void* z;                      // [B][L] TZ
   float* kl_part;               // one slot per block
   void* hs;                     // optional [B][L] TZ: sigma * eps / 2, stashed for the backward pass
+  const uint64_t* offset_dev;   // clf_fused_kernel<..., DEV_OFF = true>: the Philox offset lives here (device step counters)
 };
 __host__ __device__ __forceinline__ int clf_part_len(int L) { return 8 + CLF_MAXC * L + CLF_MAXC; }   // nll[4] acc[4] dW[8][L] db[8]
 
@@ -562,10 +606,12 @@ static inline size_t clf_fused_smem_bytes(int L) { return ((size_t)CLF_TILE * (L
 // L is a template parameter (16/32/64/128) so that the row/column index arithmetic is shifts and everything moves as float4; class
 // loops run over the classes that exist (2..3 per head), not over the CLF_MAXC slots.
 // GROWS (option "clf_grad_in_bwd"): only g_rows leaves the pass; phase 3 and the classifier-gradient tail are compiled out
-template <int L, typename TZ, bool REPARAM, bool GROWS = false>
+// DEV_OFF: the Philox offset is *rp.offset_dev, read after the grid dependency
+template <int L, typename TZ, bool REPARAM, bool GROWS = false, bool DEV_OFF = false>
 __global__ void __launch_bounds__(CLF_TILE) clf_fused_kernel(const float* __restrict__ params, const float* __restrict__ mu, const int64_t* __restrict__ y,
                                                              int64_t B, ClfFusedArgs a, float* __restrict__ dmu_clf, float* __restrict__ part, ReparamArgs rp) {
   PSVAE_GRID_DEP();
+  if constexpr (DEV_OFF) rp.offset = *rp.offset_dev;
   float kl = 0.f;
   extern __shared__ __align__(16) float clf_smem[];
   __shared__ float scratch[32];

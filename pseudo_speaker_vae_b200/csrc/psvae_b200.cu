@@ -740,6 +740,8 @@ struct StepArgs {
   // ... or the same batch already in bf16 (PSVAE_X_BF16; tensor-core mode only): the operand of the first GEMM as it is, no cast pass, and the
   // reconstruction target of the MSE epilogue (the data ARE these bf16 values: a bf16 embedding store, data.py)
   const bf16* x16 = nullptr;
+  // device step counters (psvae_train_fwd_bwd_dc): the Philox offset of the eps draw is read from here instead of `offset`
+  const uint64_t* offset_dev = nullptr;
 };
 
 template <typename TAct> static const TAct* weights_of(const StepArgs& a);
@@ -757,6 +759,16 @@ static int decoder_forward(const Net& n, const TAct* Wt, const float* params, co
     a = hd[j];
   }
   return Engine<TAct>::template gemm<G_FWD>(a, n.H, Wt + n.d->dec_w[n.nh], n.H, rows, n.D, n.H, 1, n.D % 4 == 0, last_epi, st);
+}
+
+// clf_fused_kernel<REPARAM> with its dynamic shared memory; GROWS: option clf_grad_in_bwd, DEV_OFF: device step counters
+template <int LL, typename TAct, bool GROWS, bool DEV_OFF>
+static int launch_clf_fused(int blocks, size_t smem, cudaStream_t st, const float* P, const float* mu, const int64_t* y, int64_t B, const ClfFusedArgs& ca,
+                            float* dmu_out, float* part, const ReparamArgs& rp) {
+  auto kern = clf_fused_kernel<LL, TAct, true, GROWS, DEV_OFF>;
+  PSVAE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  launch_dep(kern, dim3(blocks), dim3(CLF_TILE), smem, st, P, mu, y, B, ca, dmu_out, part, rp);
+  return 0;
 }
 
 template <typename TAct>
@@ -866,23 +878,31 @@ static int run_step(const StepArgs& a) {
   int fused_ctas = 0;
   if constexpr (sizeof(TAct) == 2) {
     if (fused_head) {
-      EpiLatent<TAct> e;
-      memset(&e, 0, sizeof(e));
-      e.out = mu; e.ldo = n.L;
-      e.bias = P + d->enc_b[n.nh];
-      e.z = w.z;
-      e.eps = a.eps; e.seed = a.seed; e.offset = a.offset; e.first_quad = first_elem >> 2;
-      e.L = n.L;
-      e.nc = n.has_clf() ? d->clf_head_classes[0] : 0;
-      e.clf_w = n.has_clf() ? P + d->clf_head_w[0] : nullptr;
-      e.clf_b = n.has_clf() ? P + d->clf_head_b[0] : nullptr;
-      e.y = a.y;
-      e.gscale = a.clf_w / (float)B;
-      e.g_rows = n.has_clf() ? w.clf_grows : nullptr;
-      e.kl_part = w.kl_part;
-      e.nll_part = n.has_clf() ? w.clf_part : nullptr;
-      e.acc_part = n.has_clf() ? w.clf_part + PSVAE_NUM_SMS : nullptr;
-      PSVAE_TRY(gemm_tc_launch_latent<TAct>(w.he[n.nh - 1], 2 * n.H, Wt + d->enc_w[n.nh], n.H, B, e, mu, ls, w.z, w.hs, st, &fused_ctas));
+      auto launch = [&](auto& e) -> int {
+        memset(&e, 0, sizeof(e));
+        e.out = mu; e.ldo = n.L;
+        e.bias = P + d->enc_b[n.nh];
+        e.z = w.z;
+        e.eps = a.eps; e.seed = a.seed; e.offset = a.offset; e.offset_dev = a.offset_dev; e.first_quad = first_elem >> 2;
+        e.L = n.L;
+        e.nc = n.has_clf() ? d->clf_head_classes[0] : 0;
+        e.clf_w = n.has_clf() ? P + d->clf_head_w[0] : nullptr;
+        e.clf_b = n.has_clf() ? P + d->clf_head_b[0] : nullptr;
+        e.y = a.y;
+        e.gscale = a.clf_w / (float)B;
+        e.g_rows = n.has_clf() ? w.clf_grows : nullptr;
+        e.kl_part = w.kl_part;
+        e.nll_part = n.has_clf() ? w.clf_part : nullptr;
+        e.acc_part = n.has_clf() ? w.clf_part + PSVAE_NUM_SMS : nullptr;
+        return gemm_tc_launch_latent(w.he[n.nh - 1], 2 * n.H, Wt + d->enc_w[n.nh], n.H, B, e, mu, ls, w.z, w.hs, st, &fused_ctas);
+      };
+      if (a.offset_dev) {
+        EpiLatent<TAct, true> e;
+        PSVAE_TRY(launch(e));
+      } else {
+        EpiLatent<TAct> e;
+        PSVAE_TRY(launch(e));
+      }
       head_done = true;
       if (a.mu) PSVAE_CUDA(cudaMemcpyAsync(a.mu, mu, (size_t)B * n.L * sizeof(float), cudaMemcpyDeviceToDevice, st));
       if (a.ls) PSVAE_CUDA(cudaMemcpyAsync(a.ls, ls, (size_t)B * n.L * sizeof(float), cudaMemcpyDeviceToDevice, st));
@@ -909,8 +929,8 @@ static int run_step(const StepArgs& a) {
   if (fused_head) {
     n_kl_used = fused_ctas;            // the fused kernel wrote one KL / NLL / accuracy record per CTA
   } else if (!fuse_latent) {
-    launch_dep(latent_fwd_kernel<TAct>, dim3((unsigned)w.n_kl), dim3(256), 0, st, mu, ls, a.eps, a.seed, a.offset, first_elem, B * n.L, w.z, nullptr, w.kl_part,
-                                                                  a.want_grads ? w.hs : nullptr);
+    launch_dep(a.offset_dev ? latent_fwd_kernel<TAct, true> : latent_fwd_kernel<TAct>, dim3((unsigned)w.n_kl), dim3(256), 0, st, mu, ls, a.eps, a.seed,
+               a.offset, first_elem, B * n.L, w.z, nullptr, w.kl_part, a.want_grads ? w.hs : nullptr, a.offset_dev);
     count_launch();
     PSVAE_LAUNCH_CHECK("latent_fwd_kernel");
   } else {
@@ -935,18 +955,15 @@ static int run_step(const StepArgs& a) {
     const int blocks = clf_fused_blocks(B);
     const size_t smem = clf_fused_smem_bytes(n.L);
     float* dmu_out = a.want_grads ? w.dmu_clf : nullptr;
-    ReparamArgs rp{ls, a.eps, a.seed, a.offset, first_elem >> 2, w.z, w.kl_part, a.want_grads ? w.hs : nullptr};
+    ReparamArgs rp{ls, a.eps, a.seed, a.offset, first_elem >> 2, w.z, w.kl_part, a.want_grads ? w.hs : nullptr, a.offset_dev};
     n_kl_used = blocks;
     switch (n.L) {
 #define PSVAE_CLF_CASE(LL)                                                                                                              \
       case LL:                                                                                                                          \
-        if (ca.g_rows) {                                                                                                                \
-          PSVAE_CUDA(cudaFuncSetAttribute(clf_fused_kernel<LL, TAct, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-          launch_dep(clf_fused_kernel<LL, TAct, true, true>, dim3(blocks), dim3(CLF_TILE), smem, st, P, mu, a.y, B, ca, dmu_out, w.clf_part, rp); \
-          break;                                                                                                                        \
-        }                                                                                                                               \
-        PSVAE_CUDA(cudaFuncSetAttribute(clf_fused_kernel<LL, TAct, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));    \
-        launch_dep(clf_fused_kernel<LL, TAct, true>, dim3(blocks), dim3(CLF_TILE), smem, st, P, mu, a.y, B, ca, dmu_out, w.clf_part, rp); \
+        if (a.offset_dev) PSVAE_TRY((ca.g_rows ? launch_clf_fused<LL, TAct, true, true>(blocks, smem, st, P, mu, a.y, B, ca, dmu_out, w.clf_part, rp)  \
+                                               : launch_clf_fused<LL, TAct, false, true>(blocks, smem, st, P, mu, a.y, B, ca, dmu_out, w.clf_part, rp))); \
+        else PSVAE_TRY((ca.g_rows ? launch_clf_fused<LL, TAct, true, false>(blocks, smem, st, P, mu, a.y, B, ca, dmu_out, w.clf_part, rp)                 \
+                                  : launch_clf_fused<LL, TAct, false, false>(blocks, smem, st, P, mu, a.y, B, ca, dmu_out, w.clf_part, rp)));              \
         break;
       PSVAE_CLF_CASE(16)
       PSVAE_CLF_CASE(32)
@@ -1604,6 +1621,48 @@ int psvae_adam_step_ex(float* p, const float* g, float* m, float* v, float* vmax
   return 0;
 }
 
+int psvae_adam_step_dc(float* p, const float* g, float* m, float* v, float* vmax, int64_t n, const double* lr, const psvae_step_counters* counters,
+                       double beta1, double beta2, double eps, double weight_decay, double grad_scale, int32_t amsgrad, int32_t maximize, void* shadow_bf16,
+                       void* stream) {
+  PSVAE_TRY(tc_device_check());
+  if (!p || !g || !m || !v || !lr || !counters || (amsgrad && !vmax)) {
+    set_error("p, g, m, v, lr, counters (and vmax with amsgrad) must not be NULL");
+    return -1;
+  }
+  if (n <= 0) return 0;
+  const bool ex = amsgrad || maximize;
+  if (!ex && ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v)) & 15) != 0) {
+    set_error("Adam buffers must be 16-byte aligned");
+    return -2;
+  }
+  AdamArgs a;      // lr_step / bc2_sqrt are formed on the device from *lr and the step counter
+  a.lr_step = 0.f; a.bc2_sqrt = 1.f;
+  a.beta1 = (float)beta1; a.beta2 = (float)beta2;
+  a.one_minus_beta1 = (float)(1.0 - beta1);
+  a.one_minus_beta2 = (float)(1.0 - beta2);
+  a.eps = (float)eps; a.weight_decay = (float)weight_decay; a.grad_scale = (float)grad_scale;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  bf16* sh = static_cast<bf16*>(shadow_bf16);
+  if (ex)
+    launch_dep(adam_dc_kernel<true>, dim3(ew_grid(n)), dim3(256), 0, st, p, g, m, v, vmax, n, a, beta1, beta2, lr, &counters->adam_step, (int)amsgrad,
+               (int)maximize, sh);
+  else
+    launch_dep(adam_dc_kernel<false>, dim3(ew_grid(n / 4 + 1)), dim3(256), 0, st, p, g, m, v, (float*)nullptr, n, a, beta1, beta2, lr, &counters->adam_step,
+               0, 0, sh);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("adam_dc_kernel");
+  return 0;
+}
+
+int psvae_step_counters_advance(psvae_step_counters* counters, void* stream) {
+  PSVAE_TRY(tc_device_check());
+  if (!counters) { set_error("counters must not be NULL"); return -1; }
+  launch_dep(step_counters_advance_kernel, dim3(1), dim3(1), 0, static_cast<cudaStream_t>(stream), &counters->rng_offset, &counters->adam_step);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("step_counters_advance_kernel");
+  return 0;
+}
+
 int psvae_philox_uint32(uint32_t* out, int64_t n, uint64_t seed, uint64_t offset, int64_t first_elem, void* stream) {
   PSVAE_TRY(tc_device_check());
   if (!out) { set_error("out is NULL"); return -1; }
@@ -1807,6 +1866,20 @@ int psvae_train_fwd_bwd_consistency(const psvae_model_desc* desc, const float* p
              use_cos_loss ? 1 : 0, 1, compute_grads ? 1 : 0, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, static_cast<cudaStream_t>(stream)};
   PSVAE_TRY(set_x(a, x, x_dtype));
   a.cons = cons; a.cons_params = cons_params; a.cons_y = cons_y; a.cons_w = cons_weight;
+  return precision == PSVAE_BF16 ? run_step<bf16>(a) : run_step<float>(a);
+}
+
+int psvae_train_fwd_bwd_dc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
+                           const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
+                           int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
+                           void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
+                           const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters) {
+  PSVAE_TRY(check_desc(desc, precision));
+  StepArgs a{desc, params, static_cast<const bf16*>(shadow_bf16), grads, nullptr, y, eps, seed, offset, row0, rows, kl_weight, clf_weight,
+             use_cos_loss ? 1 : 0, 1, compute_grads ? 1 : 0, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, static_cast<cudaStream_t>(stream)};
+  PSVAE_TRY(set_x(a, x, x_dtype));
+  a.cons = cons; a.cons_params = cons_params; a.cons_y = cons_y; a.cons_w = cons_weight;
+  a.offset_dev = counters ? &counters->rng_offset : nullptr;
   return precision == PSVAE_BF16 ? run_step<bf16>(a) : run_step<float>(a);
 }
 

@@ -454,11 +454,15 @@ class HotPath:
 
     def step(self, x: torch.Tensor, y=None, eps: Optional[torch.Tensor] = None, *, kl_weight: float = 1.0, clf_weight: float = 1.0,
              use_cos_loss: bool = False, compute_grads: bool = True, grads: Optional[torch.Tensor] = None, want_outputs: bool = False,
-             consistency: Optional[nn.Module] = None, consistency_y: Optional[torch.Tensor] = None, consistency_weight: float = 1.0):
+             consistency: Optional[nn.Module] = None, consistency_y: Optional[torch.Tensor] = None, consistency_weight: float = 1.0,
+             counters: Optional[torch.Tensor] = None):
         """One fused forward(+backward).  Returns (losses[16] device tensor, flat grads or None, outputs or None).
 
         ``consistency``: a frozen ``EmbeddingClassifier`` whose ``consistency_weight * CE(consistency(x_hat), consistency_y)``
-        joins the loss (lightning.py:100-108, 119-124).  losses slots: _lib.LOSS_*; nothing here synchronises with the host."""
+        joins the loss (lightning.py:100-108, 119-124).  losses slots: _lib.LOSS_*; nothing here synchronises with the host.
+        ``counters``: a device ``psvae_step_counters`` block (int64 [_lib.COUNTER_SLOTS]); the Philox offset of the eps draw is then read
+        from it on the device (``psvae_train_fwd_bwd_dc``), so that a CUDA graph of this call draws fresh noise at every replay.  The host
+        offset still advances as usual: it is the mirror the caller keeps the block in step with."""
         dev = self._device()
         flat = self.arena.ensure()
         D, Lz = self.desc.input_dim, self.desc.latent_dim
@@ -490,12 +494,8 @@ class HotPath:
         args = (self._dref, flat.data_ptr(), self._shadow(), L.ptr(grads) if compute_grads else None, x.data_ptr(), _xflag(x), L.ptr(yy),
                 L.ptr(eps), seed, off, self.row0, B, float(kl_weight), float(clf_weight), int(bool(use_cos_loss)),
                 int(bool(compute_grads)), self.precision, L.ptr(xh), L.ptr(mu), L.ptr(ls), losses.data_ptr())
-        if consistency is None:
-            with _on(dev):
-                ws = self._workspace(dev, B, mode)
-                rc = L.lib().psvae_train_fwd_bwd(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev))
-            L.check(rc, "psvae_train_fwd_bwd")
-        else:
+        cons_args = (None, None, None, 0.0)
+        if consistency is not None:
             if consistency.input_dim != D:
                 raise ValueError(f"consistency classifier input_dim={consistency.input_dim} must equal the VAE input_dim={D}")
             if consistency_y is None or isinstance(consistency_y, dict):
@@ -507,10 +507,23 @@ class HotPath:
             extra = int(L.lib().psvae_consistency_workspace_bytes(C.byref(cdesc), B, mode))
             if extra < 0:
                 raise ValueError(L.last_error())
+            cons_args = (C.byref(cdesc), cflat.data_ptr(), cy.data_ptr(), float(consistency_weight))
+        if counters is not None:
+            if counters.device != dev or counters.dtype != torch.int64 or counters.numel() != L.COUNTER_SLOTS:
+                raise ValueError(f"counters must be an int64 [{L.COUNTER_SLOTS}] tensor on {dev}")
+            with _on(dev):
+                ws = self._workspace(dev, B, mode, extra if consistency is not None else 0)
+                rc = L.lib().psvae_train_fwd_bwd_dc(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args, counters.data_ptr())
+            L.check(rc, "psvae_train_fwd_bwd_dc")
+        elif consistency is None:
+            with _on(dev):
+                ws = self._workspace(dev, B, mode)
+                rc = L.lib().psvae_train_fwd_bwd(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev))
+            L.check(rc, "psvae_train_fwd_bwd")
+        else:
             with _on(dev):
                 ws = self._workspace(dev, B, mode, extra)
-                rc = L.lib().psvae_train_fwd_bwd_consistency(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), C.byref(cdesc), cflat.data_ptr(),
-                                                             cy.data_ptr(), float(consistency_weight))
+                rc = L.lib().psvae_train_fwd_bwd_consistency(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args)
             L.check(rc, "psvae_train_fwd_bwd_consistency")
         return losses, (grads if compute_grads else None), outs
 

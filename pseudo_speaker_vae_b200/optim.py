@@ -120,6 +120,15 @@ class FusedAdam(torch.optim.Optimizer):
         if closure is not None:
             with torch.enable_grad():
                 loss = closure()
+        self._update()
+        return loss
+
+    def _update(self, counters: Optional[torch.Tensor] = None, lrs: Optional[torch.Tensor] = None) -> None:
+        """The update of every group with gradients, one pass per merged span.  ``counters`` / ``lrs``: the device-counter form a CUDA graph
+        of the train step replays (graphs.py) -- one ``psvae_step_counters`` block per group (int64 [groups, COUNTER_SLOTS]) and one fp64
+        learning rate per group, read on the device (``psvae_adam_step_dc``).  That form moves no host state: the caller advances the step
+        counts, the arena epoch and the shadow mark, and the device block, itself."""
+        dc = counters is not None
         flat = self.arena.ensure()
         dev = flat.device
         if dev.type != "cuda":
@@ -129,11 +138,13 @@ class FusedAdam(torch.optim.Optimizer):
         lib = L.lib()
         stream = _stream_ptr(dev)
         touched = False
-        for group in self.param_groups:
+        for gi, group in enumerate(self.param_groups):
             with_grad = [p for p in group["params"] if p.grad is not None]
             if not with_grad:
                 continue
             if gflat is None:
+                if dc:
+                    raise NotImplementedError("the device-counter update reads the gradients from the arena's flat gradient buffer")
                 # gradients were produced outside the fused step (plain autograd on a caller's own loss): gather them
                 gflat = self.arena.stage_buffer()
                 gflat.zero_()          # padding between merged spans must read as zero gradient
@@ -141,16 +152,21 @@ class FusedAdam(torch.optim.Optimizer):
                     off = self._offsets[id(p)]
                     gflat[off:off + p.numel()].copy_(p.grad.reshape(-1))
             step_t = self.state[with_grad[0]]["step"]
-            step = int(step_t.item()) + 1
+            step = 0 if dc else int(step_t.item()) + 1
             beta1, beta2 = group["betas"]
             spans = [(self._offsets[id(p)], self._offsets[id(p)] + p.numel()) for p in with_grad]
             for a, b in self._ranges(spans):
                 shadow = None
                 if self.arena.shadow is not None and self.arena.shadow.device == dev:
                     shadow = self.arena.shadow.data_ptr() + 2 * a
+                vmax = self._vmax.data_ptr() + 4 * a if group["amsgrad"] else None
                 with _on(dev):
-                    if group["amsgrad"] or group["maximize"]:
-                        vmax = self._vmax.data_ptr() + 4 * a if group["amsgrad"] else None
+                    if dc:
+                        rc = lib.psvae_adam_step_dc(flat.data_ptr() + 4 * a, gflat.data_ptr() + 4 * a, m.data_ptr() + 4 * a, v.data_ptr() + 4 * a, vmax, b - a,
+                                                    lrs[gi].data_ptr(), counters[gi].data_ptr(), float(beta1), float(beta2), float(group["eps"]),
+                                                    float(group["weight_decay"]), float(self.grad_scale), int(bool(group["amsgrad"])),
+                                                    int(bool(group["maximize"])), shadow, stream)
+                    elif group["amsgrad"] or group["maximize"]:
                         rc = lib.psvae_adam_step_ex(flat.data_ptr() + 4 * a, gflat.data_ptr() + 4 * a, m.data_ptr() + 4 * a, v.data_ptr() + 4 * a, vmax, b - a,
                                                     float(group["lr"]), float(beta1), float(beta2), float(group["eps"]), float(group["weight_decay"]),
                                                     step, float(self.grad_scale), int(bool(group["amsgrad"])), int(bool(group["maximize"])), shadow, stream)
@@ -160,11 +176,14 @@ class FusedAdam(torch.optim.Optimizer):
                                                  step, float(self.grad_scale), shadow, stream)
                 L.check(rc, "psvae_adam_step")
                 touched = True
-            step_t += 1
-        if touched:
+            if not dc:
+                step_t += 1
+        if touched and not dc:
             self.arena.epoch += 1
-            covered = all(p.grad is not None for g in self.param_groups for p in g["params"]) and \
-                sum(len(g["params"]) for g in self.param_groups) == len(self.arena.entries)
-            if covered and self.arena.shadow is not None:
+            if self.covers_arena() and self.arena.shadow is not None:
                 self.arena.mark_shadow_current()
-        return loss
+
+    def covers_arena(self) -> bool:
+        """Does one update rewrite every parameter of the arena (so that it also leaves the whole bf16 copy current)?"""
+        return all(p.grad is not None for g in self.param_groups for p in g["params"]) and \
+            sum(len(g["params"]) for g in self.param_groups) == len(self.arena.entries)

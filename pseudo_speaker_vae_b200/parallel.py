@@ -181,23 +181,32 @@ class DataParallelTrainer:
 
     def train_step(self, x_local: torch.Tensor, y_local=None, eps_local: Optional[torch.Tensor] = None) -> torch.Tensor:
         """One optimiser step on this rank's shard.  Returns the device tensor of local loss scalars."""
+        losses, gflat = self._fwd_bwd(x_local, y_local, eps_local)
+        self._all_reduce(gflat)
+        if self._views_of is not gflat:        # bind .grad views once; the same flat buffer is reused every step
+            for (p, _), v in zip(self.hot.arena.entries, self.hot.arena.grad_views(gflat)):
+                p.grad = v if p.requires_grad else None
+            self._views_of = gflat
+        self.optimizer.step()
+        return losses
+
+    def _fwd_bwd(self, x_local: torch.Tensor, y_local=None, eps_local: Optional[torch.Tensor] = None, counters: Optional[torch.Tensor] = None):
+        """The fused forward + backward of train_step into the gradient buffer the all-reduce reads.  ``counters``: see HotPath.step."""
         m, hot = self.module, self.hot
         gflat = self.symm.buf if self.symm is not None else (hot.arena.stage_buffer() if self._views_of is None else self._views_of)
         cons = getattr(m, "consistency_classifier", None)
         losses, gflat, _ = hot.step(x_local, y_local if m.classifier is not None else None, eps_local, kl_weight=m.kl_loss_weight,
                                     clf_weight=m.classifier_loss_weight, use_cos_loss=m.use_cos_loss, compute_grads=True, grads=gflat,
                                     consistency=cons, consistency_y=y_local if cons is not None else None,
-                                    consistency_weight=m.consitency_loss_weight)
+                                    consistency_weight=m.consitency_loss_weight, counters=counters)
+        return losses, gflat
+
+    def _all_reduce(self, gflat: torch.Tensor, kind: Optional[str] = None) -> None:
+        """The gradient all-reduce; ``kind`` overrides the symmetric-memory kind ``pick()`` chose (a CUDA graph may need NCCL)."""
         if self.symm is not None:
-            self.symm.all_reduce()
+            self.symm._call(kind or self.symm.kind)
         elif not self.local_only:
             all_reduce_flat(gflat, self.bucket_bytes, self.group)
-        if self._views_of is not gflat:        # bind .grad views once; the same flat buffer is reused every step
-            for (p, _), v in zip(hot.arena.entries, hot.arena.grad_views(gflat)):
-                p.grad = v if p.requires_grad else None
-            self._views_of = gflat
-        self.optimizer.step()
-        return losses
 
 
 def verify_data_parallel_step(device, steps: int = 3, global_batch: int = 8192, input_dim: int = 256, latent_dim: int = 64, num_classes: int = 2,
