@@ -254,6 +254,40 @@ int psvae_adam_step_dc(float* p, const float* g, float* m, float* v, float* vmax
 /* rng_offset += 1, adam_step += 1 (one thread); enqueue after the step's last reader of the block */
 int psvae_step_counters_advance(psvae_step_counters* counters, void* stream);
 
+/* ---- step-level training options: gradient accumulation and clipping (Lightning's accumulate_grad_batches, gradient_clip_val /
+ * gradient_clip_algorithm), device-side so that a CUDA graph replays them unchanged.  Additive to ABI 5. */
+/* psvae_train_fwd_bwd_dc plus `accumulate`: accumulate != 0 (with compute_grads != 0) ADDS this call's gradients to what `grads` holds
+ * instead of overwriting them: the gradients are computed into grad_scratch (total_numel floats, 16-byte aligned, not `grads`) exactly as
+ * the non-accumulating call computes them, then grads[i] += grad_scratch[i] (one fp32 addition per element; padding adds zero).
+ * accumulate == 0: exactly psvae_train_fwd_bwd_dc (grad_scratch unused). */
+int psvae_train_fwd_bwd_acc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x,
+                            int32_t x_dtype, const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows,
+                            float kl_weight, float clf_weight, int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat,
+                            float* mu, float* log_sigma, float* losses, void* workspace, int64_t workspace_bytes, void* stream,
+                            const psvae_consistency_desc* cons, const float* cons_params, const int64_t* cons_y, float cons_weight,
+                            const psvae_step_counters* counters, int32_t accumulate, float* grad_scratch);
+#define PSVAE_GRAD_NORM_MAX_SPANS 16
+#define PSVAE_GRAD_NORM_SCRATCH_BYTES 4096
+/* total_norm = || g * grad_scale ||_2 over the n_spans [a, b) spans (host int64 array {a0, b0, a1, b1, ...}) of the flat gradient, and
+ * coef = min(fp32(max_norm) / (total_norm + 1e-6f), 1.0f) -- torch.nn.utils.clip_grad_norm_ (norm_type 2).  Both are fp32 device scalars.
+ * Squares are summed in fp64 in a fixed order on a fixed grid: bit-identical from run to run.  scratch: PSVAE_GRAD_NORM_SCRATCH_BYTES of
+ * caller-allocated device memory, 8-byte aligned, zeroed once before the first call (the kernel leaves it ready for the next).  No host
+ * synchronisation: capturable. */
+int psvae_grad_norm(const float* g, const int64_t* spans, int32_t n_spans, double grad_scale, double max_norm, float* total_norm, float* coef,
+                    void* scratch, int64_t scratch_bytes, void* stream);
+#define PSVAE_CLIP_NONE 0
+#define PSVAE_CLIP_NORM 1  /* g_eff = g * fp32(grad_scale * *clip_coef)     (clip_coef from psvae_grad_norm; coef = 1 is the unclipped step) */
+#define PSVAE_CLIP_VALUE 2 /* g_eff = clamp(g * grad_scale, -clip_value, clip_value)  (torch.nn.utils.clip_grad_value_) */
+/* Adam with gradient clipping, applied before weight_decay is added and before maximize negates (where torch clips: before
+ * optimizer.step()).  counters == NULL: the host-scalar form (lr, step as psvae_adam_step_ex); counters != NULL: the device form
+ * (lr_dev, counters as psvae_adam_step_dc; lr and step ignored).  clip_mode PSVAE_CLIP_NONE is exactly psvae_adam_step_ex / _dc. */
+int psvae_adam_step_clip(float* p, const float* g, float* m, float* v, float* vmax, int64_t n, double lr, int64_t step, const double* lr_dev,
+                         const psvae_step_counters* counters, double beta1, double beta2, double eps, double weight_decay, double grad_scale,
+                         int32_t amsgrad, int32_t maximize, int32_t clip_mode, const float* clip_coef, double clip_value, void* shadow_bf16,
+                         void* stream);
+/* rng_offset += rng_delta, adam_step += step_delta (one thread): a micro-batch that does not step the optimiser advances the offset only */
+int psvae_step_counters_advance_by(psvae_step_counters* counters, uint64_t rng_delta, int64_t step_delta, void* stream);
+
 /* ---- conditional_synthesis Langevin loop (ps_vae/inference.py:72-103) --------------------------- */
 /* z_io [rows][L]: z0 == NULL-initialised by the caller or (init_from_philox != 0) drawn in-kernel with
  * offset `offset0`; step s uses offset `offset0 + 1 + s` unless `noise` ([num_steps][rows][L]) is given.

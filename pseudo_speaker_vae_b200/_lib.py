@@ -33,11 +33,14 @@ EXPORTS = [
     "psvae_gemm_fp32", "psvae_gemm_probe", "psvae_launch_count", "psvae_consistency_desc_init", "psvae_consistency_workspace_bytes",
     "psvae_consistency_forward", "psvae_train_fwd_bwd_consistency", "psvae_vae_backward", "psvae_gather_rows",
     "psvae_embedding_classifier_workspace_bytes", "psvae_embedding_classifier_step", "psvae_train_fwd_bwd_dc", "psvae_adam_step_dc",
-    "psvae_step_counters_advance",
+    "psvae_step_counters_advance", "psvae_train_fwd_bwd_acc", "psvae_grad_norm", "psvae_adam_step_clip", "psvae_step_counters_advance_by",
 ]
 
 #: int64 slots of ``psvae_step_counters`` (a device tensor of COUNTER_SLOTS int64)
 COUNTER_RNG_OFFSET, COUNTER_ADAM_STEP, COUNTER_SLOTS = 0, 1, 4
+#: psvae_adam_step_clip modes and the psvae_grad_norm limits
+CLIP_NONE, CLIP_NORM, CLIP_VALUE = 0, 1, 2
+GRAD_NORM_MAX_SPANS, GRAD_NORM_SCRATCH_BYTES = 16, 4096
 
 
 class ModelDesc(C.Structure):
@@ -125,6 +128,17 @@ def _declare(l: C.CDLL) -> None:
     l.psvae_adam_step_dc.argtypes = [VP, VP, VP, VP, VP, I64, VP, VP, DBL, DBL, DBL, DBL, DBL, C.c_int32, C.c_int32, VP, VP]
     l.psvae_step_counters_advance.restype = C.c_int
     l.psvae_step_counters_advance.argtypes = [VP, VP]
+    # additive to ABI 5: an earlier ABI-5 build without them (loaded through PSVAE_B200_LIB for A/B timing) still loads
+    if hasattr(l, "psvae_train_fwd_bwd_acc"):
+        l.psvae_train_fwd_bwd_acc.restype = C.c_int
+        l.psvae_train_fwd_bwd_acc.argtypes = l.psvae_train_fwd_bwd_dc.argtypes + [I32, VP]
+        l.psvae_grad_norm.restype = C.c_int
+        l.psvae_grad_norm.argtypes = [VP, P(I64), I32, DBL, DBL, VP, VP, VP, I64, VP]
+        l.psvae_adam_step_clip.restype = C.c_int
+        l.psvae_adam_step_clip.argtypes = [VP, VP, VP, VP, VP, I64, DBL, I64, VP, VP, DBL, DBL, DBL, DBL, DBL, C.c_int32, C.c_int32, C.c_int32, VP,
+                                           DBL, VP, VP]
+        l.psvae_step_counters_advance_by.restype = C.c_int
+        l.psvae_step_counters_advance_by.argtypes = [VP, U64, I64, VP]
     l.psvae_langevin.restype = C.c_int
     l.psvae_langevin.argtypes = [D, VP, VP, I64, P(I32), F, I32, F, U64, U64, I64, I32, VP, VP, VP, F, F, VP, VP, VP]
     l.psvae_gemm_bf16.restype = C.c_int

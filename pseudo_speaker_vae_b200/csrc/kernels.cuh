@@ -1,5 +1,6 @@
 // Element-wise / reduction kernels of the hot path (everything that is not a GEMM):
 //   adam_kernel            torch.optim.Adam single-tensor update (torch/optim/adam.py:416-547) over the flat buffer
+//   grad_norm_kernel       global L2 norm + clip coefficient of clip_grad_norm_ (adam_clip_kernel applies it)
 //   philox_*_kernel        torch.randn / randn_like replacement (model.py:57, inference.py:23,73,95)
 //   cast_bf16_kernel       fp32 -> bf16 operand copies
 //   latent_fwd_kernel      sigma = exp(.5 ls); z = mu + sigma*eps; KL partial sums  (model.py:56-57, lightning.py:115-117)
@@ -23,8 +24,22 @@ struct AdamArgs {
   float beta1, beta2, one_minus_beta1, one_minus_beta2, eps, weight_decay, grad_scale;
 };
 
-__device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, const AdamArgs& a) {
+// Gradient clipping inside the update (torch.nn.utils.clip_grad_norm_ / clip_grad_value_ as Lightning calls them before optimizer.step()),
+// before weight decay is added and before maximize negates.  CLIP_NORM: g_eff = g * fp32(grad_scale * coef), coef = min(max_norm /
+// (total_norm + 1e-6), 1) read from device memory (grad_norm_kernel) -- folded into grad_scale, so that the update is the unclipped
+// kernel's code with another scale (a separate multiply lets the compiler contract the moment updates differently, and coef = 1 would
+// then not reproduce the unclipped step bit for bit).  CLIP_VALUE: clamp(g * grad_scale, -v, v); NaN passes through as in torch.clamp.
+enum { CLIP_NONE = 0, CLIP_NORM = 1, CLIP_VALUE = 2 };
+template <int CLIP>
+__device__ __forceinline__ float clip_grad(float g, float c) {
+  if constexpr (CLIP == CLIP_VALUE) return g < -c ? -c : (g > c ? c : g);
+  return g;
+}
+
+template <int CLIP = CLIP_NONE>
+__device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, const AdamArgs& a, float clip = 0.f) {
   g *= a.grad_scale;
+  g = clip_grad<CLIP>(g, clip);
   if (a.weight_decay != 0.f) g = fmaf(a.weight_decay, p, g);
   m = m + (g - m) * a.one_minus_beta1;                    // exp_avg.lerp_(grad, 1-beta1)
   v = v * a.beta2 + a.one_minus_beta2 * g * g;            // mul_(beta2).addcmul_(g, g, 1-beta2)
@@ -32,8 +47,11 @@ __device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, 
   p = p - a.lr_step * (m / denom);                        // addcdiv_(m, denom, value=-step_size)
 }
 // amsgrad (torch/optim/adam.py: max_exp_avg_sqs = maximum(max_exp_avg_sqs, exp_avg_sq); denom from the maximum) / maximize (grad = -grad)
-__device__ __forceinline__ void adam_one_ex(float& p, float g, float& m, float& v, float& vmax, const AdamArgs& a, bool amsgrad, bool maximize) {
+template <int CLIP = CLIP_NONE>
+__device__ __forceinline__ void adam_one_ex(float& p, float g, float& m, float& v, float& vmax, const AdamArgs& a, bool amsgrad, bool maximize,
+                                            float clip = 0.f) {
   g *= a.grad_scale;
+  g = clip_grad<CLIP>(g, clip);
   if (maximize) g = -g;
   if (a.weight_decay != 0.f) g = fmaf(a.weight_decay, p, g);
   m = m + (g - m) * a.one_minus_beta1;
@@ -44,12 +62,14 @@ __device__ __forceinline__ void adam_one_ex(float& p, float g, float& m, float& 
   p = p - a.lr_step * (m / denom);
 }
 // the general form: one element per thread and trip (these configurations are not on any benchmarked path)
+template <int CLIP = CLIP_NONE>
 __device__ __forceinline__ void adam_ex_pass(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
-                                             float* __restrict__ vmax, int64_t n, const AdamArgs& a, int amsgrad, int maximize, bf16* __restrict__ shadow) {
+                                             float* __restrict__ vmax, int64_t n, const AdamArgs& a, int amsgrad, int maximize, bf16* __restrict__ shadow,
+                                             float clip = 0.f) {
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
     float pp = p[i], mm = m[i], vv = v[i], vx = amsgrad ? vmax[i] : 0.f;
-    adam_one_ex(pp, g[i], mm, vv, vx, a, amsgrad != 0, maximize != 0);
+    adam_one_ex<CLIP>(pp, g[i], mm, vv, vx, a, amsgrad != 0, maximize != 0, clip);
     p[i] = pp; m[i] = mm; v[i] = vv;
     if (amsgrad) vmax[i] = vx;
     if (shadow) shadow[i] = __float2bfloat16_rn(pp);
@@ -62,8 +82,9 @@ __global__ void __launch_bounds__(256) adam_ex_kernel(float* __restrict__ p, con
   adam_ex_pass(p, g, m, v, vmax, n, a, amsgrad, maximize, shadow);
 }
 
+template <int CLIP = CLIP_NONE>
 __device__ __forceinline__ void adam_pass(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, int64_t n,
-                                          const AdamArgs& a, bf16* __restrict__ shadow) {
+                                          const AdamArgs& a, bf16* __restrict__ shadow, float clip = 0.f) {
   const int64_t n4 = n >> 2;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
@@ -71,10 +92,10 @@ __device__ __forceinline__ void adam_pass(float* __restrict__ p, const float* __
     const float4 gg = __ldg(reinterpret_cast<const float4*>(g) + i);
     float4 mm = reinterpret_cast<float4*>(m)[i];
     float4 vv = reinterpret_cast<float4*>(v)[i];
-    adam_one(pp.x, gg.x, mm.x, vv.x, a);
-    adam_one(pp.y, gg.y, mm.y, vv.y, a);
-    adam_one(pp.z, gg.z, mm.z, vv.z, a);
-    adam_one(pp.w, gg.w, mm.w, vv.w, a);
+    adam_one<CLIP>(pp.x, gg.x, mm.x, vv.x, a, clip);
+    adam_one<CLIP>(pp.y, gg.y, mm.y, vv.y, a, clip);
+    adam_one<CLIP>(pp.z, gg.z, mm.z, vv.z, a, clip);
+    adam_one<CLIP>(pp.w, gg.w, mm.w, vv.w, a, clip);
     reinterpret_cast<float4*>(p)[i] = pp;
     reinterpret_cast<float4*>(m)[i] = mm;
     reinterpret_cast<float4*>(v)[i] = vv;
@@ -89,7 +110,7 @@ __device__ __forceinline__ void adam_pass(float* __restrict__ p, const float* __
   const int64_t t = (n4 << 2) + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t < n) {
     float pp = p[t], mm = m[t], vv = v[t];
-    adam_one(pp, g[t], mm, vv, a);
+    adam_one<CLIP>(pp, g[t], mm, vv, a, clip);
     p[t] = pp; m[t] = mm; v[t] = vv;
     if (shadow) shadow[t] = __float2bfloat16_rn(pp);
   }
@@ -123,6 +144,123 @@ __global__ void __launch_bounds__(256) adam_dc_kernel(float* __restrict__ p, con
   a.bc2_sqrt = s_bc2_sqrt;
   if constexpr (EX) adam_ex_pass(p, g, m, v, vmax, n, a, amsgrad, maximize, shadow);
   else adam_pass(p, g, m, v, n, a, shadow);
+}
+
+// The clipped forms of adam_kernel / adam_ex_kernel (EX) / adam_dc_kernel (DC): CLIP_NORM reads coef = *clip_coef after the grid dependency
+// (grad_norm_kernel wrote it) and runs the unclipped pass with grad_scale * coef, CLIP_VALUE clamps at clip_value.  The unclipped kernels
+// above stay as they are.
+template <bool DC, bool EX, int CLIP>
+__global__ void __launch_bounds__(256) adam_clip_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                                                        float* __restrict__ vmax, int64_t n, AdamArgs a, double beta1, double beta2,
+                                                        const double* __restrict__ lr, const int64_t* __restrict__ step_done, int amsgrad, int maximize,
+                                                        bf16* __restrict__ shadow, const float* __restrict__ clip_coef, float clip_value) {
+  PSVAE_GRID_DEP();
+  __shared__ float s_lr_step, s_bc2_sqrt, s_clip;
+  if (threadIdx.x == 0) {
+    if constexpr (DC) {
+      const double t = (double)(*step_done + 1);
+      const double bc1 = 1.0 - pow(beta1, t);
+      const double bc2 = 1.0 - pow(beta2, t);
+      s_lr_step = (float)(*lr / bc1);
+      s_bc2_sqrt = (float)sqrt(bc2);
+    }
+    s_clip = CLIP == CLIP_NORM ? a.grad_scale * *clip_coef : clip_value;
+  }
+  __syncthreads();
+  if constexpr (DC) {
+    a.lr_step = s_lr_step;
+    a.bc2_sqrt = s_bc2_sqrt;
+  }
+  const float c = s_clip;
+  if constexpr (CLIP == CLIP_NORM) {
+    a.grad_scale = c;
+    if constexpr (EX) adam_ex_pass(p, g, m, v, vmax, n, a, amsgrad, maximize, shadow);
+    else adam_pass(p, g, m, v, n, a, shadow);
+  } else {
+    if constexpr (EX) adam_ex_pass<CLIP>(p, g, m, v, vmax, n, a, amsgrad, maximize, shadow, c);
+    else adam_pass<CLIP>(p, g, m, v, n, a, shadow, c);
+  }
+}
+
+// Global L2 norm of g * scale over a list of [a, b) spans of the flat gradient buffer, and the clip coefficient of
+// torch.nn.utils.clip_grad_norm_: coef = min(max_norm / (total_norm + 1e-6), 1) in fp32.  Each thread sums its squares in fp64 in a fixed
+// order (grid-stride over the spans), the block reduces in a fixed tree and stores one fp64 partial; the last block to finish (ticket)
+// adds the partials in index order.  The grid is GRAD_NORM_BLOCKS whatever the device, so the result is bit-identical from run to run.
+// The last block resets the ticket to zero: the kernel can be replayed from a CUDA graph.
+constexpr int GRAD_NORM_MAX_SPANS = 16;
+constexpr int GRAD_NORM_BLOCKS = 296;
+struct GradNormSpans {
+  int64_t a[GRAD_NORM_MAX_SPANS], b[GRAD_NORM_MAX_SPANS];
+  int n;
+};
+__device__ __forceinline__ double block_sum_f64(double t, double* sm) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (lane == 0) sm[warp] = t;
+  __syncthreads();
+  double s = 0.0;
+  if (threadIdx.x == 0) {
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += sm[w];
+  }
+  return s;        // valid in thread 0
+}
+__global__ void __launch_bounds__(256) grad_norm_kernel(const float* __restrict__ g, GradNormSpans sp, float scale, float max_norm,
+                                                        double* __restrict__ part, unsigned* __restrict__ ticket, float* __restrict__ total_norm,
+                                                        float* __restrict__ coef) {
+  PSVAE_GRID_DEP();
+  __shared__ double sm[8];
+  __shared__ bool s_last;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  double t = 0.0;
+  for (int s = 0; s < sp.n; ++s)
+    for (int64_t i = sp.a[s] + tid; i < sp.b[s]; i += stride) {
+      const double x = (double)(__ldg(g + i) * scale);
+      t = fma(x, x, t);
+    }
+  const double bs = block_sum_f64(t, sm);
+  if (threadIdx.x == 0) {
+    part[blockIdx.x] = bs;
+    __threadfence();
+    s_last = atomicAdd(ticket, 1u) == gridDim.x - 1;
+  }
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  double u = 0.0;
+  for (int j = threadIdx.x; j < (int)gridDim.x; j += blockDim.x) u += __ldcg(part + j);
+  __syncthreads();          // sm is reused
+  const double tot = block_sum_f64(u, sm);
+  if (threadIdx.x == 0) {
+    const float tn = (float)sqrt(tot);
+    *total_norm = tn;
+    *coef = fminf(max_norm / (tn + 1e-6f), 1.0f);
+    *ticket = 0u;
+  }
+}
+
+// grads[i] += part[i]: the accumulating train step adds the gradient of this micro-batch (computed into a scratch buffer exactly as the
+// non-accumulating step computes it) to what the buffer holds -- one fp32 addition per element
+__global__ void __launch_bounds__(256) grad_accumulate_kernel(float* __restrict__ grads, const float* __restrict__ part, int64_t n) {
+  PSVAE_GRID_DEP();
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  const int64_t n4 = n >> 2;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
+    float4 a = reinterpret_cast<float4*>(grads)[i];
+    const float4 b = __ldg(reinterpret_cast<const float4*>(part) + i);
+    a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w;
+    reinterpret_cast<float4*>(grads)[i] = a;
+  }
+  const int64_t t = (n4 << 2) + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < n) grads[t] += part[t];
+}
+
+// rng_offset += d_rng, adam_step += d_step: the end of a micro-batch that does (d_step = 1) or does not (d_step = 0) step the optimiser
+__global__ void step_counters_advance_by_kernel(uint64_t* __restrict__ rng_offset, int64_t* __restrict__ adam_step, uint64_t d_rng, int64_t d_step) {
+  PSVAE_GRID_DEP();
+  *rng_offset += d_rng;
+  *adam_step += d_step;
 }
 
 // rng_offset += 1, adam_step += 1 at the end of a device-counter step (every reader of the block has finished: it is the last launch)

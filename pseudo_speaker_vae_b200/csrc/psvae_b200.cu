@@ -1663,6 +1663,102 @@ int psvae_step_counters_advance(psvae_step_counters* counters, void* stream) {
   return 0;
 }
 
+int psvae_step_counters_advance_by(psvae_step_counters* counters, uint64_t rng_delta, int64_t step_delta, void* stream) {
+  PSVAE_TRY(tc_device_check());
+  if (!counters) { set_error("counters must not be NULL"); return -1; }
+  launch_dep(step_counters_advance_by_kernel, dim3(1), dim3(1), 0, static_cast<cudaStream_t>(stream), &counters->rng_offset, &counters->adam_step,
+             rng_delta, step_delta);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("step_counters_advance_by_kernel");
+  return 0;
+}
+
+int psvae_grad_norm(const float* g, const int64_t* spans, int32_t n_spans, double grad_scale, double max_norm, float* total_norm, float* coef,
+                    void* scratch, int64_t scratch_bytes, void* stream) {
+  PSVAE_TRY(tc_device_check());
+  if (!g || !spans || !total_norm || !coef || !scratch) { set_error("g, spans, total_norm, coef and scratch must not be NULL"); return -1; }
+  if (n_spans < 1 || n_spans > GRAD_NORM_MAX_SPANS) { set_error("n_spans=%d must be in [1, %d]", (int)n_spans, GRAD_NORM_MAX_SPANS); return -2; }
+  if (scratch_bytes < PSVAE_GRAD_NORM_SCRATCH_BYTES || (reinterpret_cast<uintptr_t>(scratch) & 7) != 0) {
+    set_error("scratch must be 8-byte aligned and hold PSVAE_GRAD_NORM_SCRATCH_BYTES = %d bytes", PSVAE_GRAD_NORM_SCRATCH_BYTES);
+    return -2;
+  }
+  GradNormSpans sp{};
+  sp.n = n_spans;
+  for (int i = 0; i < n_spans; ++i) {
+    sp.a[i] = spans[2 * i];
+    sp.b[i] = spans[2 * i + 1];
+    if (sp.a[i] < 0 || sp.b[i] < sp.a[i]) { set_error("span %d = [%lld, %lld) is invalid", i, (long long)sp.a[i], (long long)sp.b[i]); return -2; }
+  }
+  double* part = static_cast<double*>(scratch);
+  unsigned* ticket = reinterpret_cast<unsigned*>(part + GRAD_NORM_BLOCKS);
+  launch_dep(grad_norm_kernel, dim3(GRAD_NORM_BLOCKS), dim3(256), 0, static_cast<cudaStream_t>(stream), g, sp, (float)grad_scale, (float)max_norm,
+             part, ticket, total_norm, coef);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("grad_norm_kernel");
+  return 0;
+}
+
+extern "C++" template <bool DC, bool EX>
+void launch_adam_clip(int clip_mode, int64_t n, cudaStream_t st, float* p, const float* g, float* m, float* v, float* vmax, const AdamArgs& a,
+                             double beta1, double beta2, const double* lr, const int64_t* step_done, int amsgrad, int maximize, bf16* sh,
+                             const float* coef, float clip_value) {
+  const dim3 grid(ew_grid(EX ? n : n / 4 + 1));
+  if (clip_mode == PSVAE_CLIP_NORM)
+    launch_dep(adam_clip_kernel<DC, EX, CLIP_NORM>, grid, dim3(256), 0, st, p, g, m, v, vmax, n, a, beta1, beta2, lr, step_done, amsgrad, maximize, sh,
+               coef, clip_value);
+  else
+    launch_dep(adam_clip_kernel<DC, EX, CLIP_VALUE>, grid, dim3(256), 0, st, p, g, m, v, vmax, n, a, beta1, beta2, lr, step_done, amsgrad, maximize, sh,
+               coef, clip_value);
+}
+
+int psvae_adam_step_clip(float* p, const float* g, float* m, float* v, float* vmax, int64_t n, double lr, int64_t step, const double* lr_dev,
+                         const psvae_step_counters* counters, double beta1, double beta2, double eps, double weight_decay, double grad_scale,
+                         int32_t amsgrad, int32_t maximize, int32_t clip_mode, const float* clip_coef, double clip_value, void* shadow_bf16,
+                         void* stream) {
+  const bool dc = counters != nullptr;
+  if (clip_mode == PSVAE_CLIP_NONE)
+    return dc ? psvae_adam_step_dc(p, g, m, v, vmax, n, lr_dev, counters, beta1, beta2, eps, weight_decay, grad_scale, amsgrad, maximize, shadow_bf16, stream)
+              : psvae_adam_step_ex(p, g, m, v, vmax, n, lr, beta1, beta2, eps, weight_decay, step, grad_scale, amsgrad, maximize, shadow_bf16, stream);
+  PSVAE_TRY(tc_device_check());
+  if (clip_mode != PSVAE_CLIP_NORM && clip_mode != PSVAE_CLIP_VALUE) { set_error("clip_mode=%d is not a PSVAE_CLIP_* value", (int)clip_mode); return -2; }
+  if (!p || !g || !m || !v || (amsgrad && !vmax) || (dc && !lr_dev) || (clip_mode == PSVAE_CLIP_NORM && !clip_coef)) {
+    set_error("p, g, m, v (vmax with amsgrad, lr_dev with counters, clip_coef with PSVAE_CLIP_NORM) must not be NULL");
+    return -1;
+  }
+  if (clip_mode == PSVAE_CLIP_VALUE && !(clip_value >= 0.0)) { set_error("clip_value=%g must be >= 0", clip_value); return -2; }
+  if (n <= 0) return 0;
+  if (!dc && step < 1) { set_error("step=%lld must be >= 1 (count after increment)", (long long)step); return -2; }
+  const bool ex = amsgrad || maximize;
+  if (!ex && ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v)) & 15) != 0) {
+    set_error("Adam buffers must be 16-byte aligned");
+    return -2;
+  }
+  AdamArgs a;
+  if (dc) {                  // formed on the device from *lr_dev and the step counter
+    a.lr_step = 0.f; a.bc2_sqrt = 1.f;
+  } else {
+    const double bc1 = 1.0 - pow(beta1, (double)step);
+    const double bc2 = 1.0 - pow(beta2, (double)step);
+    a.lr_step = (float)(lr / bc1);
+    a.bc2_sqrt = (float)sqrt(bc2);
+  }
+  a.beta1 = (float)beta1; a.beta2 = (float)beta2;
+  a.one_minus_beta1 = (float)(1.0 - beta1);
+  a.one_minus_beta2 = (float)(1.0 - beta2);
+  a.eps = (float)eps; a.weight_decay = (float)weight_decay; a.grad_scale = (float)grad_scale;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  bf16* sh = static_cast<bf16*>(shadow_bf16);
+  const int64_t* sd = dc ? &counters->adam_step : nullptr;
+  const float cv = (float)clip_value;
+  if (dc && ex) launch_adam_clip<true, true>(clip_mode, n, st, p, g, m, v, vmax, a, beta1, beta2, lr_dev, sd, amsgrad, maximize, sh, clip_coef, cv);
+  else if (dc) launch_adam_clip<true, false>(clip_mode, n, st, p, g, m, v, nullptr, a, beta1, beta2, lr_dev, sd, 0, 0, sh, clip_coef, cv);
+  else if (ex) launch_adam_clip<false, true>(clip_mode, n, st, p, g, m, v, vmax, a, beta1, beta2, nullptr, nullptr, amsgrad, maximize, sh, clip_coef, cv);
+  else launch_adam_clip<false, false>(clip_mode, n, st, p, g, m, v, nullptr, a, beta1, beta2, nullptr, nullptr, 0, 0, sh, clip_coef, cv);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("adam_clip_kernel");
+  return 0;
+}
+
 int psvae_philox_uint32(uint32_t* out, int64_t n, uint64_t seed, uint64_t offset, int64_t first_elem, void* stream) {
   PSVAE_TRY(tc_device_check());
   if (!out) { set_error("out is NULL"); return -1; }
@@ -1881,6 +1977,33 @@ int psvae_train_fwd_bwd_dc(const psvae_model_desc* desc, const float* params, co
   a.cons = cons; a.cons_params = cons_params; a.cons_y = cons_y; a.cons_w = cons_weight;
   a.offset_dev = counters ? &counters->rng_offset : nullptr;
   return precision == PSVAE_BF16 ? run_step<bf16>(a) : run_step<float>(a);
+}
+
+int psvae_train_fwd_bwd_acc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
+                            const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
+                            int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
+                            void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
+                            const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters, int32_t accumulate, float* grad_scratch) {
+  if (!accumulate || !compute_grads)
+    return psvae_train_fwd_bwd_dc(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss,
+                                  compute_grads, precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y,
+                                  cons_weight, counters);
+  PSVAE_TRY(check_desc(desc, precision));
+  if (!grads || !grad_scratch) { set_error("grads and grad_scratch must not be NULL when accumulate != 0"); return -1; }
+  if (((reinterpret_cast<uintptr_t>(grads) | reinterpret_cast<uintptr_t>(grad_scratch)) & 15) != 0) {
+    set_error("grads and grad_scratch must be 16-byte aligned");
+    return -2;
+  }
+  if (grads == grad_scratch) { set_error("grad_scratch must not be the gradient buffer"); return -2; }
+  // the step writes this micro-batch's gradient into the scratch exactly as the non-accumulating step writes `grads`; one pass then adds it
+  PSVAE_TRY(psvae_train_fwd_bwd_dc(desc, params, shadow_bf16, grad_scratch, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight,
+                                   use_cos_loss, compute_grads, precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons,
+                                   cons_params, cons_y, cons_weight, counters));
+  const int64_t n = desc->total_numel;
+  launch_dep(grad_accumulate_kernel, dim3(ew_grid(n / 4 + 1)), dim3(256), 0, static_cast<cudaStream_t>(stream), grads, (const float*)grad_scratch, n);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("grad_accumulate_kernel");
+  return 0;
 }
 
 int psvae_vae_backward(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype, const float* eps,

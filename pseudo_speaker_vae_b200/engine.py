@@ -455,14 +455,16 @@ class HotPath:
     def step(self, x: torch.Tensor, y=None, eps: Optional[torch.Tensor] = None, *, kl_weight: float = 1.0, clf_weight: float = 1.0,
              use_cos_loss: bool = False, compute_grads: bool = True, grads: Optional[torch.Tensor] = None, want_outputs: bool = False,
              consistency: Optional[nn.Module] = None, consistency_y: Optional[torch.Tensor] = None, consistency_weight: float = 1.0,
-             counters: Optional[torch.Tensor] = None):
+             counters: Optional[torch.Tensor] = None, accumulate: bool = False, grad_scratch: Optional[torch.Tensor] = None):
         """One fused forward(+backward).  Returns (losses[16] device tensor, flat grads or None, outputs or None).
 
         ``consistency``: a frozen ``EmbeddingClassifier`` whose ``consistency_weight * CE(consistency(x_hat), consistency_y)``
         joins the loss (lightning.py:100-108, 119-124).  losses slots: _lib.LOSS_*; nothing here synchronises with the host.
         ``counters``: a device ``psvae_step_counters`` block (int64 [_lib.COUNTER_SLOTS]); the Philox offset of the eps draw is then read
         from it on the device (``psvae_train_fwd_bwd_dc``), so that a CUDA graph of this call draws fresh noise at every replay.  The host
-        offset still advances as usual: it is the mirror the caller keeps the block in step with."""
+        offset still advances as usual: it is the mirror the caller keeps the block in step with.
+        ``accumulate``: ADD this batch's gradients to what ``grads`` holds (``psvae_train_fwd_bwd_acc``: they are computed into
+        ``grad_scratch``, a flat fp32 buffer of the arena's size, then added with one fp32 addition per element)."""
         dev = self._device()
         flat = self.arena.ensure()
         D, Lz = self.desc.input_dim, self.desc.latent_dim
@@ -508,9 +510,18 @@ class HotPath:
             if extra < 0:
                 raise ValueError(L.last_error())
             cons_args = (C.byref(cdesc), cflat.data_ptr(), cy.data_ptr(), float(consistency_weight))
-        if counters is not None:
-            if counters.device != dev or counters.dtype != torch.int64 or counters.numel() != L.COUNTER_SLOTS:
-                raise ValueError(f"counters must be an int64 [{L.COUNTER_SLOTS}] tensor on {dev}")
+        if counters is not None and (counters.device != dev or counters.dtype != torch.int64 or counters.numel() != L.COUNTER_SLOTS):
+            raise ValueError(f"counters must be an int64 [{L.COUNTER_SLOTS}] tensor on {dev}")
+        if accumulate and compute_grads:
+            if grads is None or grad_scratch is None or grad_scratch.device != dev or grad_scratch.dtype != torch.float32 \
+                    or grad_scratch.numel() < self.arena.numel or grad_scratch.data_ptr() == grads.data_ptr():
+                raise ValueError("an accumulating step needs `grads` and a separate fp32 `grad_scratch` of the arena's size on the same device")
+            with _on(dev):
+                ws = self._workspace(dev, B, mode, extra if consistency is not None else 0)
+                rc = L.lib().psvae_train_fwd_bwd_acc(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args, L.ptr(counters), 1,
+                                                     grad_scratch.data_ptr())
+            L.check(rc, "psvae_train_fwd_bwd_acc")
+        elif counters is not None:
             with _on(dev):
                 ws = self._workspace(dev, B, mode, extra if consistency is not None else 0)
                 rc = L.lib().psvae_train_fwd_bwd_dc(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args, counters.data_ptr())

@@ -21,6 +21,11 @@ The host keeps its usual view of the run -- ``hot_path.offset``, ``optimizer.sta
 mark -- by counting replays (no read-back), so eager steps, ``state_dict()`` and checkpoints in between see the right values; whenever
 those host values differ from what the device block holds (a scheduler step, ``load_state_dict``, an eager step, ``manual_seed``) the
 host values are written to the block before the next replay.
+
+With the trainer's ``accumulate_grad_batches = k`` each call is one micro-batch, and up to three graphs are captured, each on first use:
+the first micro-batch of a window (writes the gradient buffer), a middle one (adds to it) and the last one (adds, then all-reduce, norm
+clipping, Adam).  With k = 1 there is one graph, as without the option.  Every replay advances the Philox offset; only the last one
+advances the Adam step.  ``flush=True`` ends the window early, as it does for ``DataParallelTrainer.train_step``.
 """
 from __future__ import annotations
 
@@ -50,6 +55,7 @@ class GraphedTrainStep:
         self.lrs = torch.zeros(n_groups, dtype=torch.float64, device=self.device)
         self.graph: Optional[torch.cuda.CUDAGraph] = None
         self.losses: Optional[torch.Tensor] = None  # the graph's static output
+        self._graphs: Dict[Tuple[bool, bool], Tuple[torch.cuda.CUDAGraph, torch.Tensor]] = {}   # (accumulate, step) -> (graph, losses)
         self.replays = 0
         self.pdl: Optional[int] = None             # 1: captured with programmatic dependent launch; 0: captured without it
         self.capture_error: Optional[str] = None   # why a first capture attempt failed (kept when a fallback capture succeeded)
@@ -77,15 +83,17 @@ class GraphedTrainStep:
         self.lrs.copy_(torch.tensor(lrs, dtype=torch.float64))
         self._mirror = vals
 
-    def _advance_mirrors(self) -> None:
-        """What one replay did, on the host: the eager step's _rng() and FusedAdam.step() bookkeeping."""
+    def _advance_mirrors(self, step: bool = True) -> None:
+        """What one replay did, on the host: the eager step's _rng() and (``step``) FusedAdam.step() bookkeeping."""
         opt, arena = self.optimizer, self.hot.arena
         self.hot.offset += 1
-        for g in opt.param_groups:
-            opt.state[g["params"][0]]["step"] += 1       # one tensor shared by the group's parameters (FusedAdam._bind_state)
-        arena.epoch += 1
-        if arena.shadow is not None:
-            arena.mark_shadow_current()
+        if step:
+            for g in opt.param_groups:
+                opt.state[g["params"][0]]["step"] += 1       # one tensor shared by the group's parameters (FusedAdam._bind_state)
+            arena.epoch += 1
+            if arena.shadow is not None:
+                arena.mark_shadow_current()
+        self.trainer._end_micro_batch(step)
         self.replays += 1
         self._mirror = self._host_values()
 
@@ -99,8 +107,10 @@ class GraphedTrainStep:
                        for g in opt.param_groups)
         bufs = (hot.arena.flat.data_ptr(), L.ptr(hot.arena.shadow), opt._m.data_ptr(), opt._v.data_ptr(), L.ptr(opt._vmax),
                 tr._views_of.data_ptr() if tr._views_of is not None else None, cflat)
+        knobs = (tr.accumulate_grad_batches, tr.gradient_clip_val, tr.gradient_clip_algorithm, opt.clip_mode, opt.clip_value, L.ptr(opt.clip_coef),
+                 L.ptr(tr._acc_scratch), L.ptr(tr._norm_scratch))
         return (hot.seed, hot.row0, hot.precision, m.kl_loss_weight, m.classifier_loss_weight, m.use_cos_loss, m.consitency_loss_weight,
-                id(cons), L.OPTIONS_EPOCH, opt.grad_scale, groups, bufs)
+                id(cons), L.OPTIONS_EPOCH, opt.grad_scale, groups, bufs, knobs)
 
     # ---- capture --------------------------------------------------------------------------------
     def _check_supported(self) -> None:
@@ -113,18 +123,24 @@ class GraphedTrainStep:
         if tr._views_of is None or self.hot.arena.flat_grad() is None:
             raise NotImplementedError("a graphed train step reads the gradients from the trainer's flat gradient buffer")
 
-    def _body(self, kind: Optional[str]) -> torch.Tensor:
-        st = self._static
-        losses, gflat = self.trainer._fwd_bwd(st["x"], st["y"], None, counters=self.counters[0])
-        self.trainer._all_reduce(gflat, kind)
-        self.optimizer._update(self.counters, self.lrs)
+    def _body(self, kind: Optional[str], phase: Tuple[bool, bool] = (False, True)) -> torch.Tensor:
+        st, tr = self._static, self.trainer
+        accumulate, step = phase
+        losses, gflat = tr._fwd_bwd(st["x"], st["y"], None, counters=self.counters[0], accumulate=accumulate)
+        if step:
+            tr._all_reduce(gflat, kind)
+            tr._clip_norm(gflat)
+            self.optimizer._update(self.counters, self.lrs)
         lib, stream = L.lib(), _stream_ptr(self.device)
         with _on(self.device):
             for gi in range(self.counters.shape[0]):
-                L.check(lib.psvae_step_counters_advance(self.counters[gi].data_ptr(), stream), "psvae_step_counters_advance")
+                if phase == (False, True):
+                    L.check(lib.psvae_step_counters_advance(self.counters[gi].data_ptr(), stream), "psvae_step_counters_advance")
+                else:
+                    L.check(lib.psvae_step_counters_advance_by(self.counters[gi].data_ptr(), 1, int(step), stream), "psvae_step_counters_advance_by")
         return losses
 
-    def _try_capture(self, kind: Optional[str], pdl: int) -> Tuple[Optional[torch.cuda.CUDAGraph], Optional[torch.Tensor], Optional[BaseException]]:
+    def _try_capture(self, kind: Optional[str], pdl: int, phase: Tuple[bool, bool] = (False, True)) -> Tuple[Optional[torch.cuda.CUDAGraph], Optional[torch.Tensor], Optional[BaseException]]:
         off0 = self.hot.offset
         pdl0 = L.get_option("pdl")
         g = torch.cuda.CUDAGraph()
@@ -132,7 +148,7 @@ class GraphedTrainStep:
             if pdl != pdl0:
                 L.set_option("pdl", pdl)
             with torch.cuda.graph(g, capture_error_mode="thread_local"):
-                losses = self._body(kind)
+                losses = self._body(kind, phase)
             return g, losses, None
         except Exception as e:  # noqa: BLE001 -- reported by the caller, which may retry with another configuration
             return None, None, e
@@ -149,14 +165,20 @@ class GraphedTrainStep:
             return tuple(sorted((k, tuple(v.shape)) for k, v in y.items()))
         return tuple(y.shape)
 
-    def _capture(self, x: torch.Tensor, y) -> None:
+    def _capture(self, x: torch.Tensor, y, phase: Tuple[bool, bool] = (False, True)) -> None:
+        """Capture the graph of one window phase (accumulate, step).  A new static input layout drops the graphs of the other phases."""
         self._check_supported()
         tr, dev, hot = self.trainer, self.device, self.hot
-        self._static = {"x": torch.empty(self.rows, x.shape[1], dtype=self.x_dtype or x.dtype, device=dev), "ysig": self._label_sig(y)}
-        if isinstance(y, dict):
-            self._static["y"] = {k: torch.empty(v.shape, dtype=torch.int64, device=dev) for k, v in y.items()}
-        else:
-            self._static["y"] = None if y is None else torch.empty(tuple(y.shape), dtype=torch.int64, device=dev)
+        tr._knob_buffers(dev)
+        self.optimizer._moments()          # a window's first graphs may be captured before any Adam step has allocated the moments
+        if not self._graphs or self._capture_key() != self._key or self._label_sig(y) != self._static.get("ysig") \
+                or x.shape[1] != self._static["x"].shape[1]:
+            self._graphs = {}
+            self._static = {"x": torch.empty(self.rows, x.shape[1], dtype=self.x_dtype or x.dtype, device=dev), "ysig": self._label_sig(y)}
+            if isinstance(y, dict):
+                self._static["y"] = {k: torch.empty(v.shape, dtype=torch.int64, device=dev) for k, v in y.items()}
+            else:
+                self._static["y"] = None if y is None else torch.empty(tuple(y.shape), dtype=torch.int64, device=dev)
         self._copy_in(x, y)
         hot._shadow()                      # the graph contains no shadow refresh: the copy must be current before capture
         self.graph = self.losses = None
@@ -169,7 +191,7 @@ class GraphedTrainStep:
         attempts = [(k, pdl0) for k in kinds] + ([(k, 0) for k in kinds] if pdl0 else [])
         first_err = err = None
         for kind, pdl in attempts:
-            g, losses, err = self._try_capture(kind, pdl)
+            g, losses, err = self._try_capture(kind, pdl, phase)
             if tr.world_size > 1 and not tr.local_only:
                 # every rank must replay the same collective
                 ok = torch.tensor([0.0 if err is not None else 1.0], device=dev)
@@ -187,9 +209,10 @@ class GraphedTrainStep:
             self.capture_error = repr(first_err)
             warnings.warn(f"GraphedTrainStep: the first capture attempt failed ({first_err!r}); captured with all-reduce "
                           f"{self.allreduce_kind!r}, pdl={self.pdl}", RuntimeWarning)
+        self._graphs[phase] = (self.graph, self.losses)
         # buffers the graph writes that HotPath may replace later (a larger eager batch, a forward or decode grows the cached workspace):
         # holding them keeps the captured pointers valid; the eager path then works in the new buffer
-        self._static["ws"] = hot._ws.get(dev)
+        self._static.setdefault("ws", []).append(hot._ws.get(dev))
         cons = getattr(tr.module, "consistency_classifier", None)
         self._static["cons_flat"] = cons.flat_params(dev)[1] if cons is not None else None
         self._key = self._capture_key()
@@ -204,11 +227,11 @@ class GraphedTrainStep:
             st["y"].copy_(y)
 
     # ---- the step -------------------------------------------------------------------------------
-    def __call__(self, x: torch.Tensor, y=None) -> torch.Tensor:
-        """One optimiser step on this rank's shard; returns the device tensor of local loss scalars (for a replay: the graph's static
-        output, overwritten by the next call)."""
+    def __call__(self, x: torch.Tensor, y=None, *, flush: bool = False) -> torch.Tensor:
+        """One micro-batch (one optimiser step without accumulation) on this rank's shard; returns the device tensor of local loss
+        scalars (for a replay: the graph's static output, overwritten by the next call).  ``flush``: see DataParallelTrainer.train_step."""
         if x.dim() != 2 or x.shape[0] != self.rows:
-            return self.trainer.train_step(x, y)
+            return self.trainer.train_step(x, y, flush=flush)
         static_x = self._static.get("x")
         want = self.x_dtype or (static_x.dtype if static_x is not None else x.dtype)
         if x.dtype != want:
@@ -216,14 +239,16 @@ class GraphedTrainStep:
                              "what the step computes (x_dtype)")
         if not self._warm:
             self._warm = True
-            return self.trainer.train_step(x, y)
-        if (self.graph is None or self._capture_key() != self._key or self._label_sig(y) != self._static["ysig"]
+            return self.trainer.train_step(x, y, flush=flush)
+        phase = self.trainer._window_phase(flush)
+        if (phase not in self._graphs or self._capture_key() != self._key or self._label_sig(y) != self._static["ysig"]
                 or x.shape[1] != static_x.shape[1]):
-            self._capture(x, y)
+            self._capture(x, y, phase)
         else:
             self._copy_in(x, y)
             self.hot._shadow()             # refreshed outside the graph if something rewrote the parameters out of band
+        self.graph, self.losses = self._graphs[phase]
         self._sync_device()
         self.graph.replay()
-        self._advance_mirrors()
+        self._advance_mirrors(phase[1])
         return self.losses

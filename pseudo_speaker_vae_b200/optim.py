@@ -11,6 +11,12 @@ In bf16 mode the same pass also refreshes the bf16 operand copy the tcgen05 GEMM
 ``amsgrad`` (state key ``max_exp_avg_sq``, a third flat buffer) and ``maximize`` -- both reachable through
 ``Adam(self.parameters(), **self.hparams["optimizer"])`` -- take the general kernel (``psvae_adam_step_ex``);
 ``capturable`` / ``differentiable`` are not on the reference's path and raise.
+
+Gradient clipping (Lightning's ``gradient_clip_val`` / ``gradient_clip_algorithm``) happens inside the same pass when ``clip_mode`` is set
+(``DataParallelTrainer`` sets it, as it sets ``grad_scale``): ``"norm"`` scales ``g`` by ``grad_scale * clip_coef`` (``clip_coef``: a device
+scalar written by ``psvae_grad_norm``), ``"value"`` clamps ``g * grad_scale`` at ``clip_value`` -- before weight decay and maximize, where
+torch clips.  The ``.grad``
+tensors themselves are not rewritten.
 """
 from __future__ import annotations
 
@@ -45,6 +51,9 @@ class FusedAdam(torch.optim.Optimizer):
             raise ValueError("FusedAdam needs the parameter arena (use PseudoSpeakerVAE.configure_optimizers or HotPath.arena)")
         self.arena = arena
         self.grad_scale = 1.0          # 1 / world_size after a SUM all-reduce
+        self.clip_mode = "none"        # "none" | "norm" (g * (grad_scale * clip_coef)) | "value" (clamp(g * grad_scale, -clip_value, clip_value))
+        self.clip_coef: Optional[torch.Tensor] = None   # device fp32 scalar written by psvae_grad_norm
+        self.clip_value = 0.0
         self._m: Optional[torch.Tensor] = None
         self._v: Optional[torch.Tensor] = None
         self._vmax: Optional[torch.Tensor] = None      # amsgrad: running maximum of exp_avg_sq
@@ -129,6 +138,9 @@ class FusedAdam(torch.optim.Optimizer):
         learning rate per group, read on the device (``psvae_adam_step_dc``).  That form moves no host state: the caller advances the step
         counts, the arena epoch and the shadow mark, and the device block, itself."""
         dc = counters is not None
+        clip = {"none": L.CLIP_NONE, "norm": L.CLIP_NORM, "value": L.CLIP_VALUE}[self.clip_mode]
+        if clip == L.CLIP_NORM and (self.clip_coef is None or self.clip_coef.dtype != torch.float32):
+            raise ValueError("clip_mode 'norm' needs clip_coef, a device fp32 scalar")
         flat = self.arena.ensure()
         dev = flat.device
         if dev.type != "cuda":
@@ -161,7 +173,13 @@ class FusedAdam(torch.optim.Optimizer):
                     shadow = self.arena.shadow.data_ptr() + 2 * a
                 vmax = self._vmax.data_ptr() + 4 * a if group["amsgrad"] else None
                 with _on(dev):
-                    if dc:
+                    if clip != L.CLIP_NONE:
+                        rc = lib.psvae_adam_step_clip(flat.data_ptr() + 4 * a, gflat.data_ptr() + 4 * a, m.data_ptr() + 4 * a, v.data_ptr() + 4 * a, vmax,
+                                                      b - a, float(group["lr"]), step, L.ptr(lrs[gi]) if dc else None,
+                                                      counters[gi].data_ptr() if dc else None, float(beta1), float(beta2), float(group["eps"]),
+                                                      float(group["weight_decay"]), float(self.grad_scale), int(bool(group["amsgrad"])),
+                                                      int(bool(group["maximize"])), clip, L.ptr(self.clip_coef), float(self.clip_value), shadow, stream)
+                    elif dc:
                         rc = lib.psvae_adam_step_dc(flat.data_ptr() + 4 * a, gflat.data_ptr() + 4 * a, m.data_ptr() + 4 * a, v.data_ptr() + 4 * a, vmax, b - a,
                                                     lrs[gi].data_ptr(), counters[gi].data_ptr(), float(beta1), float(beta2), float(group["eps"]),
                                                     float(group["weight_decay"]), float(self.grad_scale), int(bool(group["amsgrad"])),

@@ -14,11 +14,14 @@ gloo in the CPU tests).  This is what ``Trainer(strategy=DDPStrategy(...))`` doe
 """
 from __future__ import annotations
 
+import ctypes as C
 import os
 from typing import Optional, Tuple
 
 import torch
 import torch.distributed as dist
+
+from . import _lib as L
 
 DEFAULT_BUCKET_BYTES = 25 * 1024 * 1024
 
@@ -132,11 +135,43 @@ class SymmetricAllReduce:
 
 class DataParallelTrainer:
     """The per-batch body of the reference's fit loop (SURVEY 3.1) as three device-side calls:
-    fused fwd+bwd  ->  bucketed all-reduce  ->  fused Adam.  Nothing in ``train_step`` synchronises with the host."""
+    fused fwd+bwd  ->  bucketed all-reduce  ->  fused Adam.  Nothing in ``train_step`` synchronises with the host.
 
-    def __init__(self, module, optimizer=None, bucket_bytes: int = DEFAULT_BUCKET_BYTES, group=None, local_only: bool = False):
+    Two ``Trainer`` options of the reference change what one optimiser step computes; they take Lightning's names, so the keys of
+    ``config["trainer"]`` can be passed straight through:
+
+    * ``accumulate_grad_batches = k``: each ``train_step`` is one micro-batch.  The first of a window writes the gradient buffer, the
+      others add to it; the k-th call (or one with ``flush=True``, Lightning's last batch of an epoch) runs the all-reduce, the clipping
+      and Adam, with ``grad_scale = 1 / (k * world)`` -- Lightning's fixed ``loss / k``, also for a flushed partial window.  Every call
+      draws its own eps (one Philox offset), as every ``training_step`` does.
+    * ``gradient_clip_val`` / ``gradient_clip_algorithm``: ``"norm"`` is ``clip_grad_norm_(params, val)`` on the averaged gradient (the
+      global L2 norm is computed on the device, ``psvae_grad_norm``, and the coefficient is applied inside the Adam pass); ``"value"`` is
+      ``clip_grad_value_``.  None or 0 turns clipping off.  ``grad_norm`` holds the pre-clip total norm of the last optimiser step as a
+      device fp32 scalar (norm clipping only; nothing reads it back).
+
+    Unlike Lightning, ``p.grad`` keeps the unclipped, all-reduced SUM of the window's micro-batch gradients: the averaging (``1 / (k *
+    world)``) and the clipping are applied inside the Adam pass, not to the ``.grad`` tensors."""
+
+    def __init__(self, module, optimizer=None, bucket_bytes: int = DEFAULT_BUCKET_BYTES, group=None, local_only: bool = False, *,
+                 accumulate_grad_batches: int = 1, gradient_clip_val: Optional[float] = None, gradient_clip_algorithm: Optional[str] = "norm"):
         """``local_only``: a trainer that never talks to the other ranks even inside an initialised process group (the single-process
         twin ``verify_data_parallel_step`` compares the data-parallel run with)."""
+        if isinstance(accumulate_grad_batches, bool) or not isinstance(accumulate_grad_batches, int) or accumulate_grad_batches < 1:
+            raise ValueError(f"accumulate_grad_batches must be an int >= 1, got {accumulate_grad_batches!r}")
+        algo = "norm" if gradient_clip_algorithm is None else gradient_clip_algorithm
+        if algo not in ("norm", "value"):
+            raise ValueError(f"gradient_clip_algorithm must be 'norm' or 'value', got {gradient_clip_algorithm!r}")
+        clip = 0.0 if gradient_clip_val is None else float(gradient_clip_val)
+        if not clip >= 0.0:
+            raise ValueError(f"gradient_clip_val must be >= 0 (None or 0 turns clipping off), got {gradient_clip_val!r}")
+        self.accumulate_grad_batches = accumulate_grad_batches
+        self.gradient_clip_val = clip if clip > 0.0 else None
+        self.gradient_clip_algorithm = algo
+        self.grad_norm: Optional[torch.Tensor] = None     # device fp32 scalar: pre-clip total norm of the last optimiser step
+        self._clip_coef: Optional[torch.Tensor] = None
+        self._norm_scratch: Optional[torch.Tensor] = None
+        self._acc_scratch: Optional[torch.Tensor] = None
+        self._micro = 0                                   # micro-batches of the current accumulation window already run
         self.module = module
         self.hot = module.hot_path
         self.group = group
@@ -146,7 +181,10 @@ class DataParallelTrainer:
         if optimizer is None:
             optimizer = module.configure_optimizers()["optimizer"]
         self.optimizer = optimizer
-        self.optimizer.grad_scale = 1.0 / self.world_size
+        self.optimizer.grad_scale = 1.0 / (self.accumulate_grad_batches * self.world_size)
+        if self.gradient_clip_val is not None:
+            self.optimizer.clip_mode = self.gradient_clip_algorithm
+            self.optimizer.clip_value = self.gradient_clip_val
         if not self.local_only:
             broadcast_parameters(self.hot.arena.ensure(), 0, group)
         self.hot.arena.epoch += 1          # the bf16 operand copy must follow the broadcast values
@@ -179,26 +217,78 @@ class DataParallelTrainer:
         self.hot.row0 = row0
         return row0, rows
 
-    def train_step(self, x_local: torch.Tensor, y_local=None, eps_local: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """One optimiser step on this rank's shard.  Returns the device tensor of local loss scalars."""
-        losses, gflat = self._fwd_bwd(x_local, y_local, eps_local)
-        self._all_reduce(gflat)
+    def train_step(self, x_local: torch.Tensor, y_local=None, eps_local: Optional[torch.Tensor] = None, *, flush: bool = False) -> torch.Tensor:
+        """One micro-batch on this rank's shard (with ``accumulate_grad_batches = 1``: one optimiser step).  Returns the device tensor of
+        this micro-batch's local loss scalars.  ``flush``: end the accumulation window here (the last batch of an epoch)."""
+        accumulate, step = self._window_phase(flush)
+        losses, gflat = self._fwd_bwd(x_local, y_local, eps_local, accumulate=accumulate)
         if self._views_of is not gflat:        # bind .grad views once; the same flat buffer is reused every step
             for (p, _), v in zip(self.hot.arena.entries, self.hot.arena.grad_views(gflat)):
                 p.grad = v if p.requires_grad else None
             self._views_of = gflat
-        self.optimizer.step()
+        if step:
+            self._all_reduce(gflat)
+            self._clip_norm(gflat)
+            self.optimizer.step()
+        self._end_micro_batch(step)
         return losses
 
-    def _fwd_bwd(self, x_local: torch.Tensor, y_local=None, eps_local: Optional[torch.Tensor] = None, counters: Optional[torch.Tensor] = None):
-        """The fused forward + backward of train_step into the gradient buffer the all-reduce reads.  ``counters``: see HotPath.step."""
+    def _window_phase(self, flush: bool = False) -> Tuple[bool, bool]:
+        """(accumulate, step) of the next micro-batch: does it add to the gradient buffer, does it end the window."""
+        return self._micro > 0, bool(flush) or self._micro + 1 >= self.accumulate_grad_batches
+
+    def _end_micro_batch(self, step: bool) -> None:
+        self._micro = 0 if step else self._micro + 1
+
+    def _knob_buffers(self, dev: torch.device) -> None:
+        """The device buffers the options need, allocated before any capture (a CUDA graph must not own them)."""
+        n = self.hot.arena.numel
+        if self.accumulate_grad_batches > 1 and (self._acc_scratch is None or self._acc_scratch.device != dev):
+            self._acc_scratch = torch.empty(n, dtype=torch.float32, device=dev)
+        if self.gradient_clip_val is not None and self.gradient_clip_algorithm == "norm" and (self._norm_scratch is None or self._norm_scratch.device != dev):
+            self._norm_scratch = torch.zeros(L.GRAD_NORM_SCRATCH_BYTES // 8, dtype=torch.float64, device=dev)
+            self.grad_norm = torch.zeros((), dtype=torch.float32, device=dev)
+            self._clip_coef = torch.ones((), dtype=torch.float32, device=dev)
+            self.optimizer.clip_coef = self._clip_coef
+
+    def _norm_spans(self):
+        """The merged [a, b) spans the optimiser's update covers (FusedAdam._ranges over every group), as psvae_grad_norm takes them."""
+        opt = self.optimizer
+        spans = [(opt._offsets[id(p)], opt._offsets[id(p)] + p.numel()) for g in opt.param_groups for p in g["params"] if p.grad is not None]
+        merged = opt._ranges(spans)
+        if len(merged) > L.GRAD_NORM_MAX_SPANS:
+            raise NotImplementedError(f"norm clipping covers at most {L.GRAD_NORM_MAX_SPANS} disjoint gradient spans, got {len(merged)}")
+        return merged
+
+    def _clip_norm(self, gflat: torch.Tensor) -> None:
+        """Norm clipping: total norm and clip coefficient of the gradient the Adam pass is about to read (no host synchronisation)."""
+        if self.gradient_clip_val is None or self.gradient_clip_algorithm != "norm":
+            return
+        from .engine import _on, _stream_ptr
+        dev = gflat.device
+        self._knob_buffers(dev)
+        spans = self._norm_spans()
+        flat = (C.c_int64 * (2 * len(spans)))(*[v for ab in spans for v in ab])
+        with _on(dev):
+            rc = L.lib().psvae_grad_norm(gflat.data_ptr(), flat, len(spans), float(self.optimizer.grad_scale), float(self.gradient_clip_val),
+                                         self.grad_norm.data_ptr(), self._clip_coef.data_ptr(), self._norm_scratch.data_ptr(),
+                                         self._norm_scratch.numel() * 8, _stream_ptr(dev))
+        L.check(rc, "psvae_grad_norm")
+
+    def _fwd_bwd(self, x_local: torch.Tensor, y_local=None, eps_local: Optional[torch.Tensor] = None, counters: Optional[torch.Tensor] = None,
+                 accumulate: bool = False):
+        """The fused forward + backward of train_step into the gradient buffer the all-reduce reads.  ``counters``: see HotPath.step.
+        ``accumulate``: add to the buffer instead of overwriting it (a later micro-batch of an accumulation window)."""
         m, hot = self.module, self.hot
         gflat = self.symm.buf if self.symm is not None else (hot.arena.stage_buffer() if self._views_of is None else self._views_of)
         cons = getattr(m, "consistency_classifier", None)
+        if accumulate:
+            self._knob_buffers(gflat.device)
         losses, gflat, _ = hot.step(x_local, y_local if m.classifier is not None else None, eps_local, kl_weight=m.kl_loss_weight,
                                     clf_weight=m.classifier_loss_weight, use_cos_loss=m.use_cos_loss, compute_grads=True, grads=gflat,
                                     consistency=cons, consistency_y=y_local if cons is not None else None,
-                                    consistency_weight=m.consitency_loss_weight, counters=counters)
+                                    consistency_weight=m.consitency_loss_weight, counters=counters, accumulate=accumulate,
+                                    grad_scratch=self._acc_scratch if accumulate else None)
         return losses, gflat
 
     def _all_reduce(self, gflat: torch.Tensor, kind: Optional[str] = None) -> None:
