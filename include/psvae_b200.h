@@ -118,6 +118,9 @@ int psvae_model_desc_init(psvae_model_desc* desc, int32_t input_dim, int32_t lat
 #define PSVAE_MODE_TRAIN 0
 #define PSVAE_MODE_FORWARD 1
 #define PSVAE_MODE_DECODE 2
+/* the classifier-only train step (psvae_train_fwd_bwd_scoped with PSVAE_GRAD_CLASSIFIER): the forward buffers plus the classifier's
+ * backward buffers -- none of the VAE backward's */
+#define PSVAE_MODE_TRAIN_CLASSIFIER 3
 int64_t psvae_workspace_bytes(const psvae_model_desc* desc, int64_t rows, int32_t precision, int32_t mode);
 /* bytes of the bf16 shadow copy of the parameters (PSVAE_BF16 only) */
 int64_t psvae_shadow_bytes(const psvae_model_desc* desc);
@@ -266,6 +269,21 @@ int psvae_train_fwd_bwd_acc(const psvae_model_desc* desc, const float* params, c
                             float* mu, float* log_sigma, float* losses, void* workspace, int64_t workspace_bytes, void* stream,
                             const psvae_consistency_desc* cons, const float* cons_params, const int64_t* cons_y, float cons_weight,
                             const psvae_step_counters* counters, int32_t accumulate, float* grad_scratch);
+/* ---- gradient scope (additive to ABI 5).  PSVAE_GRAD_ALL: every parameter, exactly psvae_train_fwd_bwd_acc.  PSVAE_GRAD_CLASSIFIER: the
+ * second stage of a two-stage run (frozen VAE, lightning.py freeze_vae): the full forward and every loss term, as the full step computes
+ * them, but only the latent classifier's gradients -- no VAE backward.  Only the classifier span of `grads`, [vae_numel, total_numel),
+ * is written (cleared, then written; with accumulate != 0: grads[i] += grad_scratch[i] over that span only); every element outside it
+ * keeps its value.  workspace >= psvae_workspace_bytes(desc, rows, precision, PSVAE_MODE_TRAIN_CLASSIFIER) (+
+ * psvae_consistency_workspace_bytes(cons, rows, PSVAE_MODE_FORWARD) with a consistency term).  A model without a classifier, or an
+ * unknown scope, is an argument error. */
+#define PSVAE_GRAD_ALL 0
+#define PSVAE_GRAD_CLASSIFIER 1
+int psvae_train_fwd_bwd_scoped(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x,
+                               int32_t x_dtype, const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows,
+                               float kl_weight, float clf_weight, int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat,
+                               float* mu, float* log_sigma, float* losses, void* workspace, int64_t workspace_bytes, void* stream,
+                               const psvae_consistency_desc* cons, const float* cons_params, const int64_t* cons_y, float cons_weight,
+                               const psvae_step_counters* counters, int32_t accumulate, float* grad_scratch, int32_t grad_scope);
 #define PSVAE_GRAD_NORM_MAX_SPANS 16
 #define PSVAE_GRAD_NORM_SCRATCH_BYTES 4096
 /* total_norm = || g * grad_scale ||_2 over the n_spans [a, b) spans (host int64 array {a0, b0, a1, b1, ...}) of the flat gradient, and

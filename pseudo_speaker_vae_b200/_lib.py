@@ -20,7 +20,9 @@ MAX_CLF_HEADS = 4
 NUM_LOSSES = 16
 FP32, BF16 = 0, 1
 X_F32, X_BF16 = 0, 1
-MODE_TRAIN, MODE_FORWARD, MODE_DECODE = 0, 1, 2
+MODE_TRAIN, MODE_FORWARD, MODE_DECODE, MODE_TRAIN_CLASSIFIER = 0, 1, 2, 3
+#: psvae_train_fwd_bwd_scoped: which parameters get gradients
+GRAD_ALL, GRAD_CLASSIFIER = 0, 1
 ACTIVATIONS = {"relu": 0, "tanh": 1, "sigmoid": 2, "leaky_relu": 3}
 LOSS_TOTAL, LOSS_RECON, LOSS_KL, LOSS_CLF, LOSS_CLF_HEAD0, LOSS_ACC_HEAD0 = 0, 1, 2, 3, 4, 8
 LOSS_CONS, LOSS_CONS_ACC = 12, 13
@@ -34,6 +36,7 @@ EXPORTS = [
     "psvae_consistency_forward", "psvae_train_fwd_bwd_consistency", "psvae_vae_backward", "psvae_gather_rows",
     "psvae_embedding_classifier_workspace_bytes", "psvae_embedding_classifier_step", "psvae_train_fwd_bwd_dc", "psvae_adam_step_dc",
     "psvae_step_counters_advance", "psvae_train_fwd_bwd_acc", "psvae_grad_norm", "psvae_adam_step_clip", "psvae_step_counters_advance_by",
+    "psvae_train_fwd_bwd_scoped",
 ]
 
 #: int64 slots of ``psvae_step_counters`` (a device tensor of COUNTER_SLOTS int64)
@@ -139,6 +142,9 @@ def _declare(l: C.CDLL) -> None:
                                            DBL, VP, VP]
         l.psvae_step_counters_advance_by.restype = C.c_int
         l.psvae_step_counters_advance_by.argtypes = [VP, U64, I64, VP]
+    if hasattr(l, "psvae_train_fwd_bwd_scoped"):
+        l.psvae_train_fwd_bwd_scoped.restype = C.c_int
+        l.psvae_train_fwd_bwd_scoped.argtypes = l.psvae_train_fwd_bwd_acc.argtypes + [I32]
     l.psvae_langevin.restype = C.c_int
     l.psvae_langevin.argtypes = [D, VP, VP, I64, P(I32), F, I32, F, U64, U64, I64, I32, VP, VP, VP, F, F, VP, VP, VP]
     l.psvae_gemm_bf16.restype = C.c_int

@@ -1214,6 +1214,71 @@ __global__ void __launch_bounds__(256, 3) latent_bwd_clf_kernel(const float* __r
   }
 }
 
+// The classifier's own gradients from g_rows alone (classifier-only train step, fast mode, fused encoder head): the fused head leaves
+// d loss / d logits per row in g_rows, and with the VAE frozen there is no latent backward to fold them into.
+//   dW[c][k] += sum_r g[r][c] mu[r][k],   db[c] += sum_r g[r][c]
+// Same thread layout and block reduction as latent_bwd_clf_kernel (a thread keeps its 4 columns; 256 % (L / 4) == 0), atomics into the
+// zeroed classifier span.  One read of mu and g_rows.
+template <int NC>
+__global__ void __launch_bounds__(256) clf_rows_wgrad_kernel(const float* __restrict__ mu, int64_t n_elems, int L, ClfBwdArgs ca) {
+  PSVAE_GRID_DEP();
+  __shared__ float lb_smem[256 * 8];
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  const int64_t nq = n_elems >> 2;
+  const uint32_t qpr_ = (uint32_t)L >> 2;
+  const int nc = ca.total_classes;
+  float accW[NC][4], accb[NC];
+#pragma unroll
+  for (int cc = 0; cc < NC; ++cc) {
+    accb[cc] = 0.f;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) accW[cc][j] = 0.f;
+  }
+#pragma unroll 4
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nq; i += stride) {
+    const float4 m = __ldg(reinterpret_cast<const float4*>(mu) + i);
+    const int64_t row = (int64_t)((uint32_t)i / qpr_);
+    const float4 ga = __ldg(reinterpret_cast<const float4*>(ca.g_rows + row * CLF_MAXC));
+    float4 gb = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (NC > 4) gb = __ldg(reinterpret_cast<const float4*>(ca.g_rows + row * CLF_MAXC + 4));
+    const float gr[8] = {ga.x, ga.y, ga.z, ga.w, gb.x, gb.y, gb.z, gb.w};
+    const float mv[4] = {m.x, m.y, m.z, m.w};
+    const bool first_quad = ((uint32_t)i % qpr_) == 0;
+#pragma unroll
+    for (int cc = 0; cc < NC; ++cc) {
+      if (cc < nc) {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) accW[cc][j] = fmaf(gr[cc], mv[j], accW[cc][j]);
+        if (first_quad) accb[cc] += gr[cc];
+      }
+    }
+  }
+  const int qpr = L >> 2;
+  for (int cc = 0; cc < NC; ++cc) {
+    if (cc < nc) {            // block-uniform
+      __syncthreads();
+#pragma unroll
+      for (int j = 0; j < 4; ++j) lb_smem[threadIdx.x * 8 + j] = accW[cc][j];
+      lb_smem[threadIdx.x * 8 + 4] = accb[cc];
+      __syncthreads();
+      int h = 0;
+      for (int i = 0; i < ca.n_heads; ++i)
+        if (cc >= ca.head_off[i] && cc < ca.head_off[i] + ca.head_classes[i]) h = i;
+      const int lc = cc - ca.head_off[h];
+      if ((int)threadIdx.x < L) {
+        const int col = threadIdx.x, quad = col >> 2, j = col & 3;
+        float t = 0.f;
+        for (int th = quad; th < 256; th += qpr) t += lb_smem[th * 8 + j];
+        atomicAdd(ca.grads + ca.w_off[h] + (int64_t)lc * L + col, t);
+      } else if ((int)threadIdx.x == L) {
+        float t = 0.f;
+        for (int th = 0; th < 256; ++th) t += lb_smem[th * 8 + 4];      // only the threads that own a row's first quad added to it
+        atomicAdd(ca.grads + ca.b_off[h] + lc, t);
+      }
+    }
+  }
+}
+
 // The same pass for the tcgen05 mode's common shape (bf16 sigma eps / 2 and outputs, L % 8 == 0, at most 4 classes in total): one thread owns
 // EIGHT consecutive latent columns of a row per trip and two rows are in flight (16 independent 16-byte loads per thread before the first use;
 // 128 registers at two blocks per SM).  The 4-column form above ran at 2.3 TB/s with spills at its 80-register cap

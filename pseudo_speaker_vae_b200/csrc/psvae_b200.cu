@@ -469,6 +469,7 @@ static void plan(const psvae_model_desc* d, int64_t rows, int mode, Bump& b, Ste
     return;
   }
   const bool train = (mode == PSVAE_MODE_TRAIN);
+  const bool clf_train = (mode == PSVAE_MODE_TRAIN_CLASSIFIER);
   if (is_bf16) w.xa = b.take<TAct>(rows * n.D);
   for (int j = 0; j < n.nh; ++j) w.he[j] = b.take<TAct>(rows * 2 * n.H);
   w.mu = b.take<float>(rows * n.L);
@@ -493,6 +494,30 @@ static void plan(const psvae_model_desc* d, int64_t rows, int mode, Bump& b, Ste
         w.acc_part[h] = b.take<float>(w.n_ce);
       }
     }
+  }
+  if (clf_train && n.has_clf()) {
+    // the classifier's backward only.  The fused encoder head (fast mode) stays the forward kernel: it writes sigma eps / 2 next to z
+    // through one 3D output map (so it needs that buffer, right after z) and d loss / d logits per row
+    if (is_bf16 && fused_head_shape_ok(d)) {
+      w.hs = b.take<TAct>(rows * n.L);
+      w.clf_grows = b.take<float>(rows * CLF_MAXC);
+    }
+    if (!clf_fused_ok(d)) {
+      int64_t wmax = 0, cmax = d->clf_hidden;
+      auto upd = [&](int64_t M, int64_t N) {
+        const int64_t s = Engine<float>::wgrad_splits(M, N, rows);
+        if (s * M * N > wmax) wmax = s * M * N;
+      };
+      if (d->clf_num_trunk > 0) for (int i = 0; i < 2; ++i) w.clf_g[i] = b.take<float>(rows * d->clf_hidden);
+      for (int t = 0; t < d->clf_num_trunk; ++t) upd(d->clf_hidden, n.clf_trunk_in(t));
+      for (int h = 0; h < d->clf_num_heads; ++h) {
+        upd(d->clf_head_classes[h], n.clf_feat());
+        if (d->clf_head_classes[h] > cmax) cmax = d->clf_head_classes[h];
+      }
+      w.wpart = b.take<float>(wmax);
+      w.cpart = b.take<float>(ceil_div64(rows, g_opt.colsum_rows) * cmax);
+    }
+    return;
   }
   if (!train) return;
   if (is_bf16) {
@@ -742,6 +767,8 @@ struct StepArgs {
   const bf16* x16 = nullptr;
   // device step counters (psvae_train_fwd_bwd_dc): the Philox offset of the eps draw is read from here instead of `offset`
   const uint64_t* offset_dev = nullptr;
+  // PSVAE_GRAD_CLASSIFIER (frozen VAE): the full forward and losses, then only the latent classifier's gradients, into its span of grads
+  int grad_scope = PSVAE_GRAD_ALL;
 };
 
 template <typename TAct> static const TAct* weights_of(const StepArgs& a);
@@ -789,7 +816,12 @@ static int run_step(const StepArgs& a) {
   if (a.want_grads && !a.grads) { set_error("grads must not be NULL when compute_grads != 0"); return -1; }
   if (a.want_loss && !a.losses) { set_error("losses must not be NULL"); return -1; }
   if (a.want_loss && n.has_clf() && !a.y) { set_error("y must not be NULL when the model has a classifier"); return -1; }
-  const int mode = a.want_grads ? PSVAE_MODE_TRAIN : PSVAE_MODE_FORWARD;
+  // classifier-only scope: the forward half behaves as a forward with losses for everything the VAE backward would read (no ReLU masks, no
+  // sigma eps / 2, no d loss / d x_hat); `vae_grads` is what `want_grads` means for the VAE
+  const bool clf_only = a.want_grads && a.grad_scope == PSVAE_GRAD_CLASSIFIER;
+  if (clf_only && (!n.has_clf() || !a.want_loss || a.ext)) { set_error("the classifier gradient scope needs a model with a latent classifier"); return -2; }
+  const bool vae_grads = a.want_grads && !clf_only;
+  const int mode = clf_only ? PSVAE_MODE_TRAIN_CLASSIFIER : a.want_grads ? PSVAE_MODE_TRAIN : PSVAE_MODE_FORWARD;
   const bool cons_on = a.cons != nullptr && a.want_loss;
   if (cons_on) {
     PSVAE_TRY(check_cons(a.cons));
@@ -803,21 +835,23 @@ static int run_step(const StepArgs& a) {
     StepBufs<TAct> tmp;
     ConsBufs ctmp;
     plan<TAct>(d, B, mode, sz, tmp);
-    if (cons_on) plan_cons(a.cons, B, a.want_grads != 0, sz, ctmp);
+    if (cons_on) plan_cons(a.cons, B, vae_grads, sz, ctmp);
     if (sz.used > a.ws_bytes || !a.ws) {
       set_error("workspace too small: need %lld bytes, got %lld", (long long)sz.used, (long long)a.ws_bytes);
       return -2;
     }
     Bump b(a.ws);
     plan<TAct>(d, B, mode, b, w);
-    if (cons_on) plan_cons(a.cons, B, a.want_grads != 0, b, cw);
+    if (cons_on) plan_cons(a.cons, B, vae_grads, b, cw);
   }
   const TAct* Wt = weights_of<TAct>(a);
   const float* P = a.params;
   // gradients are accumulated into (TMA reduce-add / atomics in fast tcgen05 mode) or written into a zeroed buffer; padding reads as zero
   // (tcgen05 mode: the operand cast of x below clears the buffer in the same pass -- total_numel is a multiple of 64 and the buffer 16-byte aligned)
-  const bool zero_in_cast = sizeof(TAct) == 2 && a.want_grads && (reinterpret_cast<uintptr_t>(a.grads) & 15) == 0;
-  if (a.want_grads && !zero_in_cast) PSVAE_CUDA(cudaMemsetAsync(a.grads, 0, (size_t)d->total_numel * sizeof(float), st));
+  const bool zero_in_cast = sizeof(TAct) == 2 && vae_grads && (reinterpret_cast<uintptr_t>(a.grads) & 15) == 0;
+  if (vae_grads && !zero_in_cast) PSVAE_CUDA(cudaMemsetAsync(a.grads, 0, (size_t)d->total_numel * sizeof(float), st));
+  // classifier scope: its span of the buffer only, [vae_numel, total_numel) -- every other element keeps its value
+  if (clf_only) PSVAE_CUDA(cudaMemsetAsync(a.grads + d->vae_numel, 0, (size_t)(d->total_numel - d->vae_numel) * sizeof(float), st));
   // option fused_head (training, fast mode): encoder heads + reparameterisation + KL + classifier forward in one kernel.  Its 3D output maps
   // step from mu to log_sigma (and from z to sigma eps / 2) by one stride, so it writes the workspace buffers; a caller's mu / log_sigma get a copy.
   bool fused_head = false;
@@ -930,7 +964,7 @@ static int run_step(const StepArgs& a) {
     n_kl_used = fused_ctas;            // the fused kernel wrote one KL / NLL / accuracy record per CTA
   } else if (!fuse_latent) {
     launch_dep(a.offset_dev ? latent_fwd_kernel<TAct, true> : latent_fwd_kernel<TAct>, dim3((unsigned)w.n_kl), dim3(256), 0, st, mu, ls, a.eps, a.seed,
-               a.offset, first_elem, B * n.L, w.z, nullptr, w.kl_part, a.want_grads ? w.hs : nullptr, a.offset_dev);
+               a.offset, first_elem, B * n.L, w.z, nullptr, w.kl_part, vae_grads ? w.hs : nullptr, a.offset_dev);
     count_launch();
     PSVAE_LAUNCH_CHECK("latent_fwd_kernel");
   } else {
@@ -951,11 +985,11 @@ static int run_step(const StepArgs& a) {
     ca.grads = a.want_grads ? a.grads : nullptr;
     ca.sums = w.clf_sums;
     // the classifier's backward moves into the latent backward kernel (fast mode only: it adds with atomics)
-    ca.g_rows = (g_opt.clf_grad_in_bwd && a.want_grads && ca.atomic_out && w.clf_grows && latent_cs_ok(n.L)) ? w.clf_grows : nullptr;
+    ca.g_rows = (g_opt.clf_grad_in_bwd && vae_grads && ca.atomic_out && w.clf_grows && latent_cs_ok(n.L)) ? w.clf_grows : nullptr;
     const int blocks = clf_fused_blocks(B);
     const size_t smem = clf_fused_smem_bytes(n.L);
-    float* dmu_out = a.want_grads ? w.dmu_clf : nullptr;
-    ReparamArgs rp{ls, a.eps, a.seed, a.offset, first_elem >> 2, w.z, w.kl_part, a.want_grads ? w.hs : nullptr, a.offset_dev};
+    float* dmu_out = vae_grads ? w.dmu_clf : nullptr;
+    ReparamArgs rp{ls, a.eps, a.seed, a.offset, first_elem >> 2, w.z, w.kl_part, vae_grads ? w.hs : nullptr, a.offset_dev};
     n_kl_used = blocks;
     switch (n.L) {
 #define PSVAE_CLF_CASE(LL)                                                                                                              \
@@ -1009,7 +1043,7 @@ static int run_step(const StepArgs& a) {
     int chain_ctas = 0;
     if constexpr (sizeof(TAct) == 2) {
       // option train_chain: the whole decoder + MSE epilogue as one chained kernel (hidden activations stay on-chip for the forward pass)
-      if (g_opt.train_chain && a.want_grads && !g_opt.deterministic && !a.x_hat && decoder_chain_ok(n.D, n.L, n.H, n.nh) && w.mhd[0] && w.mhd[1]) {
+      if (g_opt.train_chain && vae_grads && !g_opt.deterministic && !a.x_hat && decoder_chain_ok(n.D, n.L, n.H, n.nh) && w.mhd[0] && w.mhd[1]) {
         DcArgs ca;
         memset(&ca, 0, sizeof(ca));
         ca.rows = B; ca.H = n.H; ca.D = n.D;
@@ -1029,7 +1063,7 @@ static int run_step(const StepArgs& a) {
       }
     }
     if constexpr (sizeof(TAct) == 2) {
-      if (!launched && a.want_grads && tc_colsum_ok(n.D)) {     // + column sums of dxh = bias gradient of the last decoder layer
+      if (!launched && vae_grads && tc_colsum_ok(n.D)) {     // + column sums of dxh = bias gradient of the last decoder layer
         const bool atomic = !g_opt.deterministic;
         if (a.x16) {
           EpiMse<TAct, true, bf16> e{P + d->dec_b[n.nh], a.x16, n.D, a.x_hat, n.D, w.dxh, n.D, scale, w.sse_part, atomic ? a.grads + d->dec_b[n.nh] : w.cpart,
@@ -1085,17 +1119,17 @@ static int run_step(const StepArgs& a) {
           xh = xh_out;
         }
         PSVAE_TRY(cons_forward(a.cons, a.cons_params, xh, B, cw, cw.logits, st));
-        launch_dep(ce_kernel, dim3((unsigned)cw.n_ce), dim3(256), 0, st, cw.logits, a.cons_y, B, a.cons->num_classes, a.cons_w / (float)B, a.want_grads,
+        launch_dep(ce_kernel, dim3((unsigned)cw.n_ce), dim3(256), 0, st, cw.logits, a.cons_y, B, a.cons->num_classes, a.cons_w / (float)B, vae_grads,
                                                 cw.nll_part, cw.acc_part);
         count_launch();
         PSVAE_LAUNCH_CHECK("ce_kernel");
-        if (a.want_grads) {
+        if (vae_grads) {
           PSVAE_TRY(cons_input_grad(a.cons, a.cons_params, B, cw, st));
           gx = cw.gx;
         }
       }
       launch_dep(recon_rows_kernel<TAct>, dim3(blocks), dim3(256), 0, st, w.u, a.want_loss ? a.x : nullptr, B, n.D, d->normalize_decoder, a.use_cos, gscale, a.x_hat,
-                                                      a.want_grads ? w.dxh : nullptr, a.want_loss ? w.sse_part : nullptr, gx);
+                                                      vae_grads ? w.dxh : nullptr, a.want_loss ? w.sse_part : nullptr, gx);
       count_launch();
       PSVAE_LAUNCH_CHECK("recon_rows_kernel");
       n_sse_used = blocks;
@@ -1109,7 +1143,7 @@ static int run_step(const StepArgs& a) {
   if constexpr (sizeof(TAct) == 2) {
     int total_classes = 0;
     for (int h = 0; h < d->clf_num_heads; ++h) total_classes += d->clf_head_classes[h];
-    finalize_in_latent = a.want_loss && a.want_grads && !a.ext && clf_fused && (g_opt.clf_grad_in_bwd || fused_head) && !g_opt.deterministic &&
+    finalize_in_latent = a.want_loss && vae_grads && !a.ext && clf_fused && (g_opt.clf_grad_in_bwd || fused_head) && !g_opt.deterministic &&
                          w.clf_grows && latent_cs_ok(n.L) && latent8_ok(n.L, total_classes);
   }
   if (a.want_loss) {
@@ -1158,7 +1192,7 @@ static int run_step(const StepArgs& a) {
       PSVAE_TRY(wgrad_clf<TAct>(w.logits[h], C, featp, feat_dim, B, C, feat_dim, G + d->clf_head_w[h], G + d->clf_head_b[h], w, st));
     }
     if (T == 0) {
-      for (int h = 0; h < d->clf_num_heads; ++h)
+      for (int h = 0; h < d->clf_num_heads && vae_grads; ++h)
         PSVAE_TRY(clf_dgrad(ACT_NONE, w.logits[h], d->clf_head_classes[h], P + d->clf_head_w[h], n.L, nullptr, w.dmu_clf, h > 0 ? 1.f : 0.f, B, st));
     } else {
       float* cur = w.clf_g[0];
@@ -1173,12 +1207,36 @@ static int run_step(const StepArgs& a) {
         if (t > 0) {
           PSVAE_TRY(clf_dgrad(d->clf_activation, cur, d->clf_hidden, P + d->clf_trunk_w[t], in_dim, w.clf_act[t - 1], nxt, 0.f, B, st));
           float* tmp = cur; cur = nxt; nxt = tmp;
-        } else {
+        } else if (vae_grads) {       // the classifier scope stops at the trunk's first layer: d loss / d mu has no consumer
           PSVAE_TRY(clf_dgrad(ACT_NONE, cur, d->clf_hidden, P + d->clf_trunk_w[0], n.L, nullptr, w.dmu_clf, 0.f, B, st));
         }
       }
     }
     dmu_clf = w.dmu_clf;
+  }
+  if (clf_only) {
+    // linear heads: the fused classifier pass (+ its finish kernel) already wrote the gradients, except under the fused encoder head, which
+    // leaves d loss / d logits per row in clf_grows (the full step folds them into the latent backward)
+    if (!fused_head) return 0;
+    if (!latent_cs_ok(n.L)) { set_error("classifier scope: latent_dim=%d has no row-gradient kernel", n.L); return -2; }
+    ClfBwdArgs cb;
+    memset(&cb, 0, sizeof(cb));
+    cb.n_heads = d->clf_num_heads;
+    for (int h = 0; h < d->clf_num_heads; ++h) {
+      cb.head_classes[h] = d->clf_head_classes[h];
+      cb.head_off[h] = cb.total_classes;
+      cb.total_classes += d->clf_head_classes[h];
+      cb.w_off[h] = d->clf_head_w[h];
+      cb.b_off[h] = d->clf_head_b[h];
+    }
+    cb.params = P; cb.grads = G; cb.g_rows = w.clf_grows;
+    int blocks = ew_grid(B * n.L / 4);
+    if (blocks > 2 * PSVAE_NUM_SMS) blocks = 2 * PSVAE_NUM_SMS;      // 8 blocks per SM measured slower: more atomics on the same 130 floats
+    if (cb.total_classes <= 4) launch_dep(clf_rows_wgrad_kernel<4>, dim3(blocks), dim3(256), 0, st, (const float*)mu, B * n.L, n.L, cb);
+    else launch_dep(clf_rows_wgrad_kernel<CLF_MAXC>, dim3(blocks), dim3(256), 0, st, (const float*)mu, B * n.L, n.L, cb);
+    count_launch();
+    PSVAE_LAUNCH_CHECK("clf_rows_wgrad_kernel");
+    return 0;
   }
 
   // ---- decoder backward: dY starts as d loss / d (decoder output)
@@ -1541,7 +1599,7 @@ int psvae_model_desc_init(psvae_model_desc* desc, int32_t input_dim, int32_t lat
 
 int64_t psvae_workspace_bytes(const psvae_model_desc* desc, int64_t rows, int32_t precision, int32_t mode) {
   if (check_desc(desc, precision) != 0) return -1;
-  if (rows <= 0 || mode < 0 || mode > 2) { set_error("bad rows/mode"); return -1; }
+  if (rows <= 0 || mode < 0 || mode > PSVAE_MODE_TRAIN_CLASSIFIER) { set_error("bad rows/mode"); return -1; }
   if (mode == PSVAE_MODE_DECODE && rows > g_opt.decode_chunk) rows = g_opt.decode_chunk;
   Bump b(nullptr);
   if (precision == PSVAE_BF16) { StepBufs<bf16> w; plan<bf16>(desc, rows, mode, b, w); }
@@ -1965,29 +2023,34 @@ int psvae_train_fwd_bwd_consistency(const psvae_model_desc* desc, const float* p
   return precision == PSVAE_BF16 ? run_step<bf16>(a) : run_step<float>(a);
 }
 
-int psvae_train_fwd_bwd_dc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
-                           const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
-                           int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
-                           void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
-                           const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters) {
+}  // extern "C"
+
+// psvae_train_fwd_bwd_dc / _acc with a gradient scope (psvae_train_fwd_bwd_scoped)
+static int train_dc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
+                    const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
+                    int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
+                    void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
+                    const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters, int32_t grad_scope) {
   PSVAE_TRY(check_desc(desc, precision));
   StepArgs a{desc, params, static_cast<const bf16*>(shadow_bf16), grads, nullptr, y, eps, seed, offset, row0, rows, kl_weight, clf_weight,
              use_cos_loss ? 1 : 0, 1, compute_grads ? 1 : 0, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, static_cast<cudaStream_t>(stream)};
   PSVAE_TRY(set_x(a, x, x_dtype));
   a.cons = cons; a.cons_params = cons_params; a.cons_y = cons_y; a.cons_w = cons_weight;
   a.offset_dev = counters ? &counters->rng_offset : nullptr;
+  a.grad_scope = grad_scope;
   return precision == PSVAE_BF16 ? run_step<bf16>(a) : run_step<float>(a);
 }
 
-int psvae_train_fwd_bwd_acc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
-                            const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
-                            int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
-                            void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
-                            const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters, int32_t accumulate, float* grad_scratch) {
+static int train_acc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
+                     const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
+                     int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
+                     void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
+                     const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters, int32_t accumulate, float* grad_scratch,
+                     int32_t grad_scope) {
   if (!accumulate || !compute_grads)
-    return psvae_train_fwd_bwd_dc(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss,
-                                  compute_grads, precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y,
-                                  cons_weight, counters);
+    return train_dc(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss,
+                    compute_grads, precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y,
+                    cons_weight, counters, grad_scope);
   PSVAE_TRY(check_desc(desc, precision));
   if (!grads || !grad_scratch) { set_error("grads and grad_scratch must not be NULL when accumulate != 0"); return -1; }
   if (((reinterpret_cast<uintptr_t>(grads) | reinterpret_cast<uintptr_t>(grad_scratch)) & 15) != 0) {
@@ -1996,14 +2059,57 @@ int psvae_train_fwd_bwd_acc(const psvae_model_desc* desc, const float* params, c
   }
   if (grads == grad_scratch) { set_error("grad_scratch must not be the gradient buffer"); return -2; }
   // the step writes this micro-batch's gradient into the scratch exactly as the non-accumulating step writes `grads`; one pass then adds it
-  PSVAE_TRY(psvae_train_fwd_bwd_dc(desc, params, shadow_bf16, grad_scratch, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight,
-                                   use_cos_loss, compute_grads, precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons,
-                                   cons_params, cons_y, cons_weight, counters));
-  const int64_t n = desc->total_numel;
-  launch_dep(grad_accumulate_kernel, dim3(ew_grid(n / 4 + 1)), dim3(256), 0, static_cast<cudaStream_t>(stream), grads, (const float*)grad_scratch, n);
+  // (the classifier scope: over the classifier span only -- vae_numel is a multiple of 8 floats, so the span stays 16-byte aligned)
+  PSVAE_TRY(train_dc(desc, params, shadow_bf16, grad_scratch, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight,
+                     use_cos_loss, compute_grads, precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons,
+                     cons_params, cons_y, cons_weight, counters, grad_scope));
+  const int64_t a0 = grad_scope == PSVAE_GRAD_CLASSIFIER ? desc->vae_numel : 0;
+  const int64_t n = desc->total_numel - a0;
+  launch_dep(grad_accumulate_kernel, dim3(ew_grid(n / 4 + 1)), dim3(256), 0, static_cast<cudaStream_t>(stream), grads + a0,
+             (const float*)grad_scratch + a0, n);
   count_launch();
   PSVAE_LAUNCH_CHECK("grad_accumulate_kernel");
   return 0;
+}
+
+extern "C" {
+
+int psvae_train_fwd_bwd_dc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
+                           const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
+                           int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
+                           void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
+                           const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters) {
+  return train_dc(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss, compute_grads,
+                  precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y, cons_weight, counters,
+                  PSVAE_GRAD_ALL);
+}
+
+int psvae_train_fwd_bwd_acc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
+                            const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
+                            int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
+                            void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
+                            const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters, int32_t accumulate, float* grad_scratch) {
+  return train_acc(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss, compute_grads,
+                   precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y, cons_weight, counters,
+                   accumulate, grad_scratch, PSVAE_GRAD_ALL);
+}
+
+int psvae_train_fwd_bwd_scoped(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x,
+                               int32_t x_dtype, const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows,
+                               float kl_weight, float clf_weight, int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat,
+                               float* mu, float* log_sigma, float* losses, void* workspace, int64_t workspace_bytes, void* stream,
+                               const psvae_consistency_desc* cons, const float* cons_params, const int64_t* cons_y, float cons_weight,
+                               const psvae_step_counters* counters, int32_t accumulate, float* grad_scratch, int32_t grad_scope) {
+  // argument checks first: they do not need a device
+  PSVAE_TRY(check_desc(desc, precision));
+  if (grad_scope != PSVAE_GRAD_ALL && grad_scope != PSVAE_GRAD_CLASSIFIER) { set_error("unknown grad_scope %d", grad_scope); return -2; }
+  if (grad_scope == PSVAE_GRAD_CLASSIFIER && desc->clf_num_heads <= 0) {
+    set_error("grad_scope PSVAE_GRAD_CLASSIFIER: the model has no latent classifier");
+    return -2;
+  }
+  return train_acc(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss, compute_grads,
+                   precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y, cons_weight, counters,
+                   accumulate, grad_scratch, grad_scope);
 }
 
 int psvae_vae_backward(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype, const float* eps,

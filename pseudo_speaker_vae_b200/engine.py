@@ -157,6 +157,11 @@ class ParamArena:
             self._shadow_epoch = self.epoch
         return self.shadow.data_ptr()
 
+    def shadow_current(self) -> bool:
+        """Is the bf16 copy on the arena's device and up to date with the parameters (nothing rewrote them since it was last written)?"""
+        return self.shadow is not None and self.shadow.device == self.flat.device and self._shadow_epoch == self.epoch \
+            and self._shadow_versions == tuple(p._version for p, _ in self.entries)
+
     def mark_shadow_current(self) -> None:
         """Called by the fused Adam, which writes the bf16 copy itself."""
         self._shadow_versions = tuple(p._version for p, _ in self.entries)
@@ -455,7 +460,8 @@ class HotPath:
     def step(self, x: torch.Tensor, y=None, eps: Optional[torch.Tensor] = None, *, kl_weight: float = 1.0, clf_weight: float = 1.0,
              use_cos_loss: bool = False, compute_grads: bool = True, grads: Optional[torch.Tensor] = None, want_outputs: bool = False,
              consistency: Optional[nn.Module] = None, consistency_y: Optional[torch.Tensor] = None, consistency_weight: float = 1.0,
-             counters: Optional[torch.Tensor] = None, accumulate: bool = False, grad_scratch: Optional[torch.Tensor] = None):
+             counters: Optional[torch.Tensor] = None, accumulate: bool = False, grad_scratch: Optional[torch.Tensor] = None,
+             grad_scope: str = "all"):
         """One fused forward(+backward).  Returns (losses[16] device tensor, flat grads or None, outputs or None).
 
         ``consistency``: a frozen ``EmbeddingClassifier`` whose ``consistency_weight * CE(consistency(x_hat), consistency_y)``
@@ -464,7 +470,15 @@ class HotPath:
         from it on the device (``psvae_train_fwd_bwd_dc``), so that a CUDA graph of this call draws fresh noise at every replay.  The host
         offset still advances as usual: it is the mirror the caller keeps the block in step with.
         ``accumulate``: ADD this batch's gradients to what ``grads`` holds (``psvae_train_fwd_bwd_acc``: they are computed into
-        ``grad_scratch``, a flat fp32 buffer of the arena's size, then added with one fp32 addition per element)."""
+        ``grad_scratch``, a flat fp32 buffer of the arena's size, then added with one fp32 addition per element).
+        ``grad_scope``: ``"all"``, or ``"classifier"`` for a frozen VAE (``train_scope()``): the same forward and losses, but only the latent
+        classifier's gradients are computed, and only the classifier span of ``grads`` (``classifier_span()``) is written -- or, with
+        ``accumulate``, added to; every other element of ``grads`` keeps its value (``psvae_train_fwd_bwd_scoped``)."""
+        if grad_scope not in ("all", "classifier"):
+            raise ValueError(f"grad_scope must be 'all' or 'classifier', got {grad_scope!r}")
+        if grad_scope == "classifier" and self.classifier is None:
+            raise ValueError("grad_scope 'classifier' needs a model with a latent classifier")
+        clf_scope = compute_grads and grad_scope == "classifier"
         dev = self._device()
         flat = self.arena.ensure()
         D, Lz = self.desc.input_dim, self.desc.latent_dim
@@ -492,7 +506,7 @@ class HotPath:
             mu = torch.empty(B, Lz, dtype=torch.float32, device=dev)
             ls = torch.empty(B, Lz, dtype=torch.float32, device=dev)
             outs = (xh, mu, ls)
-        mode = L.MODE_TRAIN if compute_grads else L.MODE_FORWARD
+        mode = L.MODE_TRAIN_CLASSIFIER if clf_scope else L.MODE_TRAIN if compute_grads else L.MODE_FORWARD
         args = (self._dref, flat.data_ptr(), self._shadow(), L.ptr(grads) if compute_grads else None, x.data_ptr(), _xflag(x), L.ptr(yy),
                 L.ptr(eps), seed, off, self.row0, B, float(kl_weight), float(clf_weight), int(bool(use_cos_loss)),
                 int(bool(compute_grads)), self.precision, L.ptr(xh), L.ptr(mu), L.ptr(ls), losses.data_ptr())
@@ -506,7 +520,7 @@ class HotPath:
             if cy.numel() != B:
                 raise ValueError(f"labels have {cy.numel()} rows, x has {B}")
             cdesc, cflat = consistency.flat_params(dev)
-            extra = int(L.lib().psvae_consistency_workspace_bytes(C.byref(cdesc), B, mode))
+            extra = int(L.lib().psvae_consistency_workspace_bytes(C.byref(cdesc), B, L.MODE_FORWARD if clf_scope else mode))
             if extra < 0:
                 raise ValueError(L.last_error())
             cons_args = (C.byref(cdesc), cflat.data_ptr(), cy.data_ptr(), float(consistency_weight))
@@ -516,6 +530,13 @@ class HotPath:
             if grads is None or grad_scratch is None or grad_scratch.device != dev or grad_scratch.dtype != torch.float32 \
                     or grad_scratch.numel() < self.arena.numel or grad_scratch.data_ptr() == grads.data_ptr():
                 raise ValueError("an accumulating step needs `grads` and a separate fp32 `grad_scratch` of the arena's size on the same device")
+        if clf_scope:
+            with _on(dev):
+                ws = self._workspace(dev, B, mode, extra if consistency is not None else 0)
+                rc = L.lib().psvae_train_fwd_bwd_scoped(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args, L.ptr(counters),
+                                                        int(bool(accumulate)), L.ptr(grad_scratch) if accumulate else None, L.GRAD_CLASSIFIER)
+            L.check(rc, "psvae_train_fwd_bwd_scoped")
+        elif accumulate and compute_grads:
             with _on(dev):
                 ws = self._workspace(dev, B, mode, extra if consistency is not None else 0)
                 rc = L.lib().psvae_train_fwd_bwd_acc(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args, L.ptr(counters), 1,
@@ -537,6 +558,20 @@ class HotPath:
                 rc = L.lib().psvae_train_fwd_bwd_consistency(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args)
             L.check(rc, "psvae_train_fwd_bwd_consistency")
         return losses, (grads if compute_grads else None), outs
+
+    def train_scope(self) -> str:
+        """The gradient scope the ``requires_grad`` flags call for: ``"classifier"`` when every VAE parameter is frozen and every classifier
+        parameter is trainable (the second stage of a two-stage run, ``freeze_vae``), ``"all"`` for any other mix."""
+        if self.classifier is None:
+            return "all"
+        vae_numel = int(self.desc.vae_numel)
+        vae = [p.requires_grad for p, o in self.arena.entries if o < vae_numel]
+        clf = [p.requires_grad for p, o in self.arena.entries if o >= vae_numel]
+        return "classifier" if not any(vae) and all(clf) else "all"
+
+    def classifier_span(self) -> Tuple[int, int]:
+        """[a, b) of the classifier's parameters (and the arena's tail padding) in the flat buffers: what the classifier scope writes."""
+        return int(self.desc.vae_numel), int(self.desc.total_numel)
 
     def loss_with_grad(self, losses: torch.Tensor, gflat: torch.Tensor) -> torch.Tensor:
         """The scalar a LightningModule returns from training_step: ``.backward()`` hands the fused gradients to autograd."""

@@ -109,15 +109,20 @@ class GraphedTrainStep:
                 tr._views_of.data_ptr() if tr._views_of is not None else None, cflat)
         knobs = (tr.accumulate_grad_batches, tr.gradient_clip_val, tr.gradient_clip_algorithm, opt.clip_mode, opt.clip_value, L.ptr(opt.clip_coef),
                  L.ptr(tr._acc_scratch), L.ptr(tr._norm_scratch))
+        trained = tuple(p.requires_grad for p in hot.parameters())      # the gradient scope and the Adam spans follow from it
         return (hot.seed, hot.row0, hot.precision, m.kl_loss_weight, m.classifier_loss_weight, m.use_cos_loss, m.consitency_loss_weight,
-                id(cons), L.OPTIONS_EPOCH, opt.grad_scale, groups, bufs, knobs)
+                id(cons), L.OPTIONS_EPOCH, opt.grad_scale, groups, bufs, knobs, trained)
 
     # ---- capture --------------------------------------------------------------------------------
     def _check_supported(self) -> None:
         opt, tr = self.optimizer, self.trainer
         if not isinstance(opt, FusedAdam):
             raise NotImplementedError(f"a graphed train step needs FusedAdam, got {type(opt).__name__}")
-        if not opt.covers_arena():
+        # a frozen VAE (classifier scope) is the one partial freeze a graph takes: Adam rewrites only the classifier, whose slice of the bf16
+        # copy no kernel reads, and the VAE's slice stays what the refresh before capture made it
+        frozen_vae = self.hot.train_scope() == "classifier" and \
+            {id(p) for g in opt.param_groups for p in g["params"] if p.grad is not None} == {id(p) for p in self.hot.parameters() if p.requires_grad}
+        if not opt.covers_arena() and not frozen_vae:
             raise NotImplementedError("a graphed train step needs every arena parameter trained (no frozen parameters): the bf16 operand "
                                       "copy must be rewritten by Adam, not refreshed inside the graph")
         if tr._views_of is None or self.hot.arena.flat_grad() is None:
@@ -186,6 +191,8 @@ class GraphedTrainStep:
         # the attempts, in order: the all-reduce the trainer picked, NCCL if that was a symmetric-memory kind, then the same without
         # programmatic-launch attributes (a driver that refuses them under capture)
         want = tr.symm.kind if tr.symm is not None else None
+        if hot.train_scope() == "classifier":          # the classifier's span goes through NCCL (DataParallelTrainer._all_reduce)
+            want = "nccl" if tr.world_size > 1 and not tr.local_only else None
         kinds = [want, "nccl"] if want not in (None, "nccl") else [want]
         pdl0 = L.get_option("pdl")
         attempts = [(k, pdl0) for k in kinds] + ([(k, 0) for k in kinds] if pdl0 else [])
@@ -241,6 +248,8 @@ class GraphedTrainStep:
             self._warm = True
             return self.trainer.train_step(x, y, flush=flush)
         phase = self.trainer._window_phase(flush)
+        if self.trainer._views_of is not None:
+            self.trainer._bind_grads(self.trainer._views_of)      # the trained set may have changed since the last call (unfreezing)
         if (phase not in self._graphs or self._capture_key() != self._key or self._label_sig(y) != self._static["ysig"]
                 or x.shape[1] != static_x.shape[1]):
             self._capture(x, y, phase)

@@ -108,9 +108,10 @@ class PseudoSpeakerVAE(_Base):
         hot = self._hot
         train_vae = any(p.requires_grad for p in self.model.parameters())
         need_grads = compute_grads and torch.is_grad_enabled() and (train_vae or self.classifier is not None)
+        # freeze_vae (the second stage of a two-stage run): the classifier scope skips the whole VAE backward
         losses, gflat, _ = hot.step(x, y, eps, kl_weight=self.kl_loss_weight, clf_weight=self.classifier_loss_weight,
                                     use_cos_loss=self.use_cos_loss, compute_grads=need_grads, consistency=cons, consistency_y=cons_y,
-                                    consistency_weight=self.consitency_loss_weight)
+                                    consistency_weight=self.consitency_loss_weight, grad_scope=hot.train_scope() if need_grads else "all")
         if self.classifier is not None:
             if not self.multilabel:
                 self.log(f"{prefix}_classifier_acc", losses[L.LOSS_ACC_HEAD0], sync_dist=True)

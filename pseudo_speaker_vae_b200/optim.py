@@ -150,6 +150,8 @@ class FusedAdam(torch.optim.Optimizer):
         lib = L.lib()
         stream = _stream_ptr(dev)
         touched = False
+        # every span below also rewrites its slice of the bf16 copy: a copy that was current stays current whatever the update covers
+        shadow_was_current = not dc and self.arena.shadow_current()
         for gi, group in enumerate(self.param_groups):
             with_grad = [p for p in group["params"] if p.grad is not None]
             if not with_grad:
@@ -198,7 +200,7 @@ class FusedAdam(torch.optim.Optimizer):
                 step_t += 1
         if touched and not dc:
             self.arena.epoch += 1
-            if self.covers_arena() and self.arena.shadow is not None:
+            if self.arena.shadow is not None and (self.covers_arena() or shadow_was_current):
                 self.arena.mark_shadow_current()
 
     def covers_arena(self) -> bool:

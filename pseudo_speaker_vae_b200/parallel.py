@@ -190,6 +190,7 @@ class DataParallelTrainer:
         self.hot.arena.epoch += 1          # the bf16 operand copy must follow the broadcast values
         self._views = None
         self._views_of = None
+        self._views_trained = None
         # N > 1: the gradient buffer lives in symmetric memory when one of its all-reduce kernels beats NCCL on these ranks
         # (PSVAE_ALLREDUCE = auto | nccl | two_shot | multimem)
         self.symm: Optional[SymmetricAllReduce] = None
@@ -222,16 +223,23 @@ class DataParallelTrainer:
         this micro-batch's local loss scalars.  ``flush``: end the accumulation window here (the last batch of an epoch)."""
         accumulate, step = self._window_phase(flush)
         losses, gflat = self._fwd_bwd(x_local, y_local, eps_local, accumulate=accumulate)
-        if self._views_of is not gflat:        # bind .grad views once; the same flat buffer is reused every step
-            for (p, _), v in zip(self.hot.arena.entries, self.hot.arena.grad_views(gflat)):
-                p.grad = v if p.requires_grad else None
-            self._views_of = gflat
+        self._bind_grads(gflat)
         if step:
             self._all_reduce(gflat)
             self._clip_norm(gflat)
             self.optimizer.step()
         self._end_micro_batch(step)
         return losses
+
+    def _bind_grads(self, gflat: torch.Tensor) -> None:
+        """Bind the .grad views of the trained parameters to the flat buffer: once, and again when the set of trained parameters changes
+        (unfreezing the VAE after a classifier-only stage)."""
+        trained = tuple(p.requires_grad for p, _ in self.hot.arena.entries)
+        if self._views_of is not gflat or trained != self._views_trained:
+            for (p, _), v in zip(self.hot.arena.entries, self.hot.arena.grad_views(gflat)):
+                p.grad = v if p.requires_grad else None
+            self._views_of = gflat
+            self._views_trained = trained
 
     def _window_phase(self, flush: bool = False) -> Tuple[bool, bool]:
         """(accumulate, step) of the next micro-batch: does it add to the gradient buffer, does it end the window."""
@@ -288,14 +296,24 @@ class DataParallelTrainer:
                                     clf_weight=m.classifier_loss_weight, use_cos_loss=m.use_cos_loss, compute_grads=True, grads=gflat,
                                     consistency=cons, consistency_y=y_local if cons is not None else None,
                                     consistency_weight=m.consitency_loss_weight, counters=counters, accumulate=accumulate,
-                                    grad_scratch=self._acc_scratch if accumulate else None)
+                                    grad_scratch=self._acc_scratch if accumulate else None, grad_scope=hot.train_scope())
         return losses, gflat
 
     def _all_reduce(self, gflat: torch.Tensor, kind: Optional[str] = None) -> None:
-        """The gradient all-reduce; ``kind`` overrides the symmetric-memory kind ``pick()`` chose (a CUDA graph may need NCCL)."""
-        if self.symm is not None:
+        """The gradient all-reduce; ``kind`` overrides the symmetric-memory kind ``pick()`` chose (a CUDA graph may need NCCL).
+        With a frozen VAE (classifier scope) only the classifier's span is reduced, with NCCL whatever kind was picked: the symmetric-memory
+        kernels reduce the whole 5 MB buffer, the span is a few hundred bytes.  ``allreduce_kind`` then reads "nccl"; a full-scope step sets
+        it back to the picked kind."""
+        if self.world_size == 1 or self.local_only:
+            return
+        if self.hot.train_scope() == "classifier":
+            a, b = self.hot.classifier_span()
+            all_reduce_flat(gflat[a:b], self.bucket_bytes, self.group)
+            self.allreduce_kind = "nccl"
+        elif self.symm is not None:
             self.symm._call(kind or self.symm.kind)
-        elif not self.local_only:
+            self.allreduce_kind = self.symm.kind
+        else:
             all_reduce_flat(gflat, self.bucket_bytes, self.group)
 
 
