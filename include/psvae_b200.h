@@ -323,6 +323,25 @@ int psvae_langevin(const psvae_model_desc* desc, const float* params, float* z_i
                    float* history, float* stats, float prior_weight, float threshold, int32_t* stop_step, float* last_prob,
                    void* stream);
 
+/* The same loop with a classifier target per row (additive to ABI 5).  Exactly one of:
+ *  - row_targets: device int32 [n_heads][rows], row r's class for head h at [h][r], -1 to leave head h out for that row.  A row with a
+ *    target outside [-1, classes) or naming no head gets NaN in z_io, its history rows and last_prob; the other rows are unaffected.
+ *  - a target mix of n_mix (1..PSVAE_MAX_TARGET_MIX) entries: mix_targets_host [n_mix][PSVAE_MAX_CLF_HEADS] (class or -1 per head, each
+ *    entry naming at least one head) and n_mix - 1 non-decreasing mix_thresholds_host.  Row r takes word row0 + r of the uint32 Philox
+ *    stream at offset offset0 + num_steps + 1 (psvae_philox_uint32 with first_elem = row0), u, and picks the first entry k < n_mix - 1 with
+ *    u < thresholds[k], else the last; entry k is drawn with probability (thresholds[k] - thresholds[k - 1]) / 2^32.  The drawn targets go to
+ *    row_targets_out (required), device int32 [n_heads][rows].  The draw depends on the global row only, so a sharded run draws what one
+ *    call over all rows draws.
+ * Every row computes exactly what psvae_langevin computes for it with its own target as the shared one (same seed, offset0, row0).
+ * Argument errors (no classifier, both or neither target form, n_mix > PSVAE_MAX_TARGET_MIX, a bad mix entry, decreasing thresholds, a mix
+ * without row_targets_out) are reported before the device is looked at. */
+#define PSVAE_MAX_TARGET_MIX 64
+int psvae_langevin_rows(const psvae_model_desc* desc, const float* params, float* z_io, int64_t rows, const int32_t* row_targets,
+                        int32_t n_mix, const int32_t* mix_targets_host, const uint32_t* mix_thresholds_host, int32_t* row_targets_out,
+                        float step_size, int32_t num_steps, float noise_weight, uint64_t seed, uint64_t offset0, int64_t row0,
+                        int32_t init_from_philox, const float* noise, float* history, float* stats, float prior_weight, float threshold,
+                        int32_t* stop_step, float* last_prob, void* stream);
+
 /* ---- building block exposed for tests and profiling: C = A[M,K] * B[N,K]^T (+bias) ------------- */
 /* a_mn / b_mn: operand stored MN-major (A as [K][M], B as [K][N]).  bf16 in, fp32 out, tcgen05. */
 int psvae_gemm_bf16(const void* a_bf16, const void* b_bf16, const float* bias, float* c, int64_t m, int32_t n,

@@ -36,7 +36,7 @@ EXPORTS = [
     "psvae_consistency_forward", "psvae_train_fwd_bwd_consistency", "psvae_vae_backward", "psvae_gather_rows",
     "psvae_embedding_classifier_workspace_bytes", "psvae_embedding_classifier_step", "psvae_train_fwd_bwd_dc", "psvae_adam_step_dc",
     "psvae_step_counters_advance", "psvae_train_fwd_bwd_acc", "psvae_grad_norm", "psvae_adam_step_clip", "psvae_step_counters_advance_by",
-    "psvae_train_fwd_bwd_scoped",
+    "psvae_train_fwd_bwd_scoped", "psvae_langevin_rows",
 ]
 
 #: int64 slots of ``psvae_step_counters`` (a device tensor of COUNTER_SLOTS int64)
@@ -44,6 +44,8 @@ COUNTER_RNG_OFFSET, COUNTER_ADAM_STEP, COUNTER_SLOTS = 0, 1, 4
 #: psvae_adam_step_clip modes and the psvae_grad_norm limits
 CLIP_NONE, CLIP_NORM, CLIP_VALUE = 0, 1, 2
 GRAD_NORM_MAX_SPANS, GRAD_NORM_SCRATCH_BYTES = 16, 4096
+#: psvae_langevin_rows: entries of a target mix
+MAX_TARGET_MIX = 64
 
 
 class ModelDesc(C.Structure):
@@ -147,6 +149,10 @@ def _declare(l: C.CDLL) -> None:
         l.psvae_train_fwd_bwd_scoped.argtypes = l.psvae_train_fwd_bwd_acc.argtypes + [I32]
     l.psvae_langevin.restype = C.c_int
     l.psvae_langevin.argtypes = [D, VP, VP, I64, P(I32), F, I32, F, U64, U64, I64, I32, VP, VP, VP, F, F, VP, VP, VP]
+    if hasattr(l, "psvae_langevin_rows"):
+        l.psvae_langevin_rows.restype = C.c_int
+        l.psvae_langevin_rows.argtypes = [D, VP, VP, I64, VP, I32, P(I32), P(C.c_uint32), VP, F, I32, F, U64, U64, I64, I32, VP, VP, VP, F, F, VP, VP,
+                                          VP]
     l.psvae_gemm_bf16.restype = C.c_int
     l.psvae_gemm_bf16.argtypes = [VP, VP, VP, VP, I64, I32, I64, I32, I32, I32, I32, VP, I64, VP]
     l.psvae_gemm_probe.restype = C.c_int

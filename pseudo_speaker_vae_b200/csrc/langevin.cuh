@@ -10,6 +10,11 @@
 // `prior_weight` scales the log p(z) term (the script's PRIOR_WEIGHT; inference.py has 1), `threshold` > 0 stops a sample after the update
 // of the first step whose p(y|z) exceeded it (the script's per-sample `break`), and `stop_step` / `last_prob` report, per sample, the step
 // at which that happened (num_steps if never) and the classifier probability of its last evaluated step.  A stopped sample keeps its z.
+//
+// Both kernels come in two instances: ROW_TARGETS = false takes one target for the whole batch (LangevinClf::targets), ROW_TARGETS = true
+// gives every row its own (LangevinRows): read from a device array, or drawn in the kernel from a target mix.  A row of the per-row instance
+// runs the same floating-point operations in the same order as the shared-target instance does with that row's target, so the two agree
+// bit for bit.
 #pragma once
 #include "common.cuh"
 #include "epilogue.cuh"
@@ -21,11 +26,12 @@ constexpr int LG_TILE = 32;      // samples per CTA
 constexpr int LG_THREADS = 256;  // 8 warps; lane = sample, warp = output-feature lane
 constexpr int LG_MAXC = 16;      // classes per head (padded row length in smem)
 constexpr int CLF_LG_MAXC = 8;   // fast path: classes summed over the targeted heads
+constexpr int LG_MAX_MIX = 64;   // entries of a target mix (PSVAE_MAX_TARGET_MIX)
 
 struct LangevinClf {
   int L, n_trunk, hidden, act, n_heads;
   int head_classes[4];
-  int targets[4];                 // -1: head not named by the target dict -> skipped
+  int targets[4];                 // -1: head not named by the target dict -> skipped.  Per-row instances: >= 0 marks a head some row can name
   int64_t g_trunk_w[4], g_trunk_b[4], g_head_w[4], g_head_b[4];   // offsets into the flat parameter buffer
   int s_trunk_w[4], s_trunk_b[4], s_head_w[4], s_head_b[4];       // offsets (floats) into the smem weight area
   int w_floats;                   // size of the smem weight area
@@ -50,20 +56,73 @@ __device__ __forceinline__ float lg_act_grad(int act, float a) {
   return 1.f;
 }
 
-static inline size_t langevin_smem_bytes(const LangevinClf& c) {
+// Per-row targets.  A row's targets are packed one byte per head: byte h = class + 1, 0 = head h left out for this row.
+struct LangevinRows {
+  const int32_t* targets;         // device int32 [n_heads][rows] (class, or -1: head left out), or NULL: draw from the mix
+  int32_t* targets_out;           // mix: the drawn targets, same layout
+  uint64_t mix_offset;            // Philox offset of the draw: offset0 + num_steps + 1 (no z0 or noise draw uses it)
+  int n_mix;
+  uint32_t mix[LG_MAX_MIX];       // packed targets of entry k
+  uint32_t thr[LG_MAX_MIX - 1];   // a row takes the first entry k < n_mix - 1 with u < thr[k], else the last
+};
+
+// The packed targets of row r (global row row0 + r).  A device target outside [-1, classes) or a row that names no head sets `bad` and returns
+// class 0 of every head the instance staged, so that the row computes NaN from its NaN z without an out-of-range class index.
+__device__ __forceinline__ uint32_t lg_row_targets(const LangevinClf& c, const LangevinRows& rt, int64_t rows, int64_t r, int64_t row0, uint64_t seed,
+                                                   bool store, bool& bad) {
+  uint32_t p = 0;
+  bad = false;
+  if (rt.targets) {
+    for (int h = 0; h < c.n_heads; ++h) {
+      const int t = rt.targets[(int64_t)h * rows + r];
+      bad |= t < -1 || t >= c.head_classes[h];
+      p |= (uint32_t)((t + 1) & 0xFF) << (8 * h);
+    }
+    bad |= p == 0;
+  } else {
+    // word row0 + r of the uint32 stream at offset mix_offset: the layout of psvae_philox_uint32 (oracle/philox_ref.philox_uint32)
+    const uint64_t g = (uint64_t)(row0 + r);
+    const uint4 w = philox4x32_10((uint32_t)(g >> 2), (uint32_t)(g >> 34), (uint32_t)rt.mix_offset, (uint32_t)(rt.mix_offset >> 32), (uint32_t)seed,
+                                  (uint32_t)(seed >> 32));
+    const uint32_t u = (g & 3) == 0 ? w.x : (g & 3) == 1 ? w.y : (g & 3) == 2 ? w.z : w.w;
+    int k = 0;
+    while (k < rt.n_mix - 1 && u >= rt.thr[k]) ++k;
+    p = rt.mix[k];
+    if (store)
+      for (int h = 0; h < c.n_heads; ++h) rt.targets_out[(int64_t)h * rows + r] = (int)((p >> (8 * h)) & 0xFF) - 1;
+  }
+  if (bad) {
+    p = 0;
+    for (int h = 0; h < c.n_heads; ++h)
+      if (c.targets[h] >= 0) p |= 1u << (8 * h);
+  }
+  return p;
+}
+
+// Target of head h: the shared one, or from the row's packed targets (-1: left out)
+template <bool ROW_TARGETS>
+__device__ __forceinline__ int lg_target(const LangevinClf& c, uint32_t tp, int h) {
+  if constexpr (ROW_TARGETS) return (int)((tp >> (8 * h)) & 0xFF) - 1;
+  else return c.targets[h];
+}
+
+static inline size_t langevin_smem_bytes(const LangevinClf& c, bool row_targets = false) {
   const int ldz = c.L + 1, ldh = c.hidden + 1;
   size_t f = (size_t)c.w_floats + (size_t)LG_TILE * ldz                // weights, z
              + (size_t)c.n_trunk * LG_TILE * ldh                       // trunk activations
              + 2 * (size_t)LG_TILE * (c.hidden > c.L ? ldh : ldz)      // gradient ping-pong
-             + (size_t)4 * LG_TILE * (LG_MAXC + 1);                    // logits / dlogits per head
+             + (size_t)4 * LG_TILE * (LG_MAXC + 1)                     // logits / dlogits per head
+             + (row_targets ? (size_t)2 * LG_TILE : 0);                // per-row instance: packed targets, bad-row flags
   return f * sizeof(float);
 }
 
+template <bool ROW_TARGETS>
 __global__ void __launch_bounds__(LG_THREADS) langevin_kernel(LangevinClf c, const float* __restrict__ params, float* __restrict__ z_io,
                                                               int64_t rows, float step_size, int num_steps, float noise_weight, uint64_t seed,
                                                               uint64_t offset0, int64_t row0, int init_from_philox, const float* __restrict__ noise,
                                                               float* __restrict__ history, float* __restrict__ stats, float prior_weight, float threshold,
-                                                              int32_t* __restrict__ stop_step, float* __restrict__ last_prob) {
+                                                              int32_t* __restrict__ stop_step, float* __restrict__ last_prob,
+                                                              const __grid_constant__ LangevinRows rt) {
   PSVAE_GRID_DEP();
   extern __shared__ float lg_smem[];
   __shared__ int lg_done[LG_TILE], lg_hit[LG_TILE];      // per sample: stopped (threshold reached at an earlier step) / reaches it at this step
@@ -77,11 +136,23 @@ __global__ void __launch_bounds__(LG_THREADS) langevin_kernel(LangevinClf c, con
   float* d0 = acts + c.n_trunk * LG_TILE * ldh;
   float* d1 = d0 + LG_TILE * ldd;
   float* lgt = d1 + LG_TILE * ldd;
+  uint32_t* tgt_s = reinterpret_cast<uint32_t*>(lgt + 4 * LG_TILE * ldc);   // per-row instance: packed targets of the tile's rows
+  int* bad_s = reinterpret_cast<int*>(tgt_s + LG_TILE);
 
   const int tid = threadIdx.x, s = tid & 31, g = tid >> 5;
   const int64_t tile_row0 = (int64_t)blockIdx.x * LG_TILE;
   const int64_t row = tile_row0 + s;
   const bool live = row < rows;
+  uint32_t tp = 0;                                   // per-row instance: the packed targets of this lane's sample
+  if constexpr (ROW_TARGETS) {
+    if (tid < LG_TILE) {
+      bool bad = false;
+      tgt_s[tid] = tile_row0 + tid < rows ? lg_row_targets(c, rt, rows, tile_row0 + tid, row0, seed, true, bad) : 0u;
+      bad_s[tid] = bad;
+    }
+    __syncthreads();
+    tp = tgt_s[s];
+  }
 
   // stage classifier weights once
   for (int j = 0; j < c.n_trunk; ++j) {
@@ -106,6 +177,9 @@ __global__ void __launch_bounds__(LG_THREADS) langevin_kernel(LangevinClf c, con
         v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
       } else {
         load_vec<4>(z_io + r * L + qk, v);
+      }
+      if constexpr (ROW_TARGETS) {
+        if (bad_s[qs]) v[0] = v[1] = v[2] = v[3] = __int_as_float(0x7fffffff);
       }
     }
 #pragma unroll
@@ -157,6 +231,9 @@ __global__ void __launch_bounds__(LG_THREADS) langevin_kernel(LangevinClf c, con
       float lp_y = 0.f;
       for (int h = 0; h < c.n_heads; ++h) {
         if (c.targets[h] < 0) continue;
+        if constexpr (ROW_TARGETS) {
+          if (lg_target<true>(c, tp, h) < 0) continue;
+        }
         float* lg = lgt + (h * LG_TILE + s) * ldc;
         const int C = c.head_classes[h];
         float mx = lg[0];
@@ -164,8 +241,11 @@ __global__ void __launch_bounds__(LG_THREADS) langevin_kernel(LangevinClf c, con
         float se = 0.f;
         for (int k = 0; k < C; ++k) se += expf(lg[k] - mx);
         const float lse = logf(se);
-        lp_y += lg[c.targets[h]] - mx - lse;
-        for (int k = 0; k < C; ++k) lg[k] = (k == c.targets[h] ? 1.f : 0.f) - expf(lg[k] - mx - lse);
+        lp_y += lg[lg_target<ROW_TARGETS>(c, tp, h)] - mx - lse;
+        for (int k = 0; k < C; ++k) lg[k] = (k == lg_target<ROW_TARGETS>(c, tp, h) ? 1.f : 0.f) - expf(lg[k] - mx - lse);
+      }
+      if constexpr (ROW_TARGETS) {
+        if (bad_s[s]) lp_y = __int_as_float(0x7fffffff);   // a ReLU / sigmoid trunk can map a NaN z to finite logits
       }
       if (!lg_done[s]) {
         const float p = expf(lp_y);
@@ -192,6 +272,9 @@ __global__ void __launch_bounds__(LG_THREADS) langevin_kernel(LangevinClf c, con
       float a = 0.f;
       for (int h = 0; h < c.n_heads; ++h) {
         if (c.targets[h] < 0) continue;
+        if constexpr (ROW_TARGETS) {
+          if (lg_target<true>(c, tp, h) < 0) continue;
+        }
         const float* Wh = W + c.s_head_w[h];
         const float* dl = lgt + (h * LG_TILE + s) * ldc;
         for (int o = 0; o < c.head_classes[h]; ++o) a = fmaf(dl[o], Wh[o * Kf + k], a);
@@ -283,12 +366,15 @@ namespace psvae {
 // ------------------------------------------------------------------------------------------------
 constexpr int LGF_THREADS = 128;
 
-template <int L>
+// Per-row instance: the block stages every head some row can name; a thread skips, in every loop over classes, the heads its row leaves out
+// (skipped, not multiplied by a zero coefficient, which could turn a -0 gradient into +0).
+template <int L, bool ROW_TARGETS>
 __global__ void __launch_bounds__(LGF_THREADS) langevin_fast_kernel(LangevinClf c, const float* __restrict__ params, float* __restrict__ z_io, int64_t rows,
                                                                     float step_size, int num_steps, float noise_weight, uint64_t seed, uint64_t offset0,
                                                                     int64_t row0, int init_from_philox, const float* __restrict__ noise,
                                                                     float* __restrict__ history, float* __restrict__ stats, float prior_weight, float threshold,
-                                                                    int32_t* __restrict__ stop_step, float* __restrict__ last_prob) {
+                                                                    int32_t* __restrict__ stop_step, float* __restrict__ last_prob,
+                                                                    const __grid_constant__ LangevinRows rt) {
   PSVAE_GRID_DEP();
   __shared__ __align__(16) float W[CLF_LG_MAXC * L];
   __shared__ float bias[CLF_LG_MAXC];
@@ -310,6 +396,17 @@ __global__ void __launch_bounds__(LGF_THREADS) langevin_fast_kernel(LangevinClf 
   const bool live = r < rows;
   const int64_t rr = live ? r : rows - 1;                 // dead lanes shadow the last row (no stores) so that warp-collectives stay converged
   const uint64_t q0 = (uint64_t)((row0 + rr) * L) >> 2;   // first Philox block of this row
+  uint32_t tp = 0, cmask = 0;           // per-row instance: this row's packed targets, and the staged classes cc of the heads it names
+  bool bad = false;
+  if constexpr (ROW_TARGETS) {
+    tp = lg_row_targets(c, rt, rows, rr, row0, seed, live, bad);
+    int base = 0;
+    for (int h = 0; h < c.n_heads; ++h) {
+      if (c.targets[h] < 0) continue;
+      if ((tp >> (8 * h)) & 0xFF) cmask |= ((1u << c.head_classes[h]) - 1u) << base;
+      base += c.head_classes[h];
+    }
+  }
   float z[L];
   auto draw = [&](uint64_t offset) {
 #pragma unroll 2
@@ -329,6 +426,10 @@ __global__ void __launch_bounds__(LGF_THREADS) langevin_fast_kernel(LangevinClf 
       z[4 * q] = t.x; z[4 * q + 1] = t.y; z[4 * q + 2] = t.z; z[4 * q + 3] = t.w;
     }
   }
+  if (ROW_TARGETS && bad) {
+#pragma unroll
+    for (int k = 0; k < L; ++k) z[k] = __int_as_float(0x7fffffff);
+  }
   const float half_s2 = 0.5f * step_size * step_size;
   const float nscale = step_size * noise_weight;
   bool active = true;                    // false once p(y|z) has exceeded the threshold (this sample's z is final)
@@ -341,7 +442,7 @@ __global__ void __launch_bounds__(LGF_THREADS) langevin_fast_kernel(LangevinClf 
 #pragma unroll
     for (int cc = 0; cc < CLF_LG_MAXC; ++cc) {
       float a = 0.f;
-      if (cc < n_cls) {
+      if (cc < n_cls && (!ROW_TARGETS || ((cmask >> cc) & 1u))) {
         a = bias[cc];
 #pragma unroll
         for (int k = 0; k < L; k += 4) {
@@ -358,6 +459,9 @@ __global__ void __launch_bounds__(LGF_THREADS) langevin_fast_kernel(LangevinClf 
       for (int h = 0; h < c.n_heads; ++h) {
         if (c.targets[h] < 0) continue;
         const int C = c.head_classes[h];
+        if constexpr (ROW_TARGETS) {
+          if (lg_target<true>(c, tp, h) < 0) { base += C; continue; }
+        }
         float mx = -INFINITY;
 #pragma unroll
         for (int cc = 0; cc < CLF_LG_MAXC; ++cc)
@@ -371,7 +475,7 @@ __global__ void __launch_bounds__(LGF_THREADS) langevin_fast_kernel(LangevinClf 
         for (int cc = 0; cc < CLF_LG_MAXC; ++cc)
           if (cc >= base && cc < base + C) {
             const float lp = coef[cc] - mx - lse;
-            const bool tgt = (cc - base) == c.targets[h];
+            const bool tgt = (cc - base) == lg_target<ROW_TARGETS>(c, tp, h);
             if (tgt) lp_y += lp;
             coef[cc] = (tgt ? 1.f : 0.f) - expf(lp);
           }
@@ -409,7 +513,7 @@ __global__ void __launch_bounds__(LGF_THREADS) langevin_fast_kernel(LangevinClf 
       float g[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
       for (int cc = 0; cc < CLF_LG_MAXC; ++cc)
-        if (cc < n_cls) {
+        if (cc < n_cls && (!ROW_TARGETS || ((cmask >> cc) & 1u))) {
           const float4 w = *reinterpret_cast<const float4*>(&W[cc * L + 4 * q]);
           g[0] = fmaf(coef[cc], w.x, g[0]); g[1] = fmaf(coef[cc], w.y, g[1]); g[2] = fmaf(coef[cc], w.z, g[2]); g[3] = fmaf(coef[cc], w.w, g[3]);
         }

@@ -2143,6 +2143,68 @@ int psvae_decode(const psvae_model_desc* desc, const float* params, const void* 
              : run_decode<float>(desc, params, nullptr, z, seed, offset, row0, rows, x_hat, z_out, workspace, workspace_bytes, st);
 }
 
+}  // extern "C"
+
+// The classifier part of LangevinClf (everything but the targets) from the model description.
+static LangevinClf langevin_clf(const psvae_model_desc* desc) {
+  Net n(desc);
+  LangevinClf c;
+  memset(&c, 0, sizeof(c));
+  c.L = n.L; c.n_trunk = desc->clf_num_trunk; c.hidden = desc->clf_num_trunk ? desc->clf_hidden : 0;
+  c.act = desc->clf_activation; c.n_heads = desc->clf_num_heads;
+  int off = 0;
+  for (int t = 0; t < c.n_trunk; ++t) {
+    c.g_trunk_w[t] = desc->clf_trunk_w[t]; c.g_trunk_b[t] = desc->clf_trunk_b[t];
+    c.s_trunk_w[t] = off; off += desc->clf_hidden * n.clf_trunk_in(t);
+    c.s_trunk_b[t] = off; off += desc->clf_hidden;
+  }
+  for (int h = 0; h < c.n_heads; ++h) {
+    c.head_classes[h] = desc->clf_head_classes[h];
+    c.g_head_w[h] = desc->clf_head_w[h]; c.g_head_b[h] = desc->clf_head_b[h];
+    c.s_head_w[h] = off; off += c.head_classes[h] * n.clf_feat();
+    c.s_head_b[h] = off; off += c.head_classes[h];
+  }
+  for (int h = 0; h < 4; ++h) c.targets[h] = -1;
+  c.w_floats = off;
+  return c;
+}
+
+// Launch the Langevin loop: the shared-target instances for rt == NULL, the per-row ones otherwise.  c.targets[h] >= 0 marks the heads the
+// kernel stages (and, for the shared instances, their targets).
+template <bool ROW_TARGETS>
+static int langevin_launch(const LangevinClf& c, const LangevinRows& rt, const float* params, float* z_io, int64_t rows, float step_size,
+                           int32_t num_steps, float noise_weight, uint64_t seed, uint64_t offset0, int64_t row0, int32_t init_from_philox,
+                           const float* noise, float* history, float* stats, float prior_weight, float threshold, int32_t* stop_step,
+                           float* last_prob, cudaStream_t st) {
+  if (stats && num_steps > 0) PSVAE_CUDA(cudaMemsetAsync(stats, 0, sizeof(float) * 2 * (size_t)num_steps, st));
+  // fast path: linear heads on z, one thread per sample (langevin_fast_kernel)
+  int targeted_classes = 0;
+  for (int h = 0; h < c.n_heads; ++h)
+    if (c.targets[h] >= 0) targeted_classes += c.head_classes[h];
+  if (c.n_trunk == 0 && targeted_classes <= CLF_LG_MAXC && (c.L == 16 || c.L == 32 || c.L == 64) && !g_opt.langevin_generic) {
+    const unsigned gridf = (unsigned)ceil_div64(rows, LGF_THREADS);
+    switch (c.L) {
+      case 16: launch_dep(langevin_fast_kernel<16, ROW_TARGETS>, dim3(gridf), dim3(LGF_THREADS), 0, st, c, params, z_io, rows, step_size, num_steps, noise_weight, seed, offset0, row0, init_from_philox, noise, history, stats, prior_weight, threshold, stop_step, last_prob, rt); break;
+      case 32: launch_dep(langevin_fast_kernel<32, ROW_TARGETS>, dim3(gridf), dim3(LGF_THREADS), 0, st, c, params, z_io, rows, step_size, num_steps, noise_weight, seed, offset0, row0, init_from_philox, noise, history, stats, prior_weight, threshold, stop_step, last_prob, rt); break;
+      default: launch_dep(langevin_fast_kernel<64, ROW_TARGETS>, dim3(gridf), dim3(LGF_THREADS), 0, st, c, params, z_io, rows, step_size, num_steps, noise_weight, seed, offset0, row0, init_from_philox, noise, history, stats, prior_weight, threshold, stop_step, last_prob, rt); break;
+    }
+    count_launch();
+    PSVAE_LAUNCH_CHECK("langevin_fast_kernel");
+    return 0;
+  }
+  const size_t smem = langevin_smem_bytes(c, ROW_TARGETS);
+  if (smem > 227 * 1024) { set_error("classifier too large for the Langevin kernel's shared memory (%zu bytes)", smem); return -2; }
+  PSVAE_CUDA(cudaFuncSetAttribute(langevin_kernel<ROW_TARGETS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const unsigned grid = (unsigned)ceil_div64(rows, LG_TILE);
+  launch_dep(langevin_kernel<ROW_TARGETS>, dim3(grid), dim3(LG_THREADS), smem, st, c, params, z_io, rows, step_size, num_steps, noise_weight, seed, offset0,
+             row0, init_from_philox, noise, history, stats, prior_weight, threshold, stop_step, last_prob, rt);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("langevin_kernel");
+  return 0;
+}
+
+extern "C" {
+
 int psvae_langevin(const psvae_model_desc* desc, const float* params, float* z_io, int64_t rows, const int32_t* targets_host, float step_size,
                    int32_t num_steps, float noise_weight, uint64_t seed, uint64_t offset0, int64_t row0, int32_t init_from_philox,
                    const float* noise, float* history, float* stats, float prior_weight, float threshold, int32_t* stop_step, float* last_prob,
@@ -2153,55 +2215,66 @@ int psvae_langevin(const psvae_model_desc* desc, const float* params, float* z_i
   if (desc->clf_num_heads <= 0) { set_error("conditional synthesis needs a latent classifier (ps_vae/inference.py:80)"); return -2; }
   if (rows <= 0) { set_error("rows must be positive"); return -2; }
   if (num_steps < 0) { set_error("num_steps must be >= 0"); return -2; }
-  Net n(desc);
-  LangevinClf c;
-  memset(&c, 0, sizeof(c));
-  c.L = n.L; c.n_trunk = desc->clf_num_trunk; c.hidden = desc->clf_num_trunk ? desc->clf_hidden : 0;
-  c.act = desc->clf_activation; c.n_heads = desc->clf_num_heads;
-  int any = 0, off = 0;
-  for (int t = 0; t < c.n_trunk; ++t) {
-    c.g_trunk_w[t] = desc->clf_trunk_w[t]; c.g_trunk_b[t] = desc->clf_trunk_b[t];
-    c.s_trunk_w[t] = off; off += desc->clf_hidden * n.clf_trunk_in(t);
-    c.s_trunk_b[t] = off; off += desc->clf_hidden;
-  }
+  LangevinClf c = langevin_clf(desc);
+  int any = 0;
   for (int h = 0; h < c.n_heads; ++h) {
-    c.head_classes[h] = desc->clf_head_classes[h];
     c.targets[h] = targets_host[h];
     if (c.targets[h] >= c.head_classes[h]) { set_error("target %d of head %d is out of range (%d classes)", c.targets[h], h, c.head_classes[h]); return -2; }
     if (c.targets[h] >= 0) any = 1;
-    c.g_head_w[h] = desc->clf_head_w[h]; c.g_head_b[h] = desc->clf_head_b[h];
-    c.s_head_w[h] = off; off += c.head_classes[h] * n.clf_feat();
-    c.s_head_b[h] = off; off += c.head_classes[h];
   }
-  for (int h = c.n_heads; h < 4; ++h) c.targets[h] = -1;
   if (!any) { set_error("classifier_target selects no head"); return -2; }
-  c.w_floats = off;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (stats && num_steps > 0) PSVAE_CUDA(cudaMemsetAsync(stats, 0, sizeof(float) * 2 * (size_t)num_steps, st));
-  // fast path: linear heads on z, one thread per sample (langevin_fast_kernel)
-  int targeted_classes = 0;
-  for (int h = 0; h < c.n_heads; ++h)
-    if (c.targets[h] >= 0) targeted_classes += c.head_classes[h];
-  if (c.n_trunk == 0 && targeted_classes <= CLF_LG_MAXC && (n.L == 16 || n.L == 32 || n.L == 64) && !g_opt.langevin_generic) {
-    const unsigned gridf = (unsigned)ceil_div64(rows, LGF_THREADS);
-    switch (n.L) {
-      case 16: launch_dep(langevin_fast_kernel<16>, dim3(gridf), dim3(LGF_THREADS), 0, st, c, params, z_io, rows, step_size, num_steps, noise_weight, seed, offset0, row0, init_from_philox, noise, history, stats, prior_weight, threshold, stop_step, last_prob); break;
-      case 32: launch_dep(langevin_fast_kernel<32>, dim3(gridf), dim3(LGF_THREADS), 0, st, c, params, z_io, rows, step_size, num_steps, noise_weight, seed, offset0, row0, init_from_philox, noise, history, stats, prior_weight, threshold, stop_step, last_prob); break;
-      default: launch_dep(langevin_fast_kernel<64>, dim3(gridf), dim3(LGF_THREADS), 0, st, c, params, z_io, rows, step_size, num_steps, noise_weight, seed, offset0, row0, init_from_philox, noise, history, stats, prior_weight, threshold, stop_step, last_prob); break;
+  LangevinRows rt;
+  memset(&rt, 0, sizeof(rt));
+  return langevin_launch<false>(c, rt, params, z_io, rows, step_size, num_steps, noise_weight, seed, offset0, row0, init_from_philox, noise, history,
+                                stats, prior_weight, threshold, stop_step, last_prob, static_cast<cudaStream_t>(stream));
+}
+
+int psvae_langevin_rows(const psvae_model_desc* desc, const float* params, float* z_io, int64_t rows, const int32_t* row_targets, int32_t n_mix,
+                        const int32_t* mix_targets_host, const uint32_t* mix_thresholds_host, int32_t* row_targets_out, float step_size,
+                        int32_t num_steps, float noise_weight, uint64_t seed, uint64_t offset0, int64_t row0, int32_t init_from_philox,
+                        const float* noise, float* history, float* stats, float prior_weight, float threshold, int32_t* stop_step, float* last_prob,
+                        void* stream) {
+  static_assert(PSVAE_MAX_TARGET_MIX == LG_MAX_MIX, "target mix capacity");
+  // argument checks first: they do not need a device
+  PSVAE_TRY(check_desc(desc, PSVAE_FP32));
+  if (desc->clf_num_heads <= 0) { set_error("conditional synthesis needs a latent classifier (ps_vae/inference.py:80)"); return -2; }
+  if (n_mix < 0 || n_mix > PSVAE_MAX_TARGET_MIX) { set_error("n_mix=%d out of range [0,%d]", n_mix, PSVAE_MAX_TARGET_MIX); return -2; }
+  if ((row_targets != nullptr) == (n_mix > 0)) { set_error("give exactly one of row_targets and a target mix (n_mix >= 1)"); return -2; }
+  LangevinClf c = langevin_clf(desc);
+  LangevinRows rt;
+  memset(&rt, 0, sizeof(rt));
+  rt.targets = row_targets;
+  if (row_targets) {
+    for (int h = 0; h < c.n_heads; ++h) c.targets[h] = 0;         // any head can be named by some row
+  } else {
+    if (!mix_targets_host || (n_mix > 1 && !mix_thresholds_host)) { set_error("a target mix needs its targets and n_mix - 1 thresholds"); return -1; }
+    if (!row_targets_out) { set_error("a target mix needs row_targets_out for the drawn targets"); return -1; }
+    rt.targets_out = row_targets_out;
+    rt.n_mix = n_mix;
+    rt.mix_offset = offset0 + (uint64_t)num_steps + 1;
+    for (int k = 0; k < n_mix; ++k) {
+      uint32_t p = 0;
+      for (int h = 0; h < PSVAE_MAX_CLF_HEADS; ++h) {
+        const int t = mix_targets_host[k * PSVAE_MAX_CLF_HEADS + h];
+        if (t == -1) continue;
+        if (h >= c.n_heads || t < 0 || t >= c.head_classes[h]) { set_error("mix entry %d: target %d of head %d is out of range", k, t, h); return -2; }
+        p |= (uint32_t)(t + 1) << (8 * h);
+        c.targets[h] = 0;
+      }
+      if (!p) { set_error("mix entry %d names no head", k); return -2; }
+      rt.mix[k] = p;
     }
-    count_launch();
-    PSVAE_LAUNCH_CHECK("langevin_fast_kernel");
-    return 0;
+    for (int k = 0; k + 1 < n_mix; ++k) {
+      rt.thr[k] = mix_thresholds_host[k];
+      if (k > 0 && rt.thr[k] < rt.thr[k - 1]) { set_error("mix thresholds must not decrease (entry %d)", k); return -2; }
+    }
   }
-  const size_t smem = langevin_smem_bytes(c);
-  if (smem > 227 * 1024) { set_error("classifier too large for the Langevin kernel's shared memory (%zu bytes)", smem); return -2; }
-  PSVAE_CUDA(cudaFuncSetAttribute(langevin_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const unsigned grid = (unsigned)ceil_div64(rows, LG_TILE);
-  launch_dep(langevin_kernel, dim3(grid), dim3(LG_THREADS), smem, st, c, params, z_io, rows, step_size, num_steps, noise_weight, seed, offset0, row0, init_from_philox,
-                                                  noise, history, stats, prior_weight, threshold, stop_step, last_prob);
-  count_launch();
-  PSVAE_LAUNCH_CHECK("langevin_kernel");
-  return 0;
+  PSVAE_TRY(tc_device_check());
+  if (!params || !z_io) { set_error("params, z_io must not be NULL"); return -1; }
+  if (rows <= 0) { set_error("rows must be positive"); return -2; }
+  if (num_steps < 0) { set_error("num_steps must be >= 0"); return -2; }
+  return langevin_launch<true>(c, rt, params, z_io, rows, step_size, num_steps, noise_weight, seed, offset0, row0, init_from_philox, noise, history,
+                               stats, prior_weight, threshold, stop_step, last_prob, static_cast<cudaStream_t>(stream));
 }
 
 int psvae_gemm_bf16(const void* a_bf16, const void* b_bf16, const float* bias, float* c, int64_t m, int32_t n, int64_t k, int32_t a_mn, int32_t b_mn,

@@ -16,6 +16,7 @@ import ctypes as C
 import weakref
 from typing import Dict, List, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 import torch.nn as nn
 
@@ -605,18 +606,116 @@ class HotPath:
             raise KeyError(unknown[0])
         return out
 
+    def row_targets_for(self, classifier_target, num_samples: int, device, check: bool = False) -> Optional[torch.Tensor]:
+        """The device int32 ``[n_heads][N]`` targets of a per-row ``classifier_target``, or None for a shared one (an int, a 0-d tensor, a
+        dict of ints).  Per row: a 1-D integer tensor / array of length N (single-label), or a dict whose values are ints (broadcast) or
+        length-N integer tensors (multi-label); a label the dict leaves out, and -1 inside a tensor, leave that head out for the row.
+        ``check`` validates the values on the host (one synchronisation) and raises IndexError / ValueError as ``targets_for`` does;
+        without it a bad row comes out of the kernel as NaN."""
+        def per_row(v):
+            return isinstance(v, (torch.Tensor, np.ndarray)) and v.ndim >= 1
+
+        def vec(v, what):
+            t = v if isinstance(v, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(v))
+            if t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+                raise TypeError(f"{what} must be an integer tensor, got {t.dtype}")
+            if t.dim() != 1 or t.shape[0] != N:
+                raise ValueError(f"{what} must be 1-D with {N} rows, got shape {tuple(t.shape)}")
+            # clamp before the int32 cast so that no out-of-range value wraps into a valid class
+            return t.to(device=device, dtype=torch.int64, non_blocking=True).clamp(-2, 127).to(torch.int32)
+
+        c = self.classifier
+        if c is None:
+            raise ValueError("conditional synthesis needs a model with a latent classifier")
+        N = int(num_samples)
+        if isinstance(classifier_target, dict):
+            if not any(per_row(v) for v in classifier_target.values()):
+                return None
+            if c.single_label_mode:
+                raise ValueError("classifier_target must be an int or a 1-D tensor for a single-label classifier")
+            unknown = [k for k in classifier_target if k not in self.head_names]
+            if unknown:
+                raise KeyError(unknown[0])
+            out = torch.full((len(c.head_classes), N), -1, dtype=torch.int32, device=device)
+            for h, (name, ncls) in enumerate(zip(self.head_names, c.head_classes)):
+                if name not in classifier_target:
+                    continue
+                v = classifier_target[name]
+                if per_row(v):
+                    out[h] = vec(v, f"classifier_target[{name!r}]")
+                else:
+                    t = int(v)
+                    if not 0 <= t < ncls:
+                        raise IndexError(f"classifier_target[{name!r}]={t} is out of range for {ncls} classes")
+                    out[h] = t
+        elif per_row(classifier_target):
+            if not c.single_label_mode:
+                raise ValueError("classifier_target must be a dict for a multi-label classifier")
+            out = vec(classifier_target, "classifier_target").reshape(1, N)
+        else:
+            return None
+        if check and N > 0:
+            host = out.cpu().to(torch.int64)
+            for h, (name, ncls) in enumerate(zip(self.head_names, c.head_classes)):
+                bad = ((host[h] < -1) | (host[h] >= ncls)).nonzero()
+                if bad.numel():
+                    i = int(bad[0])
+                    what = "classifier_target" if c.single_label_mode else f"classifier_target[{name!r}]"
+                    raise IndexError(f"{what} of row {i} is {int(host[h, i])}: out of range for {ncls} classes")
+            none = (host < 0).all(dim=0).nonzero()
+            if none.numel():
+                raise ValueError(f"row {int(none[0])} of classifier_target names no head")
+        return out
+
+    def target_mix_for(self, target_mix) -> Tuple[List[List[int]], List[int]]:
+        """The entries (targets per head, -1 = left out) and uint32 thresholds of ``target_mix = [(target, weight), ...]``: each target is
+        what the shared form accepts, zero-weight entries are dropped (utils.mix_thresholds)."""
+        from .utils import mix_thresholds
+
+        pairs = list(target_mix)
+        if not pairs:
+            raise ValueError("target_mix is empty")
+        for p in pairs:
+            if not isinstance(p, (tuple, list)) or len(p) != 2:
+                raise ValueError(f"target_mix entry {p!r} is not a (target, weight) pair")
+        kept, thr = mix_thresholds([w for _, w in pairs], L.MAX_TARGET_MIX)
+        return [self.targets_for(pairs[i][0]) for i in kept], thr
+
+    def _targets_out(self, t: torch.Tensor):
+        """int32 [n_heads][N] kernel targets -> int64 [N] (single-label) or {label: int64 [N]}."""
+        if self.classifier.single_label_mode:
+            return t[0].to(torch.int64)
+        return {name: t[h].to(torch.int64) for h, name in enumerate(self.head_names)}
+
     def langevin(self, num_samples: int, classifier_target, step_size: float = 0.01, num_steps: int = 100, noise_weight: float = 1.0,
                  z0: Optional[torch.Tensor] = None, noise: Optional[torch.Tensor] = None, return_history: bool = False, return_stats: bool = False,
-                 row0: Optional[int] = None, prior_weight: float = 1.0, threshold: float = 0.0, return_stop: bool = False):
+                 row0: Optional[int] = None, prior_weight: float = 1.0, threshold: float = 0.0, return_stop: bool = False, *,
+                 target_mix=None, check_targets: bool = False):
         """The Langevin loop of inference.py:72-103 in one launch.  ``prior_weight`` / ``threshold`` / ``return_stop`` cover the analysis variant
         (analysis/sample_gender_transformation.py:61-99): the log p(z) term scaled by ``prior_weight``, a sample frozen after the update of the
-        first step whose p(y|z) exceeded ``threshold`` (0 = never); with ``return_stop`` the third result is ``(stats, stop_step, last_prob)``."""
+        first step whose p(y|z) exceeded ``threshold`` (0 = never); with ``return_stop`` the third result is ``(stats, stop_step, last_prob)``.
+
+        ``classifier_target`` is shared (int, dict of ints) or per row (see ``row_targets_for``; ``check_targets`` validates it on the host).
+        ``target_mix = [(target, weight), ...]`` (with ``classifier_target=None``) draws each row's target in the kernel from the global row
+        index; the drawn targets come back as a fourth result (``_targets_out`` form) and the call uses ``num_steps + 2`` Philox offsets."""
         dev = self._device()
         flat = self.arena.ensure()
         Lz = self.desc.latent_dim
-        targets = self.targets_for(classifier_target)
-        tarr = (C.c_int32 * L.MAX_CLF_HEADS)(*(targets + [-1] * (L.MAX_CLF_HEADS - len(targets))))
         N = int(num_samples)
+        rows_t = mix = None
+        if target_mix is not None:
+            if classifier_target is not None:
+                raise ValueError("give either classifier_target or target_mix, not both")
+            if self.classifier is None:
+                raise ValueError("conditional synthesis needs a model with a latent classifier")
+            mix = self.target_mix_for(target_mix)
+        else:
+            if classifier_target is None:
+                raise ValueError("conditional synthesis needs a classifier_target or a target_mix")
+            rows_t = self.row_targets_for(classifier_target, N, dev, check_targets)
+        if mix is None and rows_t is None:
+            targets = self.targets_for(classifier_target)
+            tarr = (C.c_int32 * L.MAX_CLF_HEADS)(*(targets + [-1] * (L.MAX_CLF_HEADS - len(targets))))
         if z0 is not None:
             z = self._f32(z0, dev, "z0").clone()
             if tuple(z.shape) != (N, Lz):
@@ -632,19 +731,35 @@ class HotPath:
         if self.seed is None:
             self.seed = int(torch.initial_seed()) & 0xFFFFFFFFFFFFFFFF
         off0 = self.offset
-        self.offset += num_steps + 1
+        self.offset += num_steps + (2 if mix is not None else 1)
         hist = torch.empty(num_steps, N, Lz, dtype=torch.float32, device=dev) if return_history else None
         stats = torch.empty(num_steps, 2, dtype=torch.float32, device=dev) if return_stats else None
         stop = torch.full((N,), int(num_steps), dtype=torch.int32, device=dev) if return_stop else None
         prob = torch.zeros(N, dtype=torch.float32, device=dev) if return_stop else None
-        if N > 0:
+        tout = torch.empty(len(self.classifier.head_classes), N, dtype=torch.int32, device=dev) if mix is not None else None
+        r0 = self.row0 if row0 is None else row0
+        if N > 0 and mix is None and rows_t is None:
             with _on(dev):
                 rc = L.lib().psvae_langevin(self._dref, flat.data_ptr(), z.data_ptr(), N, tarr, float(step_size), int(num_steps), float(noise_weight),
-                                            self.seed, off0, self.row0 if row0 is None else row0, init, L.ptr(noise), L.ptr(hist), L.ptr(stats),
+                                            self.seed, off0, r0, init, L.ptr(noise), L.ptr(hist), L.ptr(stats),
                                             float(prior_weight), float(threshold), L.ptr(stop), L.ptr(prob), _stream_ptr(dev))
             L.check(rc, "psvae_langevin")
+        elif N > 0:
+            n_mix, marr, tharr = 0, None, None
+            if mix is not None:
+                entries, thr = mix
+                n_mix = len(entries)
+                marr = (C.c_int32 * (n_mix * L.MAX_CLF_HEADS))(*[t for e in entries for t in e + [-1] * (L.MAX_CLF_HEADS - len(e))])
+                tharr = (C.c_uint32 * max(1, len(thr)))(*thr)
+            with _on(dev):
+                rc = L.lib().psvae_langevin_rows(self._dref, flat.data_ptr(), z.data_ptr(), N, L.ptr(rows_t), n_mix, marr, tharr, L.ptr(tout),
+                                                 float(step_size), int(num_steps), float(noise_weight), self.seed, off0, r0, init, L.ptr(noise),
+                                                 L.ptr(hist), L.ptr(stats), float(prior_weight), float(threshold), L.ptr(stop), L.ptr(prob),
+                                                 _stream_ptr(dev))
+            L.check(rc, "psvae_langevin_rows")
         if stats is not None and N > 0:
             stats = stats / N
-        if return_stop:
-            return z, hist, (stats, stop, prob)
-        return z, hist, stats
+        res = (z, hist, (stats, stop, prob) if return_stop else stats)
+        if mix is not None:
+            return res + (self._targets_out(tout),)
+        return res

@@ -13,6 +13,11 @@ Same signatures and return values (CPU tensors; ``(x_hat, history)`` with ``retu
 
 ``sample_on_device`` is the bulk path (BASELINE config 4): it writes into a caller-provided device buffer and
 returns without synchronising, and ``shard_rows`` gives each data-parallel rank its slice of the sample index range.
+
+Conditioning: ``classifier_target`` is one target for the batch (an int, or a dict of label -> class) or one per row (a length-N integer
+tensor, or a dict whose values are ints or length-N integer tensors; -1 leaves a head out for that row).  ``target_mix=[(target, weight),
+...]`` instead draws every row's target in the kernel from its global row index, so a population with a demographic mix comes out of one
+call, and a sharded run draws the same targets as a single call.  Every row is bit-identical to a shared-target call with that row's target.
 """
 from __future__ import annotations
 
@@ -23,7 +28,7 @@ from typing import List, Optional, Tuple, Union
 import torch
 from torch import Tensor
 
-from .utils import parse_classifier_target, sample_filename
+from .utils import parse_classifier_target, parse_target_mix, sample_filename
 
 
 def _hot(vae_model):
@@ -50,16 +55,20 @@ def shard_rows(num_samples: int, rank: int, world_size: int) -> Tuple[int, int]:
     return row0, rows
 
 
-def sample_on_device(vae_model, num_samples: int, classifier_target: Union[int, dict, None] = None, step_size: float = 0.01,
-                     num_steps: int = 100, noise_weight: float = 1.0, out: Optional[Tensor] = None, row0: int = 0) -> Tensor:
+def sample_on_device(vae_model, num_samples: int, classifier_target=None, step_size: float = 0.01, num_steps: int = 100,
+                     noise_weight: float = 1.0, out: Optional[Tensor] = None, row0: int = 0, *, target_mix=None):
     """Generate ``num_samples`` embeddings into ``out`` (device tensor) without any host synchronisation.
 
-    ``row0`` is the global index of the first sample: rank r of a sharded run passes ``shard_rows(N, r, W)``."""
+    ``row0`` is the global index of the first sample: rank r of a sharded run passes ``shard_rows(N, r, W)``.  Per-row targets are not
+    validated on the host (that would synchronise): a row with a target out of range comes out as NaN.  With ``target_mix`` the result is
+    ``(out, targets)``, the drawn targets on the device: int64 ``[N]`` for a single-label classifier, else ``{label: int64 [N]}`` (-1: head
+    left out)."""
     hot = _hot(vae_model)
-    if classifier_target is None:
+    if classifier_target is None and target_mix is None:
         return hot.decode(None, num_samples=num_samples, out=out, row0=row0)
-    z, _, _ = hot.langevin(num_samples, classifier_target, step_size, num_steps, noise_weight, row0=row0)
-    return hot.decode(z, out=out)
+    res = hot.langevin(num_samples, classifier_target, step_size, num_steps, noise_weight, row0=row0, target_mix=target_mix)
+    x = hot.decode(res[0], out=out)
+    return (x, res[3]) if target_mix is not None else x
 
 
 def unconditional_synthesis(vae_model, num_samples: int, device: str) -> Tensor:
@@ -68,23 +77,30 @@ def unconditional_synthesis(vae_model, num_samples: int, device: str) -> Tensor:
     return _hot(vae_model).decode(None, num_samples=num_samples).detach().cpu()
 
 
-def conditional_synthesis(vae_model, num_samples: int, classifier_target: Union[int, dict], step_size: float = 0.01, num_steps: int = 100,
+def conditional_synthesis(vae_model, num_samples: int, classifier_target=None, step_size: float = 0.01, num_steps: int = 100,
                           noise_weight: float = 1.0, return_history: bool = False, device: str = "cpu", *, z0: Optional[Tensor] = None,
-                          noise: Optional[Tensor] = None):
+                          noise: Optional[Tensor] = None, target_mix=None):
     """Classifier-guided Langevin dynamics in latent space, then decode (inference.py:29-110).
 
     ``z0`` / ``noise`` (keyword-only, optional) inject the initial draw and the per-step noise ``[num_steps, N, latent]``
-    for parity runs; by default both come from the in-kernel Philox generator."""
+    for parity runs; by default both come from the in-kernel Philox generator.  ``classifier_target`` may be per row (checked on the host:
+    IndexError / ValueError for a bad row).  With ``target_mix`` (and no ``classifier_target``) the drawn targets are returned last:
+    ``(x_hat, targets)`` or ``(x_hat, history, targets)``, on the CPU in the form ``sample_on_device`` gives."""
     _check_device(vae_model, device)
     hot = _hot(vae_model)
-    z, hist, _ = hot.langevin(num_samples, classifier_target, step_size, num_steps, noise_weight, z0=z0, noise=noise,
-                              return_history=return_history)
+    res = hot.langevin(num_samples, classifier_target, step_size, num_steps, noise_weight, z0=z0, noise=noise,
+                       return_history=return_history, target_mix=target_mix, check_targets=True)
+    z, hist = res[0], res[1]
     x_hat = hot.decode(z).detach().cpu()
+    out = (x_hat,)
     if return_history:
         h = hist.cpu().numpy()
         history: List = [h[i] for i in range(h.shape[0])]
-        return x_hat, history
-    return x_hat
+        out += (history,)
+    if target_mix is not None:
+        t = res[3]
+        out += ({k: v.cpu() for k, v in t.items()} if isinstance(t, dict) else t.cpu(),)
+    return out if len(out) > 1 else x_hat
 
 
 def latent_transformation(vae_model, embeddings: Tensor, classifier_target: Union[int, dict], step_size: float = 0.02, max_steps: int = 10000,
@@ -95,13 +111,15 @@ def latent_transformation(vae_model, embeddings: Tensor, classifier_target: Unio
     ``0.5 * step_size**2`` (plus ``step_size * noise_weight * N(0, I)``) and is frozen after the update of the first step whose
     ``p(y|z)`` exceeded ``threshold`` -- one kernel launch for all samples and all steps instead of a Python loop with two ``.item()`` syncs per
     step.  Returns ``(x_hat [N, D] cpu, z [N, L] cpu, stop_step [N] cpu int32 (max_steps: never stopped), prob [N] cpu)``, plus the list of
-    per-step latents with ``return_history``."""
+    per-step latents with ``return_history``.  ``classifier_target`` may be per row (each speaker its own target, e.g. the opposite of
+    its own gender; checked on the host)."""
     hot = _hot(vae_model)
     dev = hot.arena.device
     with torch.no_grad():
         _, mu, _ = hot.forward(embeddings.to(dev))
     z, hist, (_, stop, prob) = hot.langevin(mu.shape[0], classifier_target, step_size, max_steps, noise_weight, z0=mu, noise=noise,
-                                             return_history=return_history, prior_weight=prior_weight, threshold=threshold, return_stop=True)
+                                             return_history=return_history, prior_weight=prior_weight, threshold=threshold, return_stop=True,
+                                             check_targets=True)
     x_hat = hot.decode(z).detach().cpu()
     out = (x_hat, z.cpu(), stop.cpu(), prob.cpu())
     if return_history:
@@ -169,22 +187,40 @@ def main(argv=None) -> None:
     parser.add_argument("--n_samples", type=int, default=16, help="Number of samples to generate.")
     parser.add_argument("--save_dir", type=str, required=True, help="Directory to save the generated samples.")
     parser.add_argument("--synthesis_type", type=str, choices=["conditional", "unconditional"], required=True)
-    parser.add_argument("--classifier_target", type=str, default="1", help="Target class (int, or JSON dict for multi-label).")
+    parser.add_argument("--classifier_target", type=str, default=None, help="Target class (int, or JSON dict for multi-label); default 1.")
+    parser.add_argument("--target_mix", type=str, default=None,
+                        help='Draw each sample\'s target from a weighted mix, JSON [[target, weight], ...], e.g. '
+                             '\'[[{"gender": 0, "age": 1}, 0.3], [{"gender": 1, "age": 1}, 0.7]]\'; the drawn targets go to <save_dir>/targets.pt.')
     parser.add_argument("--num_steps", type=int, default=5000)
     parser.add_argument("--step_size", type=float, default=0.01)
     parser.add_argument("--noise_weight", type=float, default=1.0)
     parser.add_argument("--device", type=str, default="cuda", help="CUDA device (this implementation has no CPU path).")
     args = parser.parse_args(argv)
+    target_mix = None
+    if args.target_mix is not None:
+        if args.classifier_target is not None:
+            parser.error("--target_mix and --classifier_target are mutually exclusive")
+        if args.synthesis_type != "conditional":
+            parser.error("--target_mix needs --synthesis_type conditional")
+        try:
+            target_mix = parse_target_mix(args.target_mix)
+        except ValueError as e:
+            parser.error(str(e))
 
-    classifier_target = parse_classifier_target(args.classifier_target)
+    classifier_target = None if target_mix is not None else parse_classifier_target(args.classifier_target or "1")
     model = PseudoSpeakerVAE.load_from_checkpoint(args.vae_ckpt_path)
     model = model.to(args.device)
+    targets = None
     if args.synthesis_type == "conditional":
         x_hat = conditional_synthesis(model, classifier_target=classifier_target, num_samples=args.n_samples, num_steps=args.num_steps,
-                                      step_size=args.step_size, noise_weight=args.noise_weight, device=args.device)
+                                      step_size=args.step_size, noise_weight=args.noise_weight, device=args.device, target_mix=target_mix)
+        if target_mix is not None:
+            x_hat, targets = x_hat
     else:
         x_hat = unconditional_synthesis(model, num_samples=args.n_samples, device=args.device)
     save_samples(x_hat, args.save_dir)
+    if targets is not None:
+        torch.save(targets, os.path.join(args.save_dir, "targets.pt"))
 
 
 if __name__ == "__main__":
