@@ -1,6 +1,7 @@
 // Element-wise / reduction kernels of the hot path (everything that is not a GEMM):
-//   adam_kernel            torch.optim.Adam single-tensor update (torch/optim/adam.py:416-547) over the flat buffer
-//   grad_norm_kernel       global L2 norm + clip coefficient of clip_grad_norm_ (adam_clip_kernel applies it)
+//   adam_kernel            torch.optim.Adam single-tensor update (torch/optim/adam.py:416-547) over the flat buffer; one template
+//                          <DC, EX, CLIP> for the device-counter, amsgrad / maximize and clipped forms
+//   grad_norm_kernel       global L2 norm + clip coefficient of clip_grad_norm_ (adam_kernel<DC, EX, CLIP_NORM> applies it)
 //   philox_*_kernel        torch.randn / randn_like replacement (model.py:57, inference.py:23,73,95)
 //   cast_bf16_kernel       fp32 -> bf16 operand copies
 //   latent_fwd_kernel      sigma = exp(.5 ls); z = mu + sigma*eps; KL partial sums  (model.py:56-57, lightning.py:115-117)
@@ -76,12 +77,6 @@ __device__ __forceinline__ void adam_ex_pass(float* __restrict__ p, const float*
   }
 }
 
-__global__ void __launch_bounds__(256) adam_ex_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
-                                                      float* __restrict__ vmax, int64_t n, AdamArgs a, int amsgrad, int maximize, bf16* __restrict__ shadow) {
-  PSVAE_GRID_DEP();
-  adam_ex_pass(p, g, m, v, vmax, n, a, amsgrad, maximize, shadow);
-}
-
 template <int CLIP = CLIP_NONE>
 __device__ __forceinline__ void adam_pass(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, int64_t n,
                                           const AdamArgs& a, bf16* __restrict__ shadow, float clip = 0.f) {
@@ -116,70 +111,44 @@ __device__ __forceinline__ void adam_pass(float* __restrict__ p, const float* __
   }
 }
 
-__global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
-                                                   float* __restrict__ v, int64_t n, AdamArgs a, bf16* __restrict__ shadow) {
+// The one Adam update kernel.  EX: the amsgrad / maximize form (one element per thread and trip), else float4 (16-byte aligned buffers).
+// DC, the device-counter form (CUDA-graph replay): t = *step_done + 1 and lr = *lr come from device memory, read after the grid dependency
+// (the previous step's counter advance and a host write of the block are complete by then).  `a` arrives with lr_step / bc2_sqrt unset; they
+// are formed here in fp64 exactly as the host forms them for the other form, each rounded to fp32 once.  CLIP_NORM reads coef = *clip_coef
+// after the grid dependency (grad_norm_kernel wrote it) and runs the unclipped pass with grad_scale * coef; CLIP_VALUE clamps at clip_value.
+// The shared-memory prologue exists only where it is needed: <false, *, CLIP_NONE> is the bare pass.
+template <bool DC, bool EX, int CLIP>
+__global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                                                   float* __restrict__ vmax, int64_t n, AdamArgs a, double beta1, double beta2,
+                                                   const double* __restrict__ lr, const int64_t* __restrict__ step_done, int amsgrad, int maximize,
+                                                   bf16* __restrict__ shadow, const float* __restrict__ clip_coef, float clip_value) {
   PSVAE_GRID_DEP();
-  adam_pass(p, g, m, v, n, a, shadow);
-}
-
-// Device-counter form (CUDA-graph replay): t = *step_done + 1 and lr = *lr come from device memory, read after the grid dependency (the
-// previous step's counter advance and a host write of the block are complete by then).  `a` arrives with lr_step / bc2_sqrt unset; they are
-// formed here in fp64 exactly as psvae_adam_step forms them on the host, each rounded to fp32 once.  EX: the amsgrad / maximize form.
-template <bool EX>
-__global__ void __launch_bounds__(256) adam_dc_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
-                                                      float* __restrict__ vmax, int64_t n, AdamArgs a, double beta1, double beta2,
-                                                      const double* __restrict__ lr, const int64_t* __restrict__ step_done, int amsgrad, int maximize,
-                                                      bf16* __restrict__ shadow) {
-  PSVAE_GRID_DEP();
-  __shared__ float s_lr_step, s_bc2_sqrt;
-  if (threadIdx.x == 0) {
-    const double t = (double)(*step_done + 1);
-    const double bc1 = 1.0 - pow(beta1, t);
-    const double bc2 = 1.0 - pow(beta2, t);
-    s_lr_step = (float)(*lr / bc1);
-    s_bc2_sqrt = (float)sqrt(bc2);
+  if constexpr (DC || CLIP != CLIP_NONE) {
+    __shared__ float s_lr_step, s_bc2_sqrt, s_clip;
+    if (threadIdx.x == 0) {
+      if constexpr (DC) {
+        const double t = (double)(*step_done + 1);
+        const double bc1 = 1.0 - pow(beta1, t);
+        const double bc2 = 1.0 - pow(beta2, t);
+        s_lr_step = (float)(*lr / bc1);
+        s_bc2_sqrt = (float)sqrt(bc2);
+      }
+      if constexpr (CLIP != CLIP_NONE) s_clip = CLIP == CLIP_NORM ? a.grad_scale * *clip_coef : clip_value;
+    }
+    __syncthreads();
+    if constexpr (DC) {
+      a.lr_step = s_lr_step;
+      a.bc2_sqrt = s_bc2_sqrt;
+    }
+    if constexpr (CLIP == CLIP_NORM) a.grad_scale = s_clip;
+    if constexpr (CLIP == CLIP_VALUE) {
+      if constexpr (EX) adam_ex_pass<CLIP>(p, g, m, v, vmax, n, a, amsgrad, maximize, shadow, s_clip);
+      else adam_pass<CLIP>(p, g, m, v, n, a, shadow, s_clip);
+      return;
+    }
   }
-  __syncthreads();
-  a.lr_step = s_lr_step;
-  a.bc2_sqrt = s_bc2_sqrt;
   if constexpr (EX) adam_ex_pass(p, g, m, v, vmax, n, a, amsgrad, maximize, shadow);
   else adam_pass(p, g, m, v, n, a, shadow);
-}
-
-// The clipped forms of adam_kernel / adam_ex_kernel (EX) / adam_dc_kernel (DC): CLIP_NORM reads coef = *clip_coef after the grid dependency
-// (grad_norm_kernel wrote it) and runs the unclipped pass with grad_scale * coef, CLIP_VALUE clamps at clip_value.  The unclipped kernels
-// above stay as they are.
-template <bool DC, bool EX, int CLIP>
-__global__ void __launch_bounds__(256) adam_clip_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
-                                                        float* __restrict__ vmax, int64_t n, AdamArgs a, double beta1, double beta2,
-                                                        const double* __restrict__ lr, const int64_t* __restrict__ step_done, int amsgrad, int maximize,
-                                                        bf16* __restrict__ shadow, const float* __restrict__ clip_coef, float clip_value) {
-  PSVAE_GRID_DEP();
-  __shared__ float s_lr_step, s_bc2_sqrt, s_clip;
-  if (threadIdx.x == 0) {
-    if constexpr (DC) {
-      const double t = (double)(*step_done + 1);
-      const double bc1 = 1.0 - pow(beta1, t);
-      const double bc2 = 1.0 - pow(beta2, t);
-      s_lr_step = (float)(*lr / bc1);
-      s_bc2_sqrt = (float)sqrt(bc2);
-    }
-    s_clip = CLIP == CLIP_NORM ? a.grad_scale * *clip_coef : clip_value;
-  }
-  __syncthreads();
-  if constexpr (DC) {
-    a.lr_step = s_lr_step;
-    a.bc2_sqrt = s_bc2_sqrt;
-  }
-  const float c = s_clip;
-  if constexpr (CLIP == CLIP_NORM) {
-    a.grad_scale = c;
-    if constexpr (EX) adam_ex_pass(p, g, m, v, vmax, n, a, amsgrad, maximize, shadow);
-    else adam_pass(p, g, m, v, n, a, shadow);
-  } else {
-    if constexpr (EX) adam_ex_pass<CLIP>(p, g, m, v, vmax, n, a, amsgrad, maximize, shadow, c);
-    else adam_pass<CLIP>(p, g, m, v, n, a, shadow, c);
-  }
 }
 
 // Global L2 norm of g * scale over a list of [a, b) spans of the flat gradient buffer, and the clip coefficient of
@@ -256,18 +225,12 @@ __global__ void __launch_bounds__(256) grad_accumulate_kernel(float* __restrict_
   if (t < n) grads[t] += part[t];
 }
 
-// rng_offset += d_rng, adam_step += d_step: the end of a micro-batch that does (d_step = 1) or does not (d_step = 0) step the optimiser
+// rng_offset += d_rng, adam_step += d_step: the end of a device-counter micro-batch that does (d_step = 1) or does not (d_step = 0) step the
+// optimiser (every reader of the block has finished: it is the last launch)
 __global__ void step_counters_advance_by_kernel(uint64_t* __restrict__ rng_offset, int64_t* __restrict__ adam_step, uint64_t d_rng, int64_t d_step) {
   PSVAE_GRID_DEP();
   *rng_offset += d_rng;
   *adam_step += d_step;
-}
-
-// rng_offset += 1, adam_step += 1 at the end of a device-counter step (every reader of the block has finished: it is the last launch)
-__global__ void step_counters_advance_kernel(uint64_t* __restrict__ rng_offset, int64_t* __restrict__ adam_step) {
-  PSVAE_GRID_DEP();
-  *rng_offset += 1;
-  *adam_step += 1;
 }
 
 // ---------------------------------------------------------------- Philox

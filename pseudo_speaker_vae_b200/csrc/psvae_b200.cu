@@ -1628,98 +1628,78 @@ int64_t psvae_flops_per_sample(const psvae_model_desc* desc, int32_t mode) {
   return 2 * ((enc + dec) * 3 - enc_first + 3 * clf);
 }
 
-int psvae_adam_step(float* p, const float* g, float* m, float* v, int64_t n, double lr, double beta1, double beta2, double eps, double weight_decay,
-                    int64_t step, double grad_scale, void* shadow_bf16, void* stream) {
-  PSVAE_TRY(tc_device_check());
-  if (!p || !g || !m || !v) { set_error("p, g, m, v must not be NULL"); return -1; }
-  if (n <= 0) return 0;
-  if (step < 1) { set_error("step=%lld must be >= 1 (count after increment)", (long long)step); return -2; }
-  if (((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v)) & 15) != 0) {
-    set_error("Adam buffers must be 16-byte aligned");
-    return -2;
-  }
-  // host scalars exactly as torch's single-tensor Adam computes them: in python doubles, each rounded to fp32 once where
-  // the tensor op consumes it (torch/optim/adam.py:476-547)
-  const double bc1 = 1.0 - pow(beta1, (double)step);
-  const double bc2 = 1.0 - pow(beta2, (double)step);
-  AdamArgs a;
-  a.lr_step = (float)(lr / bc1);
-  a.bc2_sqrt = (float)sqrt(bc2);
-  a.beta1 = (float)beta1; a.beta2 = (float)beta2;
-  a.one_minus_beta1 = (float)(1.0 - beta1);
-  a.one_minus_beta2 = (float)(1.0 - beta2);
-  a.eps = (float)eps; a.weight_decay = (float)weight_decay; a.grad_scale = (float)grad_scale;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  launch_dep(adam_kernel, dim3(ew_grid(n / 4 + 1)), dim3(256), 0, st, p, g, m, v, n, a, static_cast<bf16*>(shadow_bf16));
-  count_launch();
-  PSVAE_LAUNCH_CHECK("adam_kernel");
-  return 0;
-}
-
-int psvae_adam_step_ex(float* p, const float* g, float* m, float* v, float* vmax, int64_t n, double lr, double beta1, double beta2, double eps,
-                       double weight_decay, int64_t step, double grad_scale, int32_t amsgrad, int32_t maximize, void* shadow_bf16, void* stream) {
-  if (!amsgrad && !maximize) return psvae_adam_step(p, g, m, v, n, lr, beta1, beta2, eps, weight_decay, step, grad_scale, shadow_bf16, stream);
-  PSVAE_TRY(tc_device_check());
-  if (!p || !g || !m || !v || (amsgrad && !vmax)) { set_error("p, g, m, v (and vmax with amsgrad) must not be NULL"); return -1; }
-  if (n <= 0) return 0;
-  if (step < 1) { set_error("step=%lld must be >= 1 (count after increment)", (long long)step); return -2; }
-  const double bc1 = 1.0 - pow(beta1, (double)step);
-  const double bc2 = 1.0 - pow(beta2, (double)step);
-  AdamArgs a;
-  a.lr_step = (float)(lr / bc1);
-  a.bc2_sqrt = (float)sqrt(bc2);
-  a.beta1 = (float)beta1; a.beta2 = (float)beta2;
-  a.one_minus_beta1 = (float)(1.0 - beta1);
-  a.one_minus_beta2 = (float)(1.0 - beta2);
-  a.eps = (float)eps; a.weight_decay = (float)weight_decay; a.grad_scale = (float)grad_scale;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  launch_dep(adam_ex_kernel, dim3(ew_grid(n)), dim3(256), 0, st, p, g, m, v, vmax, n, a, (int)amsgrad, (int)maximize, static_cast<bf16*>(shadow_bf16));
-  count_launch();
-  PSVAE_LAUNCH_CHECK("adam_ex_kernel");
-  return 0;
-}
-
-int psvae_adam_step_dc(float* p, const float* g, float* m, float* v, float* vmax, int64_t n, const double* lr, const psvae_step_counters* counters,
-                       double beta1, double beta2, double eps, double weight_decay, double grad_scale, int32_t amsgrad, int32_t maximize, void* shadow_bf16,
+// The Adam update behind every psvae_adam_step* entry point.  dc: the device-counter form (lr_dev, counters), else the host form (lr, step).
+// Without amsgrad and maximize the pass reads float4: the buffers must be 16-byte aligned.
+static int adam_update(bool dc, float* p, const float* g, float* m, float* v, float* vmax, int64_t n, double lr, int64_t step, const double* lr_dev,
+                       const psvae_step_counters* counters, double beta1, double beta2, double eps, double weight_decay, double grad_scale,
+                       int32_t amsgrad, int32_t maximize, int32_t clip_mode, const float* clip_coef, double clip_value, void* shadow_bf16,
                        void* stream) {
   PSVAE_TRY(tc_device_check());
-  if (!p || !g || !m || !v || !lr || !counters || (amsgrad && !vmax)) {
-    set_error("p, g, m, v, lr, counters (and vmax with amsgrad) must not be NULL");
+  if (clip_mode != PSVAE_CLIP_NONE && clip_mode != PSVAE_CLIP_NORM && clip_mode != PSVAE_CLIP_VALUE) {
+    set_error("clip_mode=%d is not a PSVAE_CLIP_* value", (int)clip_mode);
+    return -2;
+  }
+  if (!p || !g || !m || !v || (amsgrad && !vmax) || (dc && (!lr_dev || !counters)) || (clip_mode == PSVAE_CLIP_NORM && !clip_coef)) {
+    set_error("p, g, m, v (vmax with amsgrad, lr and counters in the device-counter form, clip_coef with PSVAE_CLIP_NORM) must not be NULL");
     return -1;
   }
+  if (clip_mode == PSVAE_CLIP_VALUE && !(clip_value >= 0.0)) { set_error("clip_value=%g must be >= 0", clip_value); return -2; }
   if (n <= 0) return 0;
+  if (!dc && step < 1) { set_error("step=%lld must be >= 1 (count after increment)", (long long)step); return -2; }
   const bool ex = amsgrad || maximize;
   if (!ex && ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v)) & 15) != 0) {
     set_error("Adam buffers must be 16-byte aligned");
     return -2;
   }
-  AdamArgs a;      // lr_step / bc2_sqrt are formed on the device from *lr and the step counter
-  a.lr_step = 0.f; a.bc2_sqrt = 1.f;
+  AdamArgs a;
+  if (dc) {                  // formed on the device from *lr_dev and the step counter
+    a.lr_step = 0.f; a.bc2_sqrt = 1.f;
+  } else {
+    // host scalars exactly as torch's single-tensor Adam computes them: in python doubles, each rounded to fp32 once where
+    // the tensor op consumes it (torch/optim/adam.py:476-547)
+    const double bc1 = 1.0 - pow(beta1, (double)step);
+    const double bc2 = 1.0 - pow(beta2, (double)step);
+    a.lr_step = (float)(lr / bc1);
+    a.bc2_sqrt = (float)sqrt(bc2);
+  }
   a.beta1 = (float)beta1; a.beta2 = (float)beta2;
   a.one_minus_beta1 = (float)(1.0 - beta1);
   a.one_minus_beta2 = (float)(1.0 - beta2);
   a.eps = (float)eps; a.weight_decay = (float)weight_decay; a.grad_scale = (float)grad_scale;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  bf16* sh = static_cast<bf16*>(shadow_bf16);
-  if (ex)
-    launch_dep(adam_dc_kernel<true>, dim3(ew_grid(n)), dim3(256), 0, st, p, g, m, v, vmax, n, a, beta1, beta2, lr, &counters->adam_step, (int)amsgrad,
-               (int)maximize, sh);
-  else
-    launch_dep(adam_dc_kernel<false>, dim3(ew_grid(n / 4 + 1)), dim3(256), 0, st, p, g, m, v, (float*)nullptr, n, a, beta1, beta2, lr, &counters->adam_step,
-               0, 0, sh);
+  static_assert(CLIP_NONE == PSVAE_CLIP_NONE && CLIP_NORM == PSVAE_CLIP_NORM && CLIP_VALUE == PSVAE_CLIP_VALUE, "kernels[dc][ex][clip_mode]");
+  static decltype(&adam_kernel<false, false, CLIP_NONE>) const kernels[2][2][3] = {
+      {{adam_kernel<false, false, CLIP_NONE>, adam_kernel<false, false, CLIP_NORM>, adam_kernel<false, false, CLIP_VALUE>},
+       {adam_kernel<false, true, CLIP_NONE>, adam_kernel<false, true, CLIP_NORM>, adam_kernel<false, true, CLIP_VALUE>}},
+      {{adam_kernel<true, false, CLIP_NONE>, adam_kernel<true, false, CLIP_NORM>, adam_kernel<true, false, CLIP_VALUE>},
+       {adam_kernel<true, true, CLIP_NONE>, adam_kernel<true, true, CLIP_NORM>, adam_kernel<true, true, CLIP_VALUE>}}};
+  launch_dep(kernels[dc][ex][clip_mode], dim3(ew_grid(ex ? n : n / 4 + 1)), dim3(256), 0, static_cast<cudaStream_t>(stream), p, g, m, v, vmax, n, a,
+             beta1, beta2, lr_dev, dc ? &counters->adam_step : nullptr, (int)amsgrad, (int)maximize, static_cast<bf16*>(shadow_bf16), clip_coef,
+             (float)clip_value);
   count_launch();
-  PSVAE_LAUNCH_CHECK("adam_dc_kernel");
+  PSVAE_LAUNCH_CHECK("adam_kernel");
   return 0;
 }
 
-int psvae_step_counters_advance(psvae_step_counters* counters, void* stream) {
-  PSVAE_TRY(tc_device_check());
-  if (!counters) { set_error("counters must not be NULL"); return -1; }
-  launch_dep(step_counters_advance_kernel, dim3(1), dim3(1), 0, static_cast<cudaStream_t>(stream), &counters->rng_offset, &counters->adam_step);
-  count_launch();
-  PSVAE_LAUNCH_CHECK("step_counters_advance_kernel");
-  return 0;
+int psvae_adam_step(float* p, const float* g, float* m, float* v, int64_t n, double lr, double beta1, double beta2, double eps, double weight_decay,
+                    int64_t step, double grad_scale, void* shadow_bf16, void* stream) {
+  return adam_update(false, p, g, m, v, nullptr, n, lr, step, nullptr, nullptr, beta1, beta2, eps, weight_decay, grad_scale, 0, 0, PSVAE_CLIP_NONE,
+                     nullptr, 0.0, shadow_bf16, stream);
 }
+
+int psvae_adam_step_ex(float* p, const float* g, float* m, float* v, float* vmax, int64_t n, double lr, double beta1, double beta2, double eps,
+                       double weight_decay, int64_t step, double grad_scale, int32_t amsgrad, int32_t maximize, void* shadow_bf16, void* stream) {
+  return adam_update(false, p, g, m, v, vmax, n, lr, step, nullptr, nullptr, beta1, beta2, eps, weight_decay, grad_scale, amsgrad, maximize,
+                     PSVAE_CLIP_NONE, nullptr, 0.0, shadow_bf16, stream);
+}
+
+int psvae_adam_step_dc(float* p, const float* g, float* m, float* v, float* vmax, int64_t n, const double* lr, const psvae_step_counters* counters,
+                       double beta1, double beta2, double eps, double weight_decay, double grad_scale, int32_t amsgrad, int32_t maximize, void* shadow_bf16,
+                       void* stream) {
+  return adam_update(true, p, g, m, v, vmax, n, 0.0, 0, lr, counters, beta1, beta2, eps, weight_decay, grad_scale, amsgrad, maximize,
+                     PSVAE_CLIP_NONE, nullptr, 0.0, shadow_bf16, stream);
+}
+
+int psvae_step_counters_advance(psvae_step_counters* counters, void* stream) { return psvae_step_counters_advance_by(counters, 1, 1, stream); }
 
 int psvae_step_counters_advance_by(psvae_step_counters* counters, uint64_t rng_delta, int64_t step_delta, void* stream) {
   PSVAE_TRY(tc_device_check());
@@ -1756,65 +1736,12 @@ int psvae_grad_norm(const float* g, const int64_t* spans, int32_t n_spans, doubl
   return 0;
 }
 
-extern "C++" template <bool DC, bool EX>
-void launch_adam_clip(int clip_mode, int64_t n, cudaStream_t st, float* p, const float* g, float* m, float* v, float* vmax, const AdamArgs& a,
-                             double beta1, double beta2, const double* lr, const int64_t* step_done, int amsgrad, int maximize, bf16* sh,
-                             const float* coef, float clip_value) {
-  const dim3 grid(ew_grid(EX ? n : n / 4 + 1));
-  if (clip_mode == PSVAE_CLIP_NORM)
-    launch_dep(adam_clip_kernel<DC, EX, CLIP_NORM>, grid, dim3(256), 0, st, p, g, m, v, vmax, n, a, beta1, beta2, lr, step_done, amsgrad, maximize, sh,
-               coef, clip_value);
-  else
-    launch_dep(adam_clip_kernel<DC, EX, CLIP_VALUE>, grid, dim3(256), 0, st, p, g, m, v, vmax, n, a, beta1, beta2, lr, step_done, amsgrad, maximize, sh,
-               coef, clip_value);
-}
-
 int psvae_adam_step_clip(float* p, const float* g, float* m, float* v, float* vmax, int64_t n, double lr, int64_t step, const double* lr_dev,
                          const psvae_step_counters* counters, double beta1, double beta2, double eps, double weight_decay, double grad_scale,
                          int32_t amsgrad, int32_t maximize, int32_t clip_mode, const float* clip_coef, double clip_value, void* shadow_bf16,
                          void* stream) {
-  const bool dc = counters != nullptr;
-  if (clip_mode == PSVAE_CLIP_NONE)
-    return dc ? psvae_adam_step_dc(p, g, m, v, vmax, n, lr_dev, counters, beta1, beta2, eps, weight_decay, grad_scale, amsgrad, maximize, shadow_bf16, stream)
-              : psvae_adam_step_ex(p, g, m, v, vmax, n, lr, beta1, beta2, eps, weight_decay, step, grad_scale, amsgrad, maximize, shadow_bf16, stream);
-  PSVAE_TRY(tc_device_check());
-  if (clip_mode != PSVAE_CLIP_NORM && clip_mode != PSVAE_CLIP_VALUE) { set_error("clip_mode=%d is not a PSVAE_CLIP_* value", (int)clip_mode); return -2; }
-  if (!p || !g || !m || !v || (amsgrad && !vmax) || (dc && !lr_dev) || (clip_mode == PSVAE_CLIP_NORM && !clip_coef)) {
-    set_error("p, g, m, v (vmax with amsgrad, lr_dev with counters, clip_coef with PSVAE_CLIP_NORM) must not be NULL");
-    return -1;
-  }
-  if (clip_mode == PSVAE_CLIP_VALUE && !(clip_value >= 0.0)) { set_error("clip_value=%g must be >= 0", clip_value); return -2; }
-  if (n <= 0) return 0;
-  if (!dc && step < 1) { set_error("step=%lld must be >= 1 (count after increment)", (long long)step); return -2; }
-  const bool ex = amsgrad || maximize;
-  if (!ex && ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v)) & 15) != 0) {
-    set_error("Adam buffers must be 16-byte aligned");
-    return -2;
-  }
-  AdamArgs a;
-  if (dc) {                  // formed on the device from *lr_dev and the step counter
-    a.lr_step = 0.f; a.bc2_sqrt = 1.f;
-  } else {
-    const double bc1 = 1.0 - pow(beta1, (double)step);
-    const double bc2 = 1.0 - pow(beta2, (double)step);
-    a.lr_step = (float)(lr / bc1);
-    a.bc2_sqrt = (float)sqrt(bc2);
-  }
-  a.beta1 = (float)beta1; a.beta2 = (float)beta2;
-  a.one_minus_beta1 = (float)(1.0 - beta1);
-  a.one_minus_beta2 = (float)(1.0 - beta2);
-  a.eps = (float)eps; a.weight_decay = (float)weight_decay; a.grad_scale = (float)grad_scale;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  bf16* sh = static_cast<bf16*>(shadow_bf16);
-  const int64_t* sd = dc ? &counters->adam_step : nullptr;
-  const float cv = (float)clip_value;
-  if (dc && ex) launch_adam_clip<true, true>(clip_mode, n, st, p, g, m, v, vmax, a, beta1, beta2, lr_dev, sd, amsgrad, maximize, sh, clip_coef, cv);
-  else if (dc) launch_adam_clip<true, false>(clip_mode, n, st, p, g, m, v, nullptr, a, beta1, beta2, lr_dev, sd, 0, 0, sh, clip_coef, cv);
-  else if (ex) launch_adam_clip<false, true>(clip_mode, n, st, p, g, m, v, vmax, a, beta1, beta2, nullptr, nullptr, amsgrad, maximize, sh, clip_coef, cv);
-  else launch_adam_clip<false, false>(clip_mode, n, st, p, g, m, v, nullptr, a, beta1, beta2, nullptr, nullptr, 0, 0, sh, clip_coef, cv);
-  count_launch();
-  PSVAE_LAUNCH_CHECK("adam_clip_kernel");
-  return 0;
+  return adam_update(counters != nullptr, p, g, m, v, vmax, n, lr, step, lr_dev, counters, beta1, beta2, eps, weight_decay, grad_scale, amsgrad,
+                     maximize, clip_mode, clip_coef, clip_value, shadow_bf16, stream);
 }
 
 int psvae_philox_uint32(uint32_t* out, int64_t n, uint64_t seed, uint64_t offset, int64_t first_elem, void* stream) {
@@ -1866,12 +1793,54 @@ int psvae_refresh_shadow(const psvae_model_desc* desc, const float* params, void
   return 0;
 }
 
-// x arrives as fp32 or (PSVAE_X_BF16) bf16
-static int set_x(StepArgs& a, const void* x, int32_t x_dtype) {
-  a.x = nullptr; a.x16 = nullptr;
+// The StepArgs of a model step with what every step takes; x arrives as fp32 or (PSVAE_X_BF16) bf16.  Losses, labels and gradients are off.
+static int make_step(StepArgs& a, const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x,
+                     int32_t x_dtype, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float* x_hat, float* mu,
+                     float* log_sigma, void* workspace, int64_t workspace_bytes, void* stream) {
+  a = StepArgs{desc, params, static_cast<const bf16*>(shadow_bf16), grads, nullptr, nullptr, eps, seed, offset, row0, rows, 0.f, 0.f,
+               0, 0, 0, x_hat, mu, log_sigma, nullptr, workspace, workspace_bytes, static_cast<cudaStream_t>(stream)};
   if (x_dtype == PSVAE_X_F32) a.x = static_cast<const float*>(x);
   else if (x_dtype == PSVAE_X_BF16) a.x16 = static_cast<const bf16*>(x);
   else { set_error("unknown x_dtype %d", x_dtype); return -2; }
+  return 0;
+}
+
+// The train step behind every psvae_train_fwd_bwd* entry point (psvae_train_fwd_bwd_scoped's arguments; cons == NULL: no consistency term,
+// counters == NULL: the host Philox offset).  accumulate (with compute_grads): the step writes this micro-batch's gradient into grad_scratch
+// exactly as the non-accumulating step writes `grads`; one pass then adds it (the classifier scope: over the classifier span only -- vae_numel
+// is a multiple of 8 floats, so the span stays 16-byte aligned).
+static int train_step(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
+                      const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
+                      int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
+                      void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
+                      const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters, int32_t accumulate, float* grad_scratch,
+                      int32_t grad_scope) {
+  PSVAE_TRY(check_desc(desc, precision));
+  const bool acc = accumulate && compute_grads;
+  if (acc) {
+    if (!grads || !grad_scratch) { set_error("grads and grad_scratch must not be NULL when accumulate != 0"); return -1; }
+    if (((reinterpret_cast<uintptr_t>(grads) | reinterpret_cast<uintptr_t>(grad_scratch)) & 15) != 0) {
+      set_error("grads and grad_scratch must be 16-byte aligned");
+      return -2;
+    }
+    if (grads == grad_scratch) { set_error("grad_scratch must not be the gradient buffer"); return -2; }
+  }
+  StepArgs a;
+  PSVAE_TRY(make_step(a, desc, params, shadow_bf16, acc ? grad_scratch : grads, x, x_dtype, eps, seed, offset, row0, rows, x_hat, mu, log_sigma,
+                      workspace, workspace_bytes, stream));
+  a.y = y; a.kl_w = kl_weight; a.clf_w = clf_weight; a.use_cos = use_cos_loss ? 1 : 0;
+  a.want_loss = 1; a.want_grads = compute_grads ? 1 : 0; a.losses = losses;
+  a.cons = cons; a.cons_params = cons_params; a.cons_y = cons_y; a.cons_w = cons_weight;
+  a.offset_dev = counters ? &counters->rng_offset : nullptr;
+  a.grad_scope = grad_scope;
+  PSVAE_TRY(precision == PSVAE_BF16 ? run_step<bf16>(a) : run_step<float>(a));
+  if (!acc) return 0;
+  const int64_t a0 = grad_scope == PSVAE_GRAD_CLASSIFIER ? desc->vae_numel : 0;
+  const int64_t n = desc->total_numel - a0;
+  launch_dep(grad_accumulate_kernel, dim3(ew_grid(n / 4 + 1)), dim3(256), 0, static_cast<cudaStream_t>(stream), grads + a0,
+             (const float*)grad_scratch + a0, n);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("grad_accumulate_kernel");
   return 0;
 }
 
@@ -1879,11 +1848,9 @@ int psvae_train_fwd_bwd(const psvae_model_desc* desc, const float* params, const
                         const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
                         int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
                         void* workspace, int64_t workspace_bytes, void* stream) {
-  PSVAE_TRY(check_desc(desc, precision));
-  StepArgs a{desc, params, static_cast<const bf16*>(shadow_bf16), grads, nullptr, y, eps, seed, offset, row0, rows, kl_weight, clf_weight,
-             use_cos_loss ? 1 : 0, 1, compute_grads ? 1 : 0, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, static_cast<cudaStream_t>(stream)};
-  PSVAE_TRY(set_x(a, x, x_dtype));
-  return precision == PSVAE_BF16 ? run_step<bf16>(a) : run_step<float>(a);
+  return train_step(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss, compute_grads,
+                    precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, nullptr, nullptr, nullptr, 0.f, nullptr, 0, nullptr,
+                    PSVAE_GRAD_ALL);
 }
 
 int psvae_consistency_desc_init(psvae_consistency_desc* cons, int32_t input_dim, int32_t hidden_dim, int32_t num_classes) {
@@ -2016,72 +1983,19 @@ int psvae_train_fwd_bwd_consistency(const psvae_model_desc* desc, const float* p
                                     const psvae_consistency_desc* cons, const float* cons_params, const int64_t* cons_y, float cons_weight) {
   PSVAE_TRY(check_desc(desc, precision));
   if (!cons) { set_error("consistency desc is NULL (use psvae_train_fwd_bwd for a step without the consistency term)"); return -1; }
-  StepArgs a{desc, params, static_cast<const bf16*>(shadow_bf16), grads, nullptr, y, eps, seed, offset, row0, rows, kl_weight, clf_weight,
-             use_cos_loss ? 1 : 0, 1, compute_grads ? 1 : 0, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, static_cast<cudaStream_t>(stream)};
-  PSVAE_TRY(set_x(a, x, x_dtype));
-  a.cons = cons; a.cons_params = cons_params; a.cons_y = cons_y; a.cons_w = cons_weight;
-  return precision == PSVAE_BF16 ? run_step<bf16>(a) : run_step<float>(a);
+  return train_step(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss, compute_grads,
+                    precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y, cons_weight, nullptr, 0,
+                    nullptr, PSVAE_GRAD_ALL);
 }
-
-}  // extern "C"
-
-// psvae_train_fwd_bwd_dc / _acc with a gradient scope (psvae_train_fwd_bwd_scoped)
-static int train_dc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
-                    const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
-                    int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
-                    void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
-                    const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters, int32_t grad_scope) {
-  PSVAE_TRY(check_desc(desc, precision));
-  StepArgs a{desc, params, static_cast<const bf16*>(shadow_bf16), grads, nullptr, y, eps, seed, offset, row0, rows, kl_weight, clf_weight,
-             use_cos_loss ? 1 : 0, 1, compute_grads ? 1 : 0, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, static_cast<cudaStream_t>(stream)};
-  PSVAE_TRY(set_x(a, x, x_dtype));
-  a.cons = cons; a.cons_params = cons_params; a.cons_y = cons_y; a.cons_w = cons_weight;
-  a.offset_dev = counters ? &counters->rng_offset : nullptr;
-  a.grad_scope = grad_scope;
-  return precision == PSVAE_BF16 ? run_step<bf16>(a) : run_step<float>(a);
-}
-
-static int train_acc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
-                     const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
-                     int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
-                     void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
-                     const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters, int32_t accumulate, float* grad_scratch,
-                     int32_t grad_scope) {
-  if (!accumulate || !compute_grads)
-    return train_dc(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss,
-                    compute_grads, precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y,
-                    cons_weight, counters, grad_scope);
-  PSVAE_TRY(check_desc(desc, precision));
-  if (!grads || !grad_scratch) { set_error("grads and grad_scratch must not be NULL when accumulate != 0"); return -1; }
-  if (((reinterpret_cast<uintptr_t>(grads) | reinterpret_cast<uintptr_t>(grad_scratch)) & 15) != 0) {
-    set_error("grads and grad_scratch must be 16-byte aligned");
-    return -2;
-  }
-  if (grads == grad_scratch) { set_error("grad_scratch must not be the gradient buffer"); return -2; }
-  // the step writes this micro-batch's gradient into the scratch exactly as the non-accumulating step writes `grads`; one pass then adds it
-  // (the classifier scope: over the classifier span only -- vae_numel is a multiple of 8 floats, so the span stays 16-byte aligned)
-  PSVAE_TRY(train_dc(desc, params, shadow_bf16, grad_scratch, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight,
-                     use_cos_loss, compute_grads, precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons,
-                     cons_params, cons_y, cons_weight, counters, grad_scope));
-  const int64_t a0 = grad_scope == PSVAE_GRAD_CLASSIFIER ? desc->vae_numel : 0;
-  const int64_t n = desc->total_numel - a0;
-  launch_dep(grad_accumulate_kernel, dim3(ew_grid(n / 4 + 1)), dim3(256), 0, static_cast<cudaStream_t>(stream), grads + a0,
-             (const float*)grad_scratch + a0, n);
-  count_launch();
-  PSVAE_LAUNCH_CHECK("grad_accumulate_kernel");
-  return 0;
-}
-
-extern "C" {
 
 int psvae_train_fwd_bwd_dc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
                            const int64_t* y, const float* eps, uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, float kl_weight, float clf_weight,
                            int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
                            void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
                            const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters) {
-  return train_dc(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss, compute_grads,
-                  precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y, cons_weight, counters,
-                  PSVAE_GRAD_ALL);
+  return train_step(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss, compute_grads,
+                    precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y, cons_weight, counters, 0,
+                    nullptr, PSVAE_GRAD_ALL);
 }
 
 int psvae_train_fwd_bwd_acc(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype,
@@ -2089,9 +2003,9 @@ int psvae_train_fwd_bwd_acc(const psvae_model_desc* desc, const float* params, c
                             int32_t use_cos_loss, int32_t compute_grads, int32_t precision, float* x_hat, float* mu, float* log_sigma, float* losses,
                             void* workspace, int64_t workspace_bytes, void* stream, const psvae_consistency_desc* cons, const float* cons_params,
                             const int64_t* cons_y, float cons_weight, const psvae_step_counters* counters, int32_t accumulate, float* grad_scratch) {
-  return train_acc(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss, compute_grads,
-                   precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y, cons_weight, counters,
-                   accumulate, grad_scratch, PSVAE_GRAD_ALL);
+  return train_step(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss, compute_grads,
+                    precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y, cons_weight, counters,
+                    accumulate, grad_scratch, PSVAE_GRAD_ALL);
 }
 
 int psvae_train_fwd_bwd_scoped(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x,
@@ -2107,18 +2021,19 @@ int psvae_train_fwd_bwd_scoped(const psvae_model_desc* desc, const float* params
     set_error("grad_scope PSVAE_GRAD_CLASSIFIER: the model has no latent classifier");
     return -2;
   }
-  return train_acc(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss, compute_grads,
-                   precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y, cons_weight, counters,
-                   accumulate, grad_scratch, grad_scope);
+  return train_step(desc, params, shadow_bf16, grads, x, x_dtype, y, eps, seed, offset, row0, rows, kl_weight, clf_weight, use_cos_loss, compute_grads,
+                    precision, x_hat, mu, log_sigma, losses, workspace, workspace_bytes, stream, cons, cons_params, cons_y, cons_weight, counters,
+                    accumulate, grad_scratch, grad_scope);
 }
 
 int psvae_vae_backward(const psvae_model_desc* desc, const float* params, const void* shadow_bf16, float* grads, const void* x, int32_t x_dtype, const float* eps,
                        uint64_t seed, uint64_t offset, int64_t row0, int64_t rows, int32_t precision, const float* g_x_hat, const float* g_mu,
                        const float* g_log_sigma, void* workspace, int64_t workspace_bytes, void* stream) {
   PSVAE_TRY(check_desc(desc, precision));
-  StepArgs a{desc, params, static_cast<const bf16*>(shadow_bf16), grads, nullptr, nullptr, eps, seed, offset, row0, rows, 0.f, 0.f,
-             0, 0, 1, nullptr, nullptr, nullptr, nullptr, workspace, workspace_bytes, static_cast<cudaStream_t>(stream)};
-  PSVAE_TRY(set_x(a, x, x_dtype));
+  StepArgs a;
+  PSVAE_TRY(make_step(a, desc, params, shadow_bf16, grads, x, x_dtype, eps, seed, offset, row0, rows, nullptr, nullptr, nullptr, workspace,
+                      workspace_bytes, stream));
+  a.want_grads = 1;
   a.ext = 1; a.ext_gx = g_x_hat; a.ext_gmu = g_mu; a.ext_gls = g_log_sigma;
   return precision == PSVAE_BF16 ? run_step<bf16>(a) : run_step<float>(a);
 }
@@ -2128,9 +2043,9 @@ int psvae_forward(const psvae_model_desc* desc, const float* params, const void*
                   int64_t workspace_bytes, void* stream) {
   PSVAE_TRY(check_desc(desc, precision));
   if (!x_hat) { set_error("x_hat must not be NULL"); return -1; }
-  StepArgs a{desc, params, static_cast<const bf16*>(shadow_bf16), nullptr, nullptr, nullptr, eps, seed, offset, row0, rows, 0.f, 0.f,
-             0, 0, 0, x_hat, mu, log_sigma, nullptr, workspace, workspace_bytes, static_cast<cudaStream_t>(stream)};
-  PSVAE_TRY(set_x(a, x, x_dtype));
+  StepArgs a;
+  PSVAE_TRY(make_step(a, desc, params, shadow_bf16, nullptr, x, x_dtype, eps, seed, offset, row0, rows, x_hat, mu, log_sigma, workspace,
+                      workspace_bytes, stream));
   return precision == PSVAE_BF16 ? run_step<bf16>(a) : run_step<float>(a);
 }
 

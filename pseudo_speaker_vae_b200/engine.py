@@ -463,18 +463,19 @@ class HotPath:
              consistency: Optional[nn.Module] = None, consistency_y: Optional[torch.Tensor] = None, consistency_weight: float = 1.0,
              counters: Optional[torch.Tensor] = None, accumulate: bool = False, grad_scratch: Optional[torch.Tensor] = None,
              grad_scope: str = "all"):
-        """One fused forward(+backward).  Returns (losses[16] device tensor, flat grads or None, outputs or None).
+        """One fused forward(+backward), ``psvae_train_fwd_bwd_scoped``.  Returns (losses[16] device tensor, flat grads or None, outputs or
+        None).
 
         ``consistency``: a frozen ``EmbeddingClassifier`` whose ``consistency_weight * CE(consistency(x_hat), consistency_y)``
         joins the loss (lightning.py:100-108, 119-124).  losses slots: _lib.LOSS_*; nothing here synchronises with the host.
         ``counters``: a device ``psvae_step_counters`` block (int64 [_lib.COUNTER_SLOTS]); the Philox offset of the eps draw is then read
-        from it on the device (``psvae_train_fwd_bwd_dc``), so that a CUDA graph of this call draws fresh noise at every replay.  The host
-        offset still advances as usual: it is the mirror the caller keeps the block in step with.
-        ``accumulate``: ADD this batch's gradients to what ``grads`` holds (``psvae_train_fwd_bwd_acc``: they are computed into
-        ``grad_scratch``, a flat fp32 buffer of the arena's size, then added with one fp32 addition per element).
+        from it on the device, so that a CUDA graph of this call draws fresh noise at every replay.  The host offset still advances as
+        usual: it is the mirror the caller keeps the block in step with.
+        ``accumulate``: ADD this batch's gradients to what ``grads`` holds (they are computed into ``grad_scratch``, a flat fp32 buffer of
+        the arena's size, then added with one fp32 addition per element).
         ``grad_scope``: ``"all"``, or ``"classifier"`` for a frozen VAE (``train_scope()``): the same forward and losses, but only the latent
         classifier's gradients are computed, and only the classifier span of ``grads`` (``classifier_span()``) is written -- or, with
-        ``accumulate``, added to; every other element of ``grads`` keeps its value (``psvae_train_fwd_bwd_scoped``)."""
+        ``accumulate``, added to; every other element of ``grads`` keeps its value."""
         if grad_scope not in ("all", "classifier"):
             raise ValueError(f"grad_scope must be 'all' or 'classifier', got {grad_scope!r}")
         if grad_scope == "classifier" and self.classifier is None:
@@ -527,37 +528,16 @@ class HotPath:
             cons_args = (C.byref(cdesc), cflat.data_ptr(), cy.data_ptr(), float(consistency_weight))
         if counters is not None and (counters.device != dev or counters.dtype != torch.int64 or counters.numel() != L.COUNTER_SLOTS):
             raise ValueError(f"counters must be an int64 [{L.COUNTER_SLOTS}] tensor on {dev}")
-        if accumulate and compute_grads:
+        acc = bool(accumulate and compute_grads)
+        if acc:
             if grads is None or grad_scratch is None or grad_scratch.device != dev or grad_scratch.dtype != torch.float32 \
                     or grad_scratch.numel() < self.arena.numel or grad_scratch.data_ptr() == grads.data_ptr():
                 raise ValueError("an accumulating step needs `grads` and a separate fp32 `grad_scratch` of the arena's size on the same device")
-        if clf_scope:
-            with _on(dev):
-                ws = self._workspace(dev, B, mode, extra if consistency is not None else 0)
-                rc = L.lib().psvae_train_fwd_bwd_scoped(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args, L.ptr(counters),
-                                                        int(bool(accumulate)), L.ptr(grad_scratch) if accumulate else None, L.GRAD_CLASSIFIER)
-            L.check(rc, "psvae_train_fwd_bwd_scoped")
-        elif accumulate and compute_grads:
-            with _on(dev):
-                ws = self._workspace(dev, B, mode, extra if consistency is not None else 0)
-                rc = L.lib().psvae_train_fwd_bwd_acc(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args, L.ptr(counters), 1,
-                                                     grad_scratch.data_ptr())
-            L.check(rc, "psvae_train_fwd_bwd_acc")
-        elif counters is not None:
-            with _on(dev):
-                ws = self._workspace(dev, B, mode, extra if consistency is not None else 0)
-                rc = L.lib().psvae_train_fwd_bwd_dc(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args, counters.data_ptr())
-            L.check(rc, "psvae_train_fwd_bwd_dc")
-        elif consistency is None:
-            with _on(dev):
-                ws = self._workspace(dev, B, mode)
-                rc = L.lib().psvae_train_fwd_bwd(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev))
-            L.check(rc, "psvae_train_fwd_bwd")
-        else:
-            with _on(dev):
-                ws = self._workspace(dev, B, mode, extra)
-                rc = L.lib().psvae_train_fwd_bwd_consistency(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args)
-            L.check(rc, "psvae_train_fwd_bwd_consistency")
+        with _on(dev):
+            ws = self._workspace(dev, B, mode, extra if consistency is not None else 0)
+            rc = L.lib().psvae_train_fwd_bwd_scoped(*args, ws.data_ptr(), ws.numel(), _stream_ptr(dev), *cons_args, L.ptr(counters), int(acc),
+                                                    L.ptr(grad_scratch) if acc else None, L.GRAD_CLASSIFIER if clf_scope else L.GRAD_ALL)
+        L.check(rc, "psvae_train_fwd_bwd_scoped")
         return losses, (grads if compute_grads else None), outs
 
     def train_scope(self) -> str:

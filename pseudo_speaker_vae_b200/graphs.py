@@ -139,10 +139,7 @@ class GraphedTrainStep:
         lib, stream = L.lib(), _stream_ptr(self.device)
         with _on(self.device):
             for gi in range(self.counters.shape[0]):
-                if phase == (False, True):
-                    L.check(lib.psvae_step_counters_advance(self.counters[gi].data_ptr(), stream), "psvae_step_counters_advance")
-                else:
-                    L.check(lib.psvae_step_counters_advance_by(self.counters[gi].data_ptr(), 1, int(step), stream), "psvae_step_counters_advance_by")
+                L.check(lib.psvae_step_counters_advance_by(self.counters[gi].data_ptr(), 1, int(step), stream), "psvae_step_counters_advance_by")
         return losses
 
     def _try_capture(self, kind: Optional[str], pdl: int, phase: Tuple[bool, bool] = (False, True)) -> Tuple[Optional[torch.cuda.CUDAGraph], Optional[torch.Tensor], Optional[BaseException]]:

@@ -9,8 +9,8 @@ all-reduce they hold the SUM over ranks: ``grad_scale = 1 / world_size`` folds t
 In bf16 mode the same pass also refreshes the bf16 operand copy the tcgen05 GEMMs read.
 
 ``amsgrad`` (state key ``max_exp_avg_sq``, a third flat buffer) and ``maximize`` -- both reachable through
-``Adam(self.parameters(), **self.hparams["optimizer"])`` -- take the general kernel (``psvae_adam_step_ex``);
-``capturable`` / ``differentiable`` are not on the reference's path and raise.
+``Adam(self.parameters(), **self.hparams["optimizer"])`` -- take the general form of the kernel (one element per thread);
+``capturable`` / ``differentiable`` are not on the reference's path and raise.  Every update goes through ``psvae_adam_step_clip``.
 
 Gradient clipping (Lightning's ``gradient_clip_val`` / ``gradient_clip_algorithm``) happens inside the same pass when ``clip_mode`` is set
 (``DataParallelTrainer`` sets it, as it sets ``grad_scale``): ``"norm"`` scales ``g`` by ``grad_scale * clip_coef`` (``clip_coef``: a device
@@ -135,7 +135,7 @@ class FusedAdam(torch.optim.Optimizer):
     def _update(self, counters: Optional[torch.Tensor] = None, lrs: Optional[torch.Tensor] = None) -> None:
         """The update of every group with gradients, one pass per merged span.  ``counters`` / ``lrs``: the device-counter form a CUDA graph
         of the train step replays (graphs.py) -- one ``psvae_step_counters`` block per group (int64 [groups, COUNTER_SLOTS]) and one fp64
-        learning rate per group, read on the device (``psvae_adam_step_dc``).  That form moves no host state: the caller advances the step
+        learning rate per group, read on the device.  That form moves no host state: the caller advances the step
         counts, the arena epoch and the shadow mark, and the device block, itself."""
         dc = counters is not None
         clip = {"none": L.CLIP_NONE, "norm": L.CLIP_NORM, "value": L.CLIP_VALUE}[self.clip_mode]
@@ -175,26 +175,12 @@ class FusedAdam(torch.optim.Optimizer):
                     shadow = self.arena.shadow.data_ptr() + 2 * a
                 vmax = self._vmax.data_ptr() + 4 * a if group["amsgrad"] else None
                 with _on(dev):
-                    if clip != L.CLIP_NONE:
-                        rc = lib.psvae_adam_step_clip(flat.data_ptr() + 4 * a, gflat.data_ptr() + 4 * a, m.data_ptr() + 4 * a, v.data_ptr() + 4 * a, vmax,
-                                                      b - a, float(group["lr"]), step, L.ptr(lrs[gi]) if dc else None,
-                                                      counters[gi].data_ptr() if dc else None, float(beta1), float(beta2), float(group["eps"]),
-                                                      float(group["weight_decay"]), float(self.grad_scale), int(bool(group["amsgrad"])),
-                                                      int(bool(group["maximize"])), clip, L.ptr(self.clip_coef), float(self.clip_value), shadow, stream)
-                    elif dc:
-                        rc = lib.psvae_adam_step_dc(flat.data_ptr() + 4 * a, gflat.data_ptr() + 4 * a, m.data_ptr() + 4 * a, v.data_ptr() + 4 * a, vmax, b - a,
-                                                    lrs[gi].data_ptr(), counters[gi].data_ptr(), float(beta1), float(beta2), float(group["eps"]),
-                                                    float(group["weight_decay"]), float(self.grad_scale), int(bool(group["amsgrad"])),
-                                                    int(bool(group["maximize"])), shadow, stream)
-                    elif group["amsgrad"] or group["maximize"]:
-                        rc = lib.psvae_adam_step_ex(flat.data_ptr() + 4 * a, gflat.data_ptr() + 4 * a, m.data_ptr() + 4 * a, v.data_ptr() + 4 * a, vmax, b - a,
-                                                    float(group["lr"]), float(beta1), float(beta2), float(group["eps"]), float(group["weight_decay"]),
-                                                    step, float(self.grad_scale), int(bool(group["amsgrad"])), int(bool(group["maximize"])), shadow, stream)
-                    else:
-                        rc = lib.psvae_adam_step(flat.data_ptr() + 4 * a, gflat.data_ptr() + 4 * a, m.data_ptr() + 4 * a, v.data_ptr() + 4 * a, b - a,
-                                                 float(group["lr"]), float(beta1), float(beta2), float(group["eps"]), float(group["weight_decay"]),
-                                                 step, float(self.grad_scale), shadow, stream)
-                L.check(rc, "psvae_adam_step")
+                    rc = lib.psvae_adam_step_clip(flat.data_ptr() + 4 * a, gflat.data_ptr() + 4 * a, m.data_ptr() + 4 * a, v.data_ptr() + 4 * a, vmax,
+                                                  b - a, float(group["lr"]), step, L.ptr(lrs[gi]) if dc else None,
+                                                  counters[gi].data_ptr() if dc else None, float(beta1), float(beta2), float(group["eps"]),
+                                                  float(group["weight_decay"]), float(self.grad_scale), int(bool(group["amsgrad"])),
+                                                  int(bool(group["maximize"])), clip, L.ptr(self.clip_coef), float(self.clip_value), shadow, stream)
+                L.check(rc, "psvae_adam_step_clip")
                 touched = True
             if not dc:
                 step_t += 1
