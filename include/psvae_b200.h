@@ -342,6 +342,24 @@ int psvae_langevin_rows(const psvae_model_desc* desc, const float* params, float
                         int32_t init_from_philox, const float* noise, float* history, float* stats, float prior_weight, float threshold,
                         int32_t* stop_step, float* last_prob, void* stream);
 
+/* ---- cosine top-k search between two embedding sets (additive to ABI 5) ----------------------------
+ * For every query row i of q [nq][dim] the k keys j of keys [nk][dim] with the highest (default) or lowest (PSVAE_TOPK_SMALLEST) cosine
+ * similarity sim = q.x / (max(|q|, 1e-8) max(|x|, 1e-8)) (torch's F.cosine_similarity: a zero row scores 0).  Each set is fp32
+ * (PSVAE_X_F32) or bf16 (PSVAE_X_BF16), contiguous, 1 <= k <= 16, dim a multiple of 8 and <= 512; q and keys may be the same array.
+ * Candidates are selected from bf16-rounded unit vectors (fp32 accumulation on the tensor cores), the best 2k per row are re-scored in
+ * fp32 from the inputs, and the best k of those are returned: out_sim fp32 [nq][k], out_idx int64 [nq][k] (global: k_row0 + j).  Equal
+ * similarities go to the lower key index; a NaN similarity is never chosen; a slot without a candidate holds -1 / NaN.  With
+ * PSVAE_TOPK_EXCLUDE_SELF the pairs q_row0 + i == k_row0 + j are skipped (k <= nk - 1).  The result is bit-identical from run to run, for
+ * any sharding of the queries (q_row0) and any split of the key range (option "topk_key_splits").
+ * workspace: psvae_cosine_topk_workspace_bytes(nq, nk, dim, k) bytes, 256-byte aligned (it depends on the option "topk_key_splits").
+ * Argument errors are reported before the device is looked at. */
+#define PSVAE_TOPK_SMALLEST 1
+#define PSVAE_TOPK_EXCLUDE_SELF 2
+int64_t psvae_cosine_topk_workspace_bytes(int64_t nq, int64_t nk, int32_t dim, int32_t k);
+int psvae_cosine_topk(const void* q, int32_t q_dtype, int64_t nq, int64_t q_row0, const void* keys, int32_t k_dtype, int64_t nk,
+                      int64_t k_row0, int32_t dim, int32_t k, int32_t flags, float* out_sim, int64_t* out_idx, void* workspace,
+                      int64_t workspace_bytes, void* stream);
+
 /* ---- building block exposed for tests and profiling: C = A[M,K] * B[N,K]^T (+bias) ------------- */
 /* a_mn / b_mn: operand stored MN-major (A as [K][M], B as [K][N]).  bf16 in, fp32 out, tcgen05. */
 int psvae_gemm_bf16(const void* a_bf16, const void* b_bf16, const float* bias, float* c, int64_t m, int32_t n,

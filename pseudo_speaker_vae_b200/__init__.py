@@ -10,10 +10,11 @@ from .lightning import PseudoSpeakerVAE
 from .model import VAEModel
 from .optim import FusedAdam
 from .parallel import DataParallelTrainer
+from .search import cosine_topk
 from .utils import map_cv_age_to_label, map_cv_gender_to_label, map_vctk_gender_to_label, parse_classifier_target, sample_filename
 
 __all__ = [
     "VAEModel", "LatentClassifier", "EmbeddingClassifier", "PseudoSpeakerVAE", "FusedAdam", "DataParallelTrainer", "GraphedTrainStep", "unconditional_synthesis",
-    "conditional_synthesis", "latent_transformation", "PackedEmbeddingStore", "PinnedBatchLoader", "get_packed_dataloaders", "sample_on_device", "save_samples", "shard_rows", "map_cv_age_to_label", "map_cv_gender_to_label",
+    "conditional_synthesis", "latent_transformation", "PackedEmbeddingStore", "PinnedBatchLoader", "get_packed_dataloaders", "sample_on_device", "save_samples", "shard_rows", "cosine_topk", "map_cv_age_to_label", "map_cv_gender_to_label",
     "map_vctk_gender_to_label", "parse_classifier_target", "sample_filename",
 ]

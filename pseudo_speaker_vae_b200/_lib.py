@@ -36,7 +36,7 @@ EXPORTS = [
     "psvae_consistency_forward", "psvae_train_fwd_bwd_consistency", "psvae_vae_backward", "psvae_gather_rows",
     "psvae_embedding_classifier_workspace_bytes", "psvae_embedding_classifier_step", "psvae_train_fwd_bwd_dc", "psvae_adam_step_dc",
     "psvae_step_counters_advance", "psvae_train_fwd_bwd_acc", "psvae_grad_norm", "psvae_adam_step_clip", "psvae_step_counters_advance_by",
-    "psvae_train_fwd_bwd_scoped", "psvae_langevin_rows",
+    "psvae_train_fwd_bwd_scoped", "psvae_langevin_rows", "psvae_cosine_topk_workspace_bytes", "psvae_cosine_topk",
 ]
 
 #: int64 slots of ``psvae_step_counters`` (a device tensor of COUNTER_SLOTS int64)
@@ -46,6 +46,9 @@ CLIP_NONE, CLIP_NORM, CLIP_VALUE = 0, 1, 2
 GRAD_NORM_MAX_SPANS, GRAD_NORM_SCRATCH_BYTES = 16, 4096
 #: psvae_langevin_rows: entries of a target mix
 MAX_TARGET_MIX = 64
+#: psvae_cosine_topk flags and limits
+TOPK_SMALLEST, TOPK_EXCLUDE_SELF = 1, 2
+TOPK_MAX_K, TOPK_MAX_DIM = 16, 512
 
 
 class ModelDesc(C.Structure):
@@ -153,6 +156,11 @@ def _declare(l: C.CDLL) -> None:
         l.psvae_langevin_rows.restype = C.c_int
         l.psvae_langevin_rows.argtypes = [D, VP, VP, I64, VP, I32, P(I32), P(C.c_uint32), VP, F, I32, F, U64, U64, I64, I32, VP, VP, VP, F, F, VP, VP,
                                           VP]
+    if hasattr(l, "psvae_cosine_topk"):
+        l.psvae_cosine_topk_workspace_bytes.restype = I64
+        l.psvae_cosine_topk_workspace_bytes.argtypes = [I64, I64, I32, I32]
+        l.psvae_cosine_topk.restype = C.c_int
+        l.psvae_cosine_topk.argtypes = [VP, I32, I64, I64, VP, I32, I64, I64, I32, I32, I32, VP, VP, VP, I64, VP]
     l.psvae_gemm_bf16.restype = C.c_int
     l.psvae_gemm_bf16.argtypes = [VP, VP, VP, VP, I64, I32, I64, I32, I32, I32, I32, VP, I64, VP]
     l.psvae_gemm_probe.restype = C.c_int

@@ -23,6 +23,7 @@
 
 #include "../../include/psvae_b200.h"
 #include "common.cuh"
+#include "cosine_topk.cuh"
 #include "epilogue.cuh"
 #include "gemm_tc.cuh"
 #include "decoder_chain.cuh"
@@ -86,6 +87,7 @@ struct Options {
   int64_t tc_trace_select = 0;         // profiling: 1 = only ONE launch is traced (set "tc_trace_skip" = k to pick the (k+1)-th launch from now on)
   int64_t tc_max_stages = 0;           // experiments: cap the depth of the operand ring (0 = what fits)
   int64_t deterministic = 0;           // 1: split-K / bias partials go through ordered two-stage sums instead of TMA reduce-add / atomics
+  int64_t topk_key_splits = 0;         // tests: force the number of key ranges per query tile of psvae_cosine_topk (0 = chosen by topk_plan)
 };
 static Options g_opt;
 
@@ -1528,6 +1530,7 @@ int psvae_set_option(const char* name, int64_t value) {
   if (!strcmp(name, "tc_merged_wgrad")) { g_opt.tc_merged_wgrad = value ? 1 : 0; return 0; }
   if (!strcmp(name, "decode_chain")) { g_opt.decode_chain = value ? 1 : 0; return 0; }
   if (!strcmp(name, "train_chain")) { g_opt.train_chain = value ? 1 : 0; return 0; }
+  if (!strcmp(name, "topk_key_splits")) { g_opt.topk_key_splits = value < 0 ? 0 : value; return 0; }
   set_error("unknown option '%s'", name);
   return -2;
 }
@@ -1554,6 +1557,7 @@ int64_t psvae_get_option(const char* name) {
   if (!strcmp(name, "tc_merged_wgrad")) return g_opt.tc_merged_wgrad;
   if (!strcmp(name, "decode_chain")) return g_opt.decode_chain;
   if (!strcmp(name, "train_chain")) return g_opt.train_chain;
+  if (!strcmp(name, "topk_key_splits")) return g_opt.topk_key_splits;
   return -1;
 }
 
@@ -2298,6 +2302,166 @@ int psvae_gemm_fp32(const float* a, const float* b, const float* bias, float* c,
   }
   EpiBiasAct<float, ACT_NONE> e{bias, c, n, nullptr};
   return sgemm_launch(oa, ob, m, n, k, 1, vec, e, st);
+}
+
+}  // extern "C"
+
+// =================================================================================================
+// cosine top-k search (cosine_topk.cuh)
+// =================================================================================================
+namespace psvae {
+
+// Workspace carving and work split of one psvae_cosine_topk call.  Depends on the arguments and the option "topk_key_splits" only (not on the
+// device), so psvae_cosine_topk_workspace_bytes answers without a GPU.
+struct TopkPlan {
+  int64_t m_tiles, k_tiles, splits, tiles_per_split;
+  int64_t off_qn, off_kn, off_iq, off_ik, off_part, bytes;
+};
+
+static int topk_plan(int64_t nq, int64_t nk, int32_t dim, int32_t k, TopkPlan* p) {
+  if (nq <= 0 || nk <= 0) { set_error("nq and nk must be positive (nq=%lld nk=%lld)", (long long)nq, (long long)nk); return -2; }
+  if (nq > INT32_MAX || nk > INT32_MAX) { set_error("nq and nk must be < 2^31 (tensor-map coordinates)"); return -2; }
+  if (dim <= 0 || dim % 8 != 0 || dim > TK_MAX_DIM) { set_error("dim=%d: must be a positive multiple of 8, at most %d", dim, TK_MAX_DIM); return -2; }
+  if (k < 1 || k > TK_MAX_K) { set_error("k=%d out of range [1,%d]", k, TK_MAX_K); return -2; }
+  p->m_tiles = ceil_div64(nq, TK_BM);
+  p->k_tiles = ceil_div64(nk, TK_BN);
+  int64_t s = g_opt.topk_key_splits;
+  if (s <= 0) {
+    // few query tiles: split the key range so that (query tile, key range) items fill whole rounds of the persistent grid -- the
+    // fewest splits within 2 % of the best round efficiency among those giving at least one item per SM
+    s = 1;
+    if (p->m_tiles < 4 * PSVAE_NUM_SMS) {
+      const int64_t lo = std::min<int64_t>(p->k_tiles, ceil_div64(PSVAE_NUM_SMS, p->m_tiles)), hi = std::min<int64_t>(p->k_tiles, 4 * lo);
+      double best = -1.0;
+      for (int64_t c = lo; c <= hi; ++c) {
+        const int64_t items = p->m_tiles * ceil_div64(p->k_tiles, ceil_div64(p->k_tiles, c));
+        const double eff = (double)items / (double)(ceil_div64(items, PSVAE_NUM_SMS) * PSVAE_NUM_SMS);
+        if (eff > best + 0.02) { best = eff; s = c; }
+      }
+    }
+  }
+  if (s > p->k_tiles) s = p->k_tiles;
+  p->tiles_per_split = ceil_div64(p->k_tiles, s);
+  p->splits = ceil_div64(p->k_tiles, p->tiles_per_split);     // no empty key range
+  const int64_t C = 2 * (int64_t)k;
+  int64_t off = 0;
+  auto take = [&](int64_t bytes) { const int64_t o = off; off = align_up64(off + bytes, 256); return o; };
+  p->off_qn = take(nq * dim * 2);
+  p->off_kn = take(nk * dim * 2);
+  p->off_iq = take(nq * 4);
+  p->off_ik = take(nk * 4);
+  p->off_part = take(p->splits * p->m_tiles * TK_BM * C * 8);
+  p->bytes = off;
+  return 0;
+}
+
+template <typename TQ, typename TK, bool LARGEST>
+static int topk_launch(const TopkPlan& p, const void* q, int64_t nq, int64_t q_row0, const void* keys, int64_t nk, int64_t k_row0, int32_t dim,
+                       int32_t k, bool excl, float* out_sim, int64_t* out_idx, uint8_t* ws, cudaStream_t st) {
+  const TQ* qt = static_cast<const TQ*>(q);
+  const TK* kt = static_cast<const TK*>(keys);
+  bf16* qn = reinterpret_cast<bf16*>(ws + p.off_qn);
+  bf16* kn = reinterpret_cast<bf16*>(ws + p.off_kn);
+  float* iq = reinterpret_cast<float*>(ws + p.off_iq);
+  float* ik = reinterpret_cast<float*>(ws + p.off_ik);
+  int2* part = reinterpret_cast<int2*>(ws + p.off_part);
+  const int C = 2 * k;
+
+  topk_normalize_kernel<TQ><<<ew_grid(nq * 32), 256, 0, st>>>(qt, nq, dim, qn, iq);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("topk_normalize_kernel");
+  topk_normalize_kernel<TK><<<ew_grid(nk * 32), 256, 0, st>>>(kt, nk, dim, kn, ik);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("topk_normalize_kernel");
+
+  CUtensorMap tq, tk;
+  PSVAE_TRY(tc_tensor_map(TcOperand{qn, nq, dim, false}, dim, TK_BM, &tq));
+  PSVAE_TRY(tc_tensor_map(TcOperand{kn, nk, dim, false}, dim, TK_BN, &tk));
+  TopkShape s;
+  memset(&s, 0, sizeof(s));
+  s.nk = nk;
+  s.q_row0 = q_row0;
+  s.k_row0 = k_row0;
+  s.kb = (int32_t)ceil_div64(dim, TK_BK);
+  s.C = C;
+  s.m_tiles = (int32_t)p.m_tiles;
+  s.k_tiles = (int32_t)p.k_tiles;
+  s.splits = (int32_t)p.splits;
+  s.tiles_per_split = (int32_t)p.tiles_per_split;
+  s.exclude_self = excl ? 1 : 0;
+  s.part = part;
+  // shared memory: [barriers 1 KB][candidate lists C x 128 x 8 B][query tile kb x 16 KB][key ring stages x 32 KB]
+  s.list_off = TK_BAR_BYTES;
+  s.q_off = s.list_off + (uint32_t)align_up64((int64_t)C * TK_BM * 8, 1024);
+  s.ring_off = s.q_off + (uint32_t)(s.kb * TK_QBLOCK_BYTES);
+  const int64_t room = (int64_t)TK_SMEM_MAX - 1024 /*align slack*/ - s.ring_off;
+  s.stages = (int32_t)std::min<int64_t>(TK_MAX_STAGES, room / TK_STAGE_BYTES);
+  if (s.stages < 2) { set_error("cosine top-k: no room for the key ring (dim=%d, k=%d)", dim, k); return -2; }
+  const size_t smem = (size_t)s.ring_off + (size_t)s.stages * TK_STAGE_BYTES + 1024;
+  auto kern = topk_search_kernel<LARGEST>;
+  static unsigned long long attr_mask = 0;   // per instantiation, one bit per device
+  int dev = 0;
+  PSVAE_CUDA(cudaGetDevice(&dev));
+  if (!(attr_mask >> (dev & 63) & 1ull)) {
+    PSVAE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, TK_SMEM_MAX));
+    attr_mask |= 1ull << (dev & 63);
+  }
+  const int64_t items = p.m_tiles * p.splits;
+  const int grid = (int)std::min<int64_t>(items, tc_grid_size());
+  kern<<<grid, TK_THREADS, smem, st>>>(tq, tk, s);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("topk_search_kernel");
+
+  topk_merge_kernel<TQ, TK, LARGEST><<<ew_grid(nq * 32), 256, 0, st>>>(part, p.m_tiles * TK_BM, (int)p.splits, C, k, qt, kt, iq, ik, nq, dim, k_row0,
+                                                                  out_sim, out_idx);
+  count_launch();
+  PSVAE_LAUNCH_CHECK("topk_merge_kernel");
+  return 0;
+}
+
+template <typename TQ>
+static int topk_dispatch(int32_t k_dtype, bool smallest, const TopkPlan& p, const void* q, int64_t nq, int64_t q_row0, const void* keys, int64_t nk,
+                         int64_t k_row0, int32_t dim, int32_t k, bool excl, float* out_sim, int64_t* out_idx, uint8_t* ws, cudaStream_t st) {
+  if (k_dtype == PSVAE_X_F32) {
+    return smallest ? topk_launch<TQ, float, false>(p, q, nq, q_row0, keys, nk, k_row0, dim, k, excl, out_sim, out_idx, ws, st)
+                    : topk_launch<TQ, float, true>(p, q, nq, q_row0, keys, nk, k_row0, dim, k, excl, out_sim, out_idx, ws, st);
+  }
+  return smallest ? topk_launch<TQ, bf16, false>(p, q, nq, q_row0, keys, nk, k_row0, dim, k, excl, out_sim, out_idx, ws, st)
+                  : topk_launch<TQ, bf16, true>(p, q, nq, q_row0, keys, nk, k_row0, dim, k, excl, out_sim, out_idx, ws, st);
+}
+
+}  // namespace psvae
+
+extern "C" {
+
+int64_t psvae_cosine_topk_workspace_bytes(int64_t nq, int64_t nk, int32_t dim, int32_t k) {
+  TopkPlan p;
+  if (topk_plan(nq, nk, dim, k, &p) != 0) return -1;
+  return p.bytes;
+}
+
+int psvae_cosine_topk(const void* q, int32_t q_dtype, int64_t nq, int64_t q_row0, const void* keys, int32_t k_dtype, int64_t nk, int64_t k_row0,
+                      int32_t dim, int32_t k, int32_t flags, float* out_sim, int64_t* out_idx, void* workspace, int64_t workspace_bytes, void* stream) {
+  // argument checks first: they do not need a device
+  if ((q_dtype != PSVAE_X_F32 && q_dtype != PSVAE_X_BF16) || (k_dtype != PSVAE_X_F32 && k_dtype != PSVAE_X_BF16)) {
+    set_error("q_dtype=%d k_dtype=%d: each must be PSVAE_X_F32 or PSVAE_X_BF16", q_dtype, k_dtype);
+    return -2;
+  }
+  if (flags & ~(PSVAE_TOPK_SMALLEST | PSVAE_TOPK_EXCLUDE_SELF)) { set_error("unknown flags 0x%x", flags); return -2; }
+  if (q_row0 < 0 || k_row0 < 0) { set_error("q_row0 and k_row0 must be >= 0"); return -2; }
+  TopkPlan p;
+  PSVAE_TRY(topk_plan(nq, nk, dim, k, &p));
+  const bool excl = (flags & PSVAE_TOPK_EXCLUDE_SELF) != 0;
+  if (k > nk - (excl ? 1 : 0)) { set_error("k=%d exceeds the %lld keys available%s", k, (long long)(nk - (excl ? 1 : 0)), excl ? " (exclude_self)" : ""); return -2; }
+  if (workspace_bytes < p.bytes) { set_error("workspace of %lld bytes is too small: need %lld", (long long)workspace_bytes, (long long)p.bytes); return -2; }
+  PSVAE_TRY(tc_device_check());
+  if (!q || !keys || !out_sim || !out_idx || !workspace) { set_error("q, keys, out_sim, out_idx, workspace must not be NULL"); return -1; }
+  if ((reinterpret_cast<uintptr_t>(workspace) & 255) != 0) { set_error("workspace must be 256-byte aligned"); return -2; }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  const bool smallest = (flags & PSVAE_TOPK_SMALLEST) != 0;
+  if (q_dtype == PSVAE_X_F32) return topk_dispatch<float>(k_dtype, smallest, p, q, nq, q_row0, keys, nk, k_row0, dim, k, excl, out_sim, out_idx, ws, st);
+  return topk_dispatch<bf16>(k_dtype, smallest, p, q, nq, q_row0, keys, nk, k_row0, dim, k, excl, out_sim, out_idx, ws, st);
 }
 
 }  // extern "C"

@@ -195,7 +195,16 @@ def main(argv=None) -> None:
     parser.add_argument("--step_size", type=float, default=0.01)
     parser.add_argument("--noise_weight", type=float, default=1.0)
     parser.add_argument("--device", type=str, default="cuda", help="CUDA device (this implementation has no CPU path).")
+    parser.add_argument("--nearest_store", type=str, default=None,
+                        help="A PackedEmbeddingStore directory (e.g. the training set): each sample's nearest entries by cosine similarity, "
+                             "computed on the device, go to <save_dir>/nearest.pt as {'index': int64 [N, k], 'similarity': float32 [N, k]}.")
+    parser.add_argument("--nearest_k", type=int, default=1, help="Entries per sample for --nearest_store (1..16).")
     args = parser.parse_args(argv)
+    if args.nearest_store is not None:
+        if not 1 <= args.nearest_k <= 16:
+            parser.error(f"--nearest_k must be in [1, 16], got {args.nearest_k}")
+        if not os.path.isfile(os.path.join(args.nearest_store, "index.json")):
+            parser.error(f"--nearest_store {args.nearest_store!r} is not a PackedEmbeddingStore (no index.json)")
     target_mix = None
     if args.target_mix is not None:
         if args.classifier_target is not None:
@@ -221,6 +230,13 @@ def main(argv=None) -> None:
     save_samples(x_hat, args.save_dir)
     if targets is not None:
         torch.save(targets, os.path.join(args.save_dir, "targets.pt"))
+    if args.nearest_store is not None:
+        from .data import PackedEmbeddingStore
+        from .search import cosine_topk
+
+        keys = PackedEmbeddingStore(args.nearest_store).to_device(args.device)[0]
+        sim, idx = cosine_topk(x_hat.to(keys.device), keys, args.nearest_k)
+        torch.save({"index": idx.cpu(), "similarity": sim.cpu()}, os.path.join(args.save_dir, "nearest.pt"))
 
 
 if __name__ == "__main__":
