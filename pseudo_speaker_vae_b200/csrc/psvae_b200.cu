@@ -427,7 +427,7 @@ static int flush_wgrads(StepBufs<TAct>& w, int64_t rows, cudaStream_t st) {
   return gemm_tc_launch_multi_wgrad(w.pending, n, rows, st, g_opt.wgrad_order >= 2 ? 1 : 0);
 }
 
-// the fused classifier kernel covers the common shape: heads directly on mu (no trunk), L = 32/64/96/128, <= 8 classes in total
+// the fused classifier kernel covers the common shape: heads directly on mu (no trunk), L = 16/32/64/128, <= 8 classes in total
 static bool clf_fused_ok(const psvae_model_desc* d) {
   if (d->clf_num_heads <= 0 || d->clf_num_trunk != 0) return false;
   if (d->latent_dim != 16 && d->latent_dim != 32 && d->latent_dim != 64 && d->latent_dim != 128) return false;   // kernel instantiations
